@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — headline benchmark of the CRFConv hot path (BASELINE.json metric: CRFConv fwd+bwd points/s at N=40,960, k=16).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--config S1|C3|C4|C5] [--clouds B] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--config S1|C3|C4|C5] [--clouds B] [--impl reference] [--dump-outputs DIR]
 
 --config S1 (default; SURVEY.md §8 S1 = BASELINE configs[0] shape on the GPU): one *step* = forward + backward of ONE
 ``ContinuousGaussianCRFConv(128, 64, 64, steps=1)`` layer (N=40,960 points, Nc=10,240 coarse points, K=16, Cu=128, Cp=Co=64,
@@ -27,6 +27,17 @@ roofline     : the WHOLE step against SURVEY.md §8(d)'s algorithmic bytes (S1: 
 cpu_baseline / --impl reference: the CPU port of the reference (oracle/layers.py, PyTorch CPU, all host threads) on the SAME
                workload (S1: the same 6 clouds per step; C3-C5: a bounded 2-cloud sample).  The reference itself is Python and is
                not present on the GPU box.
+--dump-outputs DIR: after the timed steps, rank 0 writes what the last timed step returned to its caller as DIR/<name>.npy (float32),
+               so that two builds can be compared output for output on the same seeded inputs.  S1: `out` and `grad_unary` /
+               `grad_pairwise` (a fixed sample of 32,768 of the B x 40,960 point rows, 8,192 of the B x 10,240 coarse rows of
+               `grad_unary`: ≈21 MB whatever B; `out_rows` / `grad_unary_rows` are the sampled row indices into the flattened
+               batch); C3-C5: `loss`.  Both: `grad_params`, the flat fp32 parameter gradient that the step hands to the
+               all-reduce / optimiser (parameters in `module.parameters()` order).  With N > 1 GPUs only rank 0 writes (its own
+               clouds).  Several kernels accumulate with atomics, so two runs of one build agree to fp32 rounding, not bit for bit:
+               compare with a tolerance relative to each array's scale (a gradient that is zero in exact arithmetic, such as the
+               bias of a BatchNorm that feeds another batch-statistics BatchNorm, is rounding noise on its own).
+--steps K    : the number of timed steps of every timed loop (the headline, the e2e arm and --impl reference).  The reference arm
+               runs K full fwd+bwd passes on the CPU (S1: 6 x 40,960 points, seconds each): pass a small K there.
 """
 from __future__ import annotations
 
@@ -238,15 +249,15 @@ def cpu_network_points_per_s(cfg, clouds=2, repeats=2, warm=1):
 def run_reference(args, rank, world):
     if rank != 0:
         return
-    steps = max(args.steps, 1)
+    steps = args.steps
     if args.config == "S1":
-        v, t, cb = cpu_layer_points_per_s(clouds=args.clouds or 6, repeats=max(2, min(steps, 6)), warm=min(max(args.warmup, 1), 2))
+        v, t, cb = cpu_layer_points_per_s(clouds=args.clouds or 6, repeats=steps, warm=min(max(args.warmup, 1), 2))
         workload = (f"single ContinuousGaussianCRFConv(128,64,64,steps=1) fwd+bwd, N=40960, Nc=10240, K=16, {args.clouds or 6} clouds per step "
                     "(the same step as the GPU arm)")
         metric = METRIC
     else:
         cfg = NET_CONFIGS[args.config]
-        v, t, cb = cpu_network_points_per_s(cfg, clouds=2, repeats=max(1, min(steps, 3)), warm=1)
+        v, t, cb = cpu_network_points_per_s(cfg, clouds=2, repeats=steps, warm=1)
         workload = f"PointConvResNet(6,{cfg['classes']},use_crf=True) fwd+CE+bwd, {cfg['name']}; CPU arm: 2 clouds per step (bounded sample)"
         metric = "PointConvResNet fwd+bwd points/s"
     line = {"impl": "reference", "metric": metric, "value": v, "unit": "points/s", "n_gpus": args.gpus,
@@ -326,6 +337,19 @@ def _ncu_traffic(name):
         return None
 
 
+def sample_rows(torch, n, keep, dev):
+    """Sorted fixed sample of `keep` of `n` rows (its own seeded generator: the same rows in every run)."""
+    return torch.randperm(n, generator=torch.Generator(device="cpu").manual_seed(0))[:keep].sort().values.to(dev)
+
+
+def dump_outputs(path, arrays):
+    """Writes every tensor of `arrays` as <path>/<name>.npy in float32."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), t.detach().float().cpu().numpy())
+
+
 def run_gpu(args, rank, local_rank, world):
     import torch
     import torch.distributed as dist
@@ -360,6 +384,13 @@ def run_gpu(args, rank, local_rank, world):
         s["unary"].requires_grad_(True)
         s["pairwise"].requires_grad_(True)
     cot = torch.ones(B, N_POINTS, CP, device=dev)
+    # --dump-outputs: input set -> what a step on it returns to the caller (a replayed graph overwrites the tensors of its capture)
+    results = {}
+
+    def keep(k, out, s):
+        if args.dump_outputs:
+            results[k] = {"out": out, "grad_unary": s["unary"].grad, "grad_pairwise": s["pairwise"].grad,
+                          "grad_params": [p.grad for p in fg.params]}
 
     def eager_step(i, reduce=True):
         s = sets[i % nsets]
@@ -368,6 +399,7 @@ def run_gpu(args, rank, local_rank, world):
         out.backward(cot)
         if reduce:
             fg.all_reduce()                       # no-op at world == 1
+        keep(i % nsets, out, s)
         s["unary"].grad = None
         s["pairwise"].grad = None
 
@@ -392,6 +424,7 @@ def run_gpu(args, rank, local_rank, world):
                 out = layer(s["unary"], s["pairwise"], s["up_idx"], s["neighbor_idx"])
                 out.backward(cot)
             launches_per_step = ops.COUNTERS["launches"]
+            keep(k, out, s)
             s["unary"].grad = None
             s["pairwise"].grad = None
             graphs.append(g)
@@ -420,6 +453,13 @@ def run_gpu(args, rank, local_rank, world):
     ms = _timed(torch, dist, world, dev, step, args.steps, barrier)
     launches = ops.COUNTERS["launches"]
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:                      # before the e2e arm and the profiled step overwrite the gradients
+        last = dict(results[(args.steps - 1) % nsets])
+        rows, urows = sample_rows(torch, B * N_POINTS, 32768, dev), sample_rows(torch, B * (N_POINTS // RATIO), 8192, dev)
+        for name, r in (("out", rows), ("grad_pairwise", rows), ("grad_unary", urows)):
+            last[name] = last[name].reshape(-1, last[name].shape[-1])[r]
+        last["grad_params"] = torch.cat([g.reshape(-1) for g in last["grad_params"]])
+        dump_outputs(args.dump_outputs, {**last, "out_rows": rows, "grad_unary_rows": urows})
     ms_step = ms / args.steps
     value = world * B * N_POINTS / (ms_step * 1e-3)
 
@@ -649,11 +689,13 @@ def run_gpu_network(args, rank, local_rank, world, dev, numa):
     gs = GraphedStep(net_step) if args.graph else None
     launches_per_step = 0
 
+    last = {}
+
     def step(i):
         if gs is not None:
-            gs.replay()
+            last["loss"] = gs.replay()
         else:
-            net_step()
+            last["loss"] = net_step()
         if world > 1:
             grads.all_reduce()
 
@@ -662,8 +704,13 @@ def run_gpu_network(args, rank, local_rank, world, dev, numa):
         sampler.start()
     warm_up(torch, dist, world, dev, step, max(args.warmup, 3), chunk=4)
     barrier()
+    # the classifier's dropout draws a new mask every step and the warm-up ends on a clock: reseeding here gives the timed steps
+    # the same masks in every run
+    torch.cuda.manual_seed(1234)
     ms = _timed(torch, dist, world, dev, step, args.steps, barrier)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:                      # before the eager step below overwrites the gradients
+        dump_outputs(args.dump_outputs, {"loss": last["loss"].reshape(1), "grad_params": grads.flat[:grads.numel]})
     ms_step = ms / args.steps
     value = world * B * N / (ms_step * 1e-3)
     ops.COUNTERS["launches"] = 0
@@ -696,7 +743,7 @@ def run_gpu_network(args, rank, local_rank, world, dev, numa):
 
     for i in range(2):
         e2e_step(i)
-    n_e2e = max(3, min(args.steps, 10))
+    n_e2e = args.steps
     ms_e2e = _timed(torch, dist, world, dev, e2e_step, n_e2e, barrier)
     e2e_value = world * B * N / (ms_e2e / n_e2e * 1e-3)
     if rank != 0:
@@ -731,7 +778,7 @@ def run_gpu_network(args, rank, local_rank, world, dev, numa):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=100)
+    ap.add_argument("--steps", type=int, default=100, help="timed steps (--impl reference runs this many CPU passes: keep it small there)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--config", default="S1", choices=["S1", "C3", "C4", "C5"])
     ap.add_argument("--clouds", type=int, default=0, help="clouds per GPU per step (default: 6 for S1/C3, 8 for C4, 2 for C5)")
@@ -740,7 +787,13 @@ def main():
                     help="e2e arm: narrow the int64 index tensors to 16 bits on the host before the copy (auto: time both forms, keep the faster)")
     ap.add_argument("--pack-threads", type=int, default=0, help="host threads of the index packing (default: min(16, cores per rank - 2); measured 1 / 2 / 4 / 8 / 16 threads: 2.84 / 2.18 / 2.04 / 2.05 / 1.92 ms per step)")
     ap.add_argument("--no-graph", dest="graph", action="store_false", help="launch every kernel from Python instead of replaying CUDA graphs")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write what the last timed step returned as DIR/<name>.npy (float32; S1: a fixed sample of the rows)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the GPU arm")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -752,7 +805,8 @@ def main():
         cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", f"--nproc-per-node={args.gpus}", "--master-addr", "127.0.0.1",
                "--master-port", str(29500 + os.getpid() % 2000), os.path.abspath(__file__), "--gpus", str(args.gpus), "--steps", str(args.steps),
                "--warmup", str(args.warmup), "--config", args.config, "--clouds", str(args.clouds), "--pack-index", args.pack_index,
-               "--pack-threads", str(args.pack_threads)] + ([] if args.graph else ["--no-graph"])
+               "--pack-threads", str(args.pack_threads)] + ([] if args.graph else ["--no-graph"]) \
+            + (["--dump-outputs", args.dump_outputs] if args.dump_outputs else [])
         sys.exit(subprocess.call(cmd))
     run_gpu(args, rank, local_rank, world)
 

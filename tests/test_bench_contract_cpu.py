@@ -33,6 +33,20 @@ def test_product_arm_refuses_to_run_without_a_gpu():
     assert not [l for l in r.stdout.strip().splitlines() if l.startswith("{") and '"value"' in l]
 
 
+def test_dump_outputs_writes_float32_on_fixed_rows(tmp_path):
+    """--dump-outputs: the same sampled rows in every run, every array written as float32; --steps 0 is refused."""
+    import numpy as np
+    import torch
+    sys.path.insert(0, ROOT)
+    import bench
+    rows = bench.sample_rows(torch, 6 * 40960, 32768, "cpu")
+    assert torch.equal(rows, bench.sample_rows(torch, 6 * 40960, 32768, "cpu")) and bool((rows[1:] > rows[:-1]).all())
+    bench.dump_outputs(str(tmp_path), {"loss": torch.tensor([2.5], dtype=torch.float64), "out_rows": rows})
+    assert np.load(tmp_path / "loss.npy").dtype == np.float32 and np.array_equal(np.load(tmp_path / "out_rows.npy"), rows.numpy())
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "0"], capture_output=True, text=True, timeout=600, cwd=ROOT)
+    assert r.returncode != 0 and "--steps" in r.stderr
+
+
 def test_algorithmic_bytes_match_the_survey():
     """SURVEY.md §8(d): 79,298,560 algorithmic bytes per 40,960-point cloud for one CRF layer fwd+bwd at S1 — the roofline numerator."""
     sys.path.insert(0, ROOT)
