@@ -42,6 +42,7 @@ SIGNATURES = {
     "crfconv_linear_bwd": (_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _f32,
                                   _vp, _int, _vp, _vp, _f32, _vp, _i64, _i64, _vp, _int, _vp, _vp, _int, _vp, _int, _vp, _vp, _vp, _i64,
                                   _i64, _int, _int, _vp]),
+    "crfconv_linear_bwd_launches": (_int, []),
     "crfconv_grad_slots_reduce": (_int, [_vp, _vp, _i64, _i64, _vp]),
     "crfconv_relpos": (_int, [_vp, _vp, _vp, _vp, _i64, _i64, _i64, _int, _vp]),
     "crfconv_pointconv_aggregate_fwd": (_int, [_vp, _vp, _vp, _vp, _vp, _vp, _i64, _i64, _i64, _int, _int, _vp]),

@@ -238,18 +238,7 @@ class _CRFConvFunction(torch.autograd.Function):
                 None, None, *_param_grads(ctx.gbuf, [Gc, *grads]))
 
 
-WGRAD_BRANCH = True   # fusion_nn's weight gradient on its own stream / graph branch (fused path)
 PACKED = False         # measured experiment, off (module attribute, no environment switch; steps = 1): mean-field operands {Hy | z} interleaved into 128-byte rows (crf.cu); measured: no gain
-_WGRAD = {}
-
-
-def _wgrad_stream(dev):
-    key = dev.index if dev.index is not None else torch.cuda.current_device()
-    if key not in _WGRAD:
-        _WGRAD[key] = torch.cuda.Stream(device=dev)
-    return _WGRAD[key]
-
-
 _THIRD = {}
 
 
@@ -280,7 +269,7 @@ def fused_eligible(unary, pairwise, neighbor_idx, steps, training, mods, F, Co):
 
 
 class _CRFConvFusedFunction(torch.autograd.Function):
-    """The same layer as _CRFConvFunction on the layer-specialised kernels: 13 launches forward, 15 backward for steps = 1
+    """The same layer as _CRFConvFunction on the layer-specialised kernels: 13 launches forward, 14 backward for steps = 1
     (was 24 + 33), every BatchNorm finalize folded into the producing kernel, out_nn's backward reduced to one pass."""
 
     @staticmethod
@@ -409,19 +398,8 @@ class _CRFConvFusedFunction(torch.autograd.Function):
         dO = torch.empty((M, Co), dtype=torch.float32, device=dev)
         dP = torch.empty((M, Cp), dtype=torch.float32, device=dev)
         main = torch.cuda.current_stream(dev)
-        if WGRAD_BRANCH:
-            # fusion_nn's weight gradient (82 us) feeds nothing but the final fold: it runs on its own graph branch, off the critical path
-            # dOut → dO → out_nn → mean field → pairwise chain
-            wstream = _wgrad_stream(dev)
-            fork_w, join_w = torch.cuda.Event(), torch.cuda.Event()
-            fork_w.record(main)
-            wstream.wait_event(fork_w)
-            with torch.cuda.stream(wstream):
-                ops.linear_bwd(g2, Hf, sf, sl[5], H3, Wf, scale1=so.scale, shift1=so.shift, slope1=sl[4], X2=P, dW=dW["f"], scratch=scr(dW["f"]), scratch_stride=n_small)
-                join_w.record(wstream)
-            ops.linear_bwd(g2, Hf, sf, sl[5], H3, Wf, scale1=so.scale, shift1=so.shift, slope1=sl[4], X2=P, dX1=dO, dX2=dP)
-        else:
-            ops.linear_bwd(g2, Hf, sf, sl[5], H3, Wf, scale1=so.scale, shift1=so.shift, slope1=sl[4], X2=P, dX1=dO, dX2=dP, dW=dW["f"], scratch=scr(dW["f"]), scratch_stride=n_small)
+        # one pass over dY, Hf, H3 and P for both gradients (csrc/linear3b.cu)
+        ops.linear_bwd(g2, Hf, sf, sl[5], H3, Wf, scale1=so.scale, shift1=so.shift, slope1=sl[4], X2=P, dX1=dO, dX2=dP, dW=dW["f"], scratch=scr(dW["f"]), scratch_stride=n_small)
         # out_nn (:74) in one pass over dO
         Q, a0 = torch.empty((F, F), dtype=torch.float32, device=dev), torch.empty(F, dtype=torch.float32, device=dev)
         T = ops.out16_bwd(dO, H3, so, sl[4], xs[-1], Wo, out_part, cnt[1], dg["o"], db["o"], dW["o"], Q, a0)
@@ -474,8 +452,6 @@ class _CRFConvFusedFunction(torch.autograd.Function):
         main.wait_event(join)
         main.wait_event(join3)
         main.wait_event(join_aux)
-        if WGRAD_BRANCH:
-            main.wait_event(join_w)
         ops.grad_slots_reduce(wscr[2 * F * F:], small[2 * F * F:], n_small - 2 * F * F, n_small)   # all weight gradients, one launch
         grads = []
         for k in ("1u", "2u", "1p", "2p", "o", "f"):

@@ -687,6 +687,7 @@ __global__ void __launch_bounds__(kThreads) wgrad_kernel(const WgradArgs a) {
 // take the generic 3xTF32 kernels (≈2^-21), which keeps ill-conditioned tiny batches inside the 1e-3 parity budget.
 // Dispatch between the kernel families is by SHAPE only (no environment switches); the one override is the tests' hook below.
 constexpr int64_t kFastMinRows = 8192;
+static thread_local int t_bwd_launches = 0;   // kernels launched by this thread's last crfconv_linear_bwd call
 static int g_fast_override = -1;   // -1: rule above; 0: never; 1: always (crfconv_set_fast_path: lets the tests reach every family at small sizes)
 inline bool use_fast(int64_t M) {
     if (g_fast_override >= 0) return g_fast_override == 1;
@@ -803,6 +804,8 @@ int crfconv_grad_slots_reduce(const float* scratch, float* dW, int64_t n, int64_
     return CRF_OK;
 }
 
+int crfconv_linear_bwd_launches(void) { return lin::t_bwd_launches; }
+
 // Gradient of crfconv_linear_fwd wrt its (post-prologue) inputs and its weight.  The upstream gradient is given wrt the
 // layer's ACTIVATION output (dY); the BN(+LeakyReLU) backward transform is applied on the fly (scale == NULL ⇒ the layer
 // had no BN: dH = dY).   dX1 / dX2 may be NULL (not needed); acc ⇒ accumulate into the destination.
@@ -812,10 +815,13 @@ int crfconv_linear_bwd(const float* dY, const float* H, const float* act_ref, co
                        int64_t rows_dst, int64_t rows_src, const float* X2, int C2, const float* W, float* dX1, int acc1,
                        float* dX2, int acc2, float* dW, float* dbias, float* dW_scratch, int64_t dW_scratch_stride, int64_t M, int Cout, int precision,
                        void* stream) {
+    lin::t_bwd_launches = 0;
     if (M < 0 || Cout <= 0 || C1 < 0 || C2 < 0 || C1 + C2 <= 0 || !dY || !W) return CRF_ERR_INVALID_ARG;
     if (M == 0) return CRF_OK;
     if (scale && (Cout & 3)) return CRF_ERR_UNSUPPORTED;
     cudaStream_t st = (cudaStream_t)stream;
+    const int n_reduce = (dW && dW_scratch && dW_scratch_stride <= 0) ? 1 : 0;
+    lin::t_bwd_launches = int(dX1 || dX2) + int(dW != nullptr) + n_reduce;     // one kernel each, unless a one-pass kernel takes both
     lin::BnBwd bn{scale, shift, mean, invstd, k1, k2, act_ref, slope};
     const int Ktot = C1 + C2;
     const int gprec = precision == 2 ? 1 : precision;    // precision seen by the generic (TF32) kernels
@@ -833,7 +839,14 @@ int crfconv_linear_bwd(const float* dY, const float* H, const float* act_ref, co
         lin::DgradArgs d{dY, H, bn, W, dX1, C1, acc1, dX2, C2, acc2, M, Cout};
         lin::WgradArgs w{dY, H, bn, X1, C1, scale1, shift1, slope1, idx1, rows_dst, rows_src, X2, C2, wdst, dbias, M, Cout, 0, wstride};
         int rc2 = CRF_OK;
-        if (lin::try_narrow_bwd(d, dW ? &w : nullptr, st, &rc2)) return rc2 != CRF_OK ? rc2 : reduce_slots();
+        if (dW && lin::try_bwd3(d, w, precision, st, &rc2)) {
+            lin::t_bwd_launches = 1 + n_reduce;
+            return rc2 != CRF_OK ? rc2 : reduce_slots();
+        }
+        if (lin::try_narrow_bwd(d, dW ? &w : nullptr, st, &rc2)) {
+            lin::t_bwd_launches = 1 + n_reduce;
+            return rc2 != CRF_OK ? rc2 : reduce_slots();
+        }
     }
     if (dX1 || dX2) {
         // with idx1, dX1 is the gradient wrt the GATHERED rows [M, C1]; scatter it with crfconv_scatter_add_rows

@@ -60,6 +60,8 @@ bool try_wgrad2(const WgradArgs& a, int precision, cudaStream_t st, int* rc);
 bool try_fwd3(const FwdArgs& a, int precision, cudaStream_t st, int* rc);
 bool try_wgrad3(const WgradArgs& a, int precision, cudaStream_t st, int* rc);   // linear3w.cu
 bool try_dgrad3(const DgradArgs& a, int precision, cudaStream_t st, int* rc);   // linear3d.cu
+// input and weight gradient in one pass (linear3b.cu); needs dW and at least one of dX1 / dX2
+bool try_bwd3(const DgradArgs& d, const WgradArgs& w, int precision, cudaStream_t st, int* rc);
 // narrow layers over many rows: operands straight from global memory in fragment order (linear_direct.cu)
 bool try_wgrad_direct(const WgradArgs& a, cudaStream_t st, int* rc);
 bool try_upproj_fwd(const FwdArgs& a, cudaStream_t st, int* rc);      // narrow input → wide output (output-bound streams)

@@ -55,6 +55,15 @@ __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
 __device__ __forceinline__ void mbar_wait_relaxed(uint64_t* bar, uint32_t parity) {
     if (!mbar_try_wait(bar, parity)) mbar_wait_slow(bar, parity, 40);
 }
+// Same bound, inline and without the printf: no call site, so a warp that keeps many registers live across the wait does not
+// spill them around a call (the trap still surfaces as a CUDA error).
+__device__ __forceinline__ void mbar_wait_relaxed_nocall(uint64_t* bar, uint32_t parity) {
+    const long long t0 = clock64();
+    while (!mbar_try_wait(bar, parity)) {
+        __nanosleep(40);
+        if (clock64() - t0 > 4000000000LL) __trap();
+    }
+}
 
 // one lane of a converged warp; unlike `lane == 0` the compiler knows the region is single-threaded and issues tcgen05
 // instructions without a per-instruction election loop

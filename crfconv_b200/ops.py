@@ -261,10 +261,11 @@ def linear_bwd(dY, H, bn, slope, X1, W, *, scale1=None, shift1=None, slope1=1.0,
     nb = _nbytes(dY, H if b else None, act_ref, X1 if dW is not None else None, X2 if dW is not None else None, dX1, dX2,
                  dX1 if acc1 else None, dX2 if acc2 else None)
     with _call(f"linear_bwd[{Cout}<-{C1 + C2}]" + ("" if dW is not None else ":dgrad") + ("" if (dX1 is not None or dX2 is not None) else ":wgrad"),
-               int(dW is not None) + int(scratch is not None and scratch_stride == 0) + int(dX1 is not None or dX2 is not None), nb):
+               0, nb):
         rc = _linear_bwd_call(L, dY, H, act_ref, b, slope, X1, C1, scale1, shift1, slope1, idx1, rows_dst, rows_src, X2, C2, W, dX1, acc1,
                               dX2, acc2, dW, dbias, scratch, scratch_stride, M, Cout)
     _lib.check(rc, "linear_bwd")
+    COUNTERS["launches"] += L.crfconv_linear_bwd_launches()     # the input and weight gradient may share one kernel
 
 
 def _linear_bwd_call(L, dY, H, act_ref, b, slope, X1, C1, scale1, shift1, slope1, idx1, rows_dst, rows_src, X2, C2, W, dX1, acc1, dX2, acc2,

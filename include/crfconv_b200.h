@@ -135,6 +135,8 @@ int crfconv_linear_bwd(const float* dY, const float* H, const float* act_ref, co
                        int64_t rows_dst, int64_t rows_src, const float* X2, int C2, const float* W, float* dX1, int acc1,
                        float* dX2, int acc2, float* dW, float* dbias, float* dW_scratch, int64_t dW_scratch_stride, int64_t M, int Cout,
                        int precision, void* stream);
+/* Number of kernels the calling thread's last crfconv_linear_bwd call launched (input and weight gradient may share one). */
+int crfconv_linear_bwd_launches(void);
 /* dW[i] += Σ_slots scratch[slot·stride + i] for i < n.  With dW_scratch_stride > 0 crfconv_linear_bwd only accumulates into the
  * slots (slot pitch = stride floats) and the caller folds all layers that share one flat gradient layout with ONE call here. */
 int crfconv_grad_slots_reduce(const float* scratch, float* dW, int64_t n, int64_t stride, void* stream);

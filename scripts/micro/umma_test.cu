@@ -433,7 +433,93 @@ static void run_mn() {
     cudaFree(dA); cudaFree(dB); cudaFree(dD);
 }
 
+
+// ---- mixed majors: D[128, N] = Σ_k A[k][m] · B[n][k], A MN-major BASE32B (lines = k), B K-major (lines = n), instruction-descriptor
+// bit 15 only.  This is the input-gradient product of csrc/linear3b.cu (A = Wᵀ, lines = output channels; B = dH, lines = rows).
+// B is in K-major SWIZZLE_128B slabs (16-byte chunk c of line n at c ^ (n & 7), SBO = 1024 B).  Inputs are tf32-representable: exact.
+template <int N, int K>
+__global__ void __launch_bounds__(128) umma_mixed_kernel(const float* __restrict__ A, const float* __restrict__ B, float* __restrict__ D) {
+    extern __shared__ __align__(1024) uint8_t smem_dyn[];
+    constexpr int ASLAB = K * 128, BSLAB = N * 128;
+    uint8_t* a_s = smem_dyn;                       // [4 channel blocks][K lines × 128 B]
+    uint8_t* b_s = smem_dyn + 4 * ASLAB;           // [K / 32 slabs][N lines × 128 B]
+    __shared__ uint64_t bar;
+    __shared__ uint32_t tmem_base;
+    const int tid = threadIdx.x, warp = tid >> 5;
+    if (warp == 0) {
+        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&tmem_base)), "r"(64));
+        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::);
+    }
+    if (tid == 0) { mbar_init(&bar, 1); asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory"); }
+    for (int i = tid; i < K * 128; i += 128) {     // A is [K][128] row-major in global
+        const int k = i / 128, m = i % 128;
+        *(float*)(a_s + (m / 32) * ASLAB + sw32_off(k, m % 32)) = A[i];
+    }
+    for (int i = tid; i < N * K; i += 128) {       // B is [N][K] row-major in global
+        const int n = i / K, k = i % K;
+        *(float*)(b_s + (k / 32) * BSLAB + sw128_off(n, k % 32)) = B[i];
+    }
+    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    __syncthreads();
+    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+    const uint32_t tmem = tmem_base;
+    if (warp == 1) {
+        if (elect_one()) {
+            constexpr uint32_t idesc = make_idesc(128, N) | (1u << 15);                // A MN-major, B K-major
+            for (int k8 = 0; k8 < K / 8; ++k8) {
+                const uint64_t bdesc = make_desc(smem_u32(b_s) + (k8 / 4) * BSLAB + (k8 % 4) * 32);
+                umma_tf32(tmem, make_desc_mn(smem_u32(a_s) + k8 * 1024, ASLAB), bdesc, idesc, k8 > 0);
+            }
+            umma_commit(&bar);
+        }
+        __syncwarp();
+    }
+    mbar_wait_bounded(&bar, 0);
+    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+    const int row = warp * 32 + (tid & 31);
+    for (int c = 0; c < N; c += 16) {
+        float v[16];
+        tmem_ld16(tmem + ((uint32_t)(warp * 32) << 16) + c, v);
+        for (int i = 0; i < 16; ++i) D[row * N + c + i] = v[i];
+    }
+    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    __syncthreads();
+    if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(64));
+}
+template <int N, int K>
+static int run_mixed() {
+    std::vector<float> A(K * 128), B(N * K), D(128 * N, -1.f), ref(128 * N);
+    srand(11);
+    for (auto& x : A) x = (float)((rand() % 17) - 8) * 0.25f;
+    for (auto& x : B) x = (float)((rand() % 17) - 8) * 0.5f;
+    for (int m = 0; m < 128; ++m)
+        for (int n = 0; n < N; ++n) {
+            double s = 0;
+            for (int k = 0; k < K; ++k) s += (double)A[k * 128 + m] * (double)B[n * K + k];
+            ref[m * N + n] = (float)s;
+        }
+    float *dA, *dB, *dD;
+    cudaMalloc(&dA, A.size() * 4); cudaMalloc(&dB, B.size() * 4); cudaMalloc(&dD, D.size() * 4);
+    cudaMemcpy(dA, A.data(), A.size() * 4, cudaMemcpyHostToDevice);
+    cudaMemcpy(dB, B.data(), B.size() * 4, cudaMemcpyHostToDevice);
+    cudaMemcpy(dD, D.data(), D.size() * 4, cudaMemcpyHostToDevice);
+    const size_t smem = (size_t)4 * K * 128 + (size_t)(K / 32) * N * 128;
+    auto kern = umma_mixed_kernel<N, K>;
+    cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    kern<<<1, 128, smem>>>(dA, dB, dD);
+    cudaError_t e = cudaDeviceSynchronize();
+    cudaMemcpy(D.data(), dD, D.size() * 4, cudaMemcpyDeviceToHost);
+    double err = 0;
+    for (int i = 0; i < 128 * N; ++i) err = fmax(err, fabs((double)D[i] - (double)ref[i]));
+    printf("mixed majors (A MN-major BASE32B, B K-major SWIZZLE_128B) M=128 N=%d K=%d: max|err| = %.3e  %s  %s\n", N, K, err,
+           err == 0.0 ? "EXACT" : "WRONG", e == cudaSuccess ? "" : cudaGetErrorString(e));
+    cudaFree(dA); cudaFree(dB); cudaFree(dD);
+    return e == cudaSuccess ? 0 : 1;
+}
+
 int main() {
+    if (run_mixed<32, 64>()) return 1;
     run_mn<128, 64, 64>();
 
     loop_rate<64, 2, 0>(); loop_rate<64, 4, 0>(); loop_rate<64, 2, 7>(); loop_rate<64, 4, 7>();

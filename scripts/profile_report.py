@@ -165,7 +165,8 @@ def metrics_csv(path, out_json=None, skip_prefixes=("at::", "knn::")):
         call_of = {"cl::step_bwd_kernel": "crf_step_bwd_fused", "mf::step_fwd_kernel<16>": "crf_step_fwd[16]", "cl::out_bwd_kernel": "out16_bwd",
                    "lin3::fwd3_kernel<64>": "linear_fwd_bn[128->64]", "cl::up16_fwd_kernel<64>": "up16_fwd[64]",
                    "lin::bn_bwd_reduce_kernel": "bn_bwd_reduce_fin[64]", "lin3d::dgrad3_kernel<128>": "linear_bwd[64<-128]:dgrad",
-                   "lin3w::wgrad3_kernel<64>": "linear_bwd[64<-128]:wgrad", "lin::bn_act_fwd_kernel": "bn_act_fwd[64]"}
+                   "lin3w::wgrad3_kernel<64>": "linear_bwd[64<-128]:wgrad", "lin3b::bwd3_kernel": "linear_bwd[64<-128]",
+                   "lin::bn_act_fwd_kernel": "bn_act_fwd[64]"}
         calls = {}
         for t in keep:
             for kname, label in call_of.items():

@@ -97,7 +97,9 @@ timeit("  bn_backward_prepare[64] (2 launches)", lambda: ops.bn_backward_prepare
 dO, dP = torch.empty(M, Co, device=dev), torch.empty(M, Co, device=dev)
 dWf = torch.zeros(Co, 2 * Co, device=dev)
 scr = torch.zeros(ops.GRAD_SLOTS * 20000, device=dev)
-timeit("linear_bwd[64<-128] dgrad3+wgrad3", lambda: ops.linear_bwd(g2, Hf, bf, 0.1, H3, Wf, scale1=b3.scale, shift1=b3.shift, slope1=0.1, X2=P, dX1=dO, dX2=dP, dW=dWf, scratch=scr, scratch_stride=20000), fb * M * (2 * Co + 2 * Co + 2 * Co))
+timeit("linear_bwd[64<-128] one pass (bwd3)", lambda: ops.linear_bwd(g2, Hf, bf, 0.1, H3, Wf, scale1=b3.scale, shift1=b3.shift, slope1=0.1, X2=P, dX1=dO, dX2=dP, dW=dWf, scratch=scr, scratch_stride=20000), fb * M * (2 * Co + 2 * Co + 2 * Co))
+timeit("  dgrad3 + wgrad3 (two calls)", lambda: (ops.linear_bwd(g2, Hf, bf, 0.1, H3, Wf, scale1=b3.scale, shift1=b3.shift, slope1=0.1, X2=P, dX1=dO, dX2=dP),
+                                                ops.linear_bwd(g2, Hf, bf, 0.1, H3, Wf, scale1=b3.scale, shift1=b3.shift, slope1=0.1, X2=P, dW=dWf, scratch=scr, scratch_stride=20000)), fb * M * (2 * Co + 2 * Co + 2 * Co))
 timeit("  dgrad only", lambda: ops.linear_bwd(g2, Hf, bf, 0.1, H3, Wf, scale1=b3.scale, shift1=b3.shift, slope1=0.1, X2=P, dX1=dO, dX2=dP), fb * M * 4 * Co)
 timeit("  wgrad only", lambda: ops.linear_bwd(g2, Hf, bf, 0.1, H3, Wf, scale1=b3.scale, shift1=b3.shift, slope1=0.1, X2=P, dW=dWf, scratch=scr, scratch_stride=20000), fb * M * 4 * Co)
 opart = torch.zeros(ops.out_bwd_part_floats(), device=dev)
