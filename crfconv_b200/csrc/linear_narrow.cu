@@ -6,8 +6,11 @@
 // thread streams its row from shared memory (conflict-free float4 reads, stride ≡ 4 mod 32) against a weight matrix that
 // every lane reads at the same address (broadcast), and accumulates in exact fp32 FFMA — no tf32/bf16 rounding at all.
 // 2-3 CTAs per SM overlap one CTA's copy with another's math (no ring needed: compute per tile is short).
-//   narrow_fwd : Y = [lrelu(X1*sc+sh) | X2]·Wᵀ (+bias), Σ/Σ² epilogue                      (Cout <= 64 if Cin <= 16, else Cout <= 16)
-//   narrow_bwd : dH on the fly; dX = dH·W (split into the two segments, optional +=); dW += dHᵀ·A   (same shapes)
+//   narrow_fwd : Y = [lrelu(X1*sc+sh) | X2]·Wᵀ (+bias), Σ/Σ² epilogue
+//   narrow_bwd : dH on the fly; dX = dH·W (split into the two segments, optional +=); dW += dHᵀ·A
+// The templates are written for Cout <= 64 if Cin <= 16, else Cout <= 16, but the dispatch (narrow_shape below) sends them only
+// Cout <= 16 AND C1 + C2 <= 16, every count a multiple of 4, no dbias; at >= 8,192 rows, and the forward only when the tcgen05
+// kernel turns the call down (gathered rows, slope1 outside [0, 1]).
 #include <algorithm>
 #include <cstdlib>
 #include <type_traits>

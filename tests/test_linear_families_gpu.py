@@ -1,0 +1,591 @@
+"""Contract tests of every Linear GEMM kernel family (csrc/linear*.cu) behind crfconv_linear_fwd / crfconv_linear_bwd /
+crfconv_linear_fwd_bn.  Those entry points give a call to the first family whose `try_*` predicate accepts it, so a test that
+only chooses a shape can pass while the kernel it was written for never runs.  Every case below therefore names the GEMM
+kernel(s) it must launch and asserts that set through the CUDA profiler before it checks a single number.
+
+The cases sit on both sides of each family's boundaries (rows 8,191 / 8,192 / 8,193 and near 245,760; channel counts at
+16 / 32 / 64 / 128 ± 4; four vs five 32-channel chunks; padded segments) and combine the options each family accepts.
+
+Checks, each against an fp64 torch statement of the formula built from the same fp32 inputs:
+* every output column, statistics column and weight-gradient row against its OWN maximum (W's output channels, H's and dY's
+  columns are scaled over 1e-2 .. 1e2, so an error confined to the small channels is not hidden by the large ones);
+* outputs that are overwritten are prefilled with NaN, accumulated ones with random values (the check is on the sum);
+* every output carries 64 guard rows (a guard tail for dW, dbias and the statistics) that must keep their sentinel;
+* the backward inputs are built directly, with every V = H·scale + shift at least 1e-3 away from the LeakyReLU kink, so the
+  kernel and the reference cannot take different branches and the bars can be strict.
+Bars: 2e-4 for the two bf16x3 kernels (dgrad2, wgrad2), 2e-5 for everything else (3xTF32 and exact-fp32 CUDA-core kernels).
+The single-pass TF32 cases (ops.PRECISION = 1) must FAIL the 3xTF32 bar, which shows the bar discriminates.
+Run with `-s` to see the worst error per kernel family."""
+import math
+import re
+import zlib
+from dataclasses import dataclass
+from typing import Optional
+
+import pytest
+import torch
+
+pytestmark = pytest.mark.gpu
+
+GUARD = 64                    # extra rows behind every output
+BAR_X3 = 2e-5                 # 3xTF32 and exact fp32
+BAR_BF16X3 = 2e-4             # bf16x3 (dgrad2, wgrad2)
+BAR_BN_FINALIZE = 1e-4        # statistics → mean / invstd / scale / shift / running statistics
+BF16_FWD_L2, BF16_GRAD_L2 = 2e-2, 2e-1    # DESIGN.md §5: single-pass bf16, relative L2
+KINK = 1e-3                   # |V| below this is moved away from the LeakyReLU kink
+
+FWD_KERNELS = ("lin::fwd_kernel", "narrow::fwd_kernel", "lin2::fwd2t_kernel", "lin2::fwd2_kernel", "lin3::fwd3_kernel",
+               "lin::sm::fwd_small_kernel", "lin::up::upproj_kernel")
+DGRAD_KERNELS = ("lin::dgrad_kernel", "lin2::dgrad2_kernel", "lin3d::dgrad3_kernel", "lin::sm::dgrad_small_kernel",
+                 "lin::up::upproj_kernel")
+WGRAD_KERNELS = ("lin::wgrad_tiny_kernel", "lin3w::wgrad3_kernel", "lin2::wgrad2_kernel", "lin2::wgrad_small_kernel",
+                 "lin::dw::wgrad_direct_kernel", "lin::sm::wgrad_rows_kernel", "lin::wgrad_kernel")
+BOTH_KERNELS = ("lin3b::bwd3_kernel", "narrow::bwd_kernel")          # input and weight gradient in one kernel
+GEMM_KERNELS = tuple(dict.fromkeys(FWD_KERNELS + DGRAD_KERNELS + WGRAD_KERNELS + BOTH_KERNELS))
+UTILITY_KERNELS = ("lin::bn_finalize_fwd_kernel", "lin::grad_slots_reduce_kernel")   # may run beside a GEMM in one call
+BF16X3 = ("lin2::dgrad2_kernel", "lin2::wgrad2_kernel")
+
+
+def bar(kernel):
+    return BAR_BF16X3 if kernel in BF16X3 else BAR_X3
+
+
+# ------------------------------------------------------------------------------------------------------------- case table
+@dataclass(frozen=True)
+class Fwd:
+    """crfconv_linear_fwd: Y = [lrelu(X1[idx]·sc + sh, slope1) | X2]·Wᵀ (+ bias), Σ / Σ² of Y into slotted statistics."""
+    name: str
+    M: int
+    C1: int
+    C2: int
+    Cout: int
+    kernels: tuple
+    slope1: Optional[float] = 0.1   # None: no prologue
+    gather: bool = False            # X1 rows gathered through idx1 from 3 clouds (M = 3·rows_dst)
+    bias: bool = False
+    stats: bool = True
+    prec: int = 0                   # ops.PRECISION
+
+
+@dataclass(frozen=True)
+class FwdBn:
+    """crfconv_linear_fwd_bn: the forward plus the training-mode BatchNorm finalize (running statistics included)."""
+    name: str
+    M: int
+    C1: int
+    C2: int
+    Cout: int
+    kernels: tuple
+    slope1: Optional[float] = 0.1
+    prec: int = 0
+
+
+@dataclass(frozen=True)
+class Bwd:
+    """crfconv_linear_bwd.  mode: "bn" = BatchNorm + LeakyReLU(0.1), "act" = LeakyReLU(0.1) without BatchNorm (k1 = k2 = 0,
+    identity affine), "plain" = plain Linear (dH = dY).  dx1 / dx2: None (not requested), "new" (overwrite), "acc" (+=).
+    dw: None, "auto" (ops.linear_bwd picks its partial slots or direct atomics) or "stride" (the caller's slots, stride > 0)."""
+    name: str
+    M: int
+    C1: int
+    C2: int
+    Cout: int
+    kernels: tuple
+    mode: str = "bn"
+    act_ref: bool = False
+    gather: bool = False
+    slope1: Optional[float] = 0.1
+    dx1: Optional[str] = "new"
+    dx2: Optional[str] = "new"
+    dw: Optional[str] = "auto"
+    dbias: bool = False
+    prec: int = 0
+
+
+F3, NF, F2T, F2, FSM, UP, FG = FWD_KERNELS[4], FWD_KERNELS[1], FWD_KERNELS[2], FWD_KERNELS[3], FWD_KERNELS[5], FWD_KERNELS[6], FWD_KERNELS[0]
+DG, DG2, DG3, DGS = DGRAD_KERNELS[:4]
+WT, WG3, WG2, WGS, WD, WR, WG = WGRAD_KERNELS
+B3, NB = BOTH_KERNELS
+FIN, RED = UTILITY_KERNELS
+
+FWD_CASES = [
+    # tcgen05 forward: M >= 8,192, Cout <= 64, <= 4 chunks of 32 input channels, no gather, slope1 in [0, 1]
+    Fwd("fwd3_64+64to64_M8192", 8192, 64, 64, 64, (F3,)),
+    Fwd("fwd3_128to60_M8193_slope0_bias", 8193, 128, 0, 60, (F3,), slope1=0.0, bias=True),
+    Fwd("fwd3_64+64to64_M245759_slope1", 245759, 64, 64, 64, (F3,), slope1=1.0),
+    Fwd("fwd3_36+44to16_padded_bias", 9000, 36, 44, 16, (F3,), bias=True),
+    Fwd("fwd3_96+32to32_4chunks_noprologue", 8192, 96, 32, 32, (F3,), slope1=None),
+    Fwd("fwd3_16to16_hidden", 8193, 16, 0, 16, (F3,)),
+    Fwd("fwd3_12to20_bias_nostats", 20000, 12, 0, 20, (F3,), bias=True, stats=False),
+    # the same shape one row below the fast-path threshold
+    Fwd("fwd_small_64+64to64_M8191", 8191, 64, 64, 64, (FSM,)),
+    # persistent cp.async forward: what fwd3 turns down (gather, slope1 outside [0, 1], 5 chunks)
+    Fwd("fwd2t_gather_32+32to32", 3 * 2731, 32, 32, 32, (F2T,), gather=True),
+    Fwd("fwd2t_100+28to64_5chunks_bias", 9000, 100, 28, 64, (F2T,), bias=True),
+    Fwd("fwd2t_64to48_slope1.5", 8192, 64, 0, 48, (F2T,), slope1=1.5),
+    Fwd("fwd2t_gather_16to20", 3 * 2731, 16, 0, 20, (F2T,), gather=True),
+    Fwd("fwd2t_gather_20to16", 3 * 2731, 20, 0, 16, (F2T,), gather=True, bias=True),
+    # CUDA-core narrow forward: Cout <= 16 and C1 + C2 <= 16, reached through a gather or a slope fwd3 turns down
+    Fwd("narrow_gather_12+4to16_bias", 3 * 2731, 12, 4, 16, (NF,), gather=True, bias=True),
+    Fwd("narrow_gather_8to4_M245757", 3 * 81919, 8, 0, 4, (NF,), gather=True),
+    Fwd("narrow_16to16_slope-0.25", 8192, 16, 0, 16, (NF,), slope1=-0.25),
+    # few rows, wide channels
+    Fwd("fwd_small_gather_64to68", 3 * 2731, 64, 0, 68, (FSM,), gather=True),
+    Fwd("fwd_small_32to132_M8192", 8192, 32, 0, 132, (FSM,)),
+    Fwd("fwd_small_256+256to128_M3841", 3841, 256, 256, 128, (FSM,), bias=True),
+    # up-projection: narrow plain input, wide output
+    Fwd("upproj_32to128_bias_M20001", 20001, 32, 0, 128, (UP,), bias=True),
+    Fwd("upproj_6to32_noprologue", 8193, 6, 0, 32, (UP,), slope1=None, bias=True),
+    # generic 128-row tiles
+    Fwd("generic_128to13_head_bias", 30001, 128, 0, 13, (FG,), slope1=None, bias=True),
+    Fwd("generic_16+16to16_M8191", 8191, 16, 16, 16, (FG,)),
+    Fwd("generic_gather_16to16_M8190", 3 * 2730, 16, 0, 16, (FG,), gather=True),
+    Fwd("generic_gather_128+4to32_M40002", 3 * 13334, 128, 4, 32, (FG,), gather=True),
+]
+
+FWDBN_CASES = [
+    # fused finalize in fwd3's tail: Cout in {16, 32, 64} only
+    FwdBn("fwd3fin_64+64to32", 9000, 64, 64, 32, (F3,)),
+    FwdBn("fwd3fin_16to16_M8193", 8193, 16, 0, 16, (F3,)),
+    FwdBn("fwd3fin_128to64_M245759", 245759, 128, 0, 64, (F3,), slope1=None),
+    FwdBn("fwd3_then_finalize_48", 9000, 64, 0, 48, (F3, FIN)),
+    FwdBn("fwd_small_then_finalize_M8191", 8191, 64, 0, 32, (FSM, FIN)),
+]
+
+BWD_CASES = [
+    # tcgen05 one-pass input + weight gradient: dW and dX, 32 < Cout <= 64, 64 < C1 + C2 <= 128, no gather / dbias / act_ref
+    Bwd("bwd3_64+64to64_M8192_acc2", 8192, 64, 64, 64, (B3,), dx2="acc"),
+    Bwd("bwd3_128to36_M245759_acc1_stride", 245759, 128, 0, 36, (B3,), dx1="acc", dw="stride"),
+    Bwd("bwd3_36+44to40_plain_dx1none", 9001, 36, 44, 40, (B3,), mode="plain", dx1=None),
+    Bwd("bwd3_68to64_act", 8193, 64, 4, 64, (B3,), mode="act", slope1=None),
+    # just outside bwd3
+    Bwd("dgrad3+wgrad2_100+28to64_5chunks", 9000, 100, 28, 64, (DG3, WG2)),
+    Bwd("dgrad3+wgrad2_gather_64+64to64", 3 * 2731, 64, 64, 64, (DG3, WG2), gather=True),
+    Bwd("dgrad3+generic_wgrad_plain_dbias", 8192, 64, 64, 64, (DG3, WG), mode="plain", dbias=True),
+    Bwd("dgrad2+wgrad2_actref_64+64to64", 8192, 64, 64, 64, (DG2, WG2), act_ref=True),
+    Bwd("dgrad_small+wgrad_rows_64+64to64_M8191", 8191, 64, 64, 64, (DGS, WR)),
+    Bwd("dgrad_small+wgrad_rows_64+64to68", 9000, 64, 64, 68, (DGS, WR)),
+    Bwd("generic_128+4to32_M40000", 40000, 128, 4, 32, (DG, WG)),
+    # input gradient only / weight gradient only
+    Bwd("dgrad3_only_dx1none_acc2", 20000, 64, 64, 64, (DG3,), dx1=None, dx2="acc", dw=None),
+    Bwd("wgrad3_only_128to64_stride", 20000, 128, 0, 64, (WG3,), dx1=None, dw="stride"),
+    Bwd("wgrad3_only_64+4to16", 8192, 64, 4, 16, (WG3,), dx1=None, dx2=None),
+    Bwd("wgrad2_only_32+32to64", 8192, 32, 32, 64, (WG2,), dx1=None, dx2=None),
+    # bf16x3 family
+    Bwd("dgrad2_only_32+32to32_acc2", 8193, 32, 32, 32, (DG2,), dw=None, dx2="acc"),
+    Bwd("dgrad2+wgrad2_64to16_M30000_slots", 30000, 64, 0, 16, (DG2, WG2, RED)),
+    Bwd("dgrad2+wgrad_direct_32to16_hole", 8192, 32, 0, 16, (DG2, WD, RED)),
+    Bwd("wgrad_direct_only_16to32_hole", 8192, 16, 0, 32, (WD, RED), dx1=None, mode="plain"),
+    Bwd("generic_wgrad_only_actref_16to32", 8192, 16, 0, 32, (WG, RED), dx1=None, act_ref=True),
+    Bwd("dgrad2+wgrad_small_32to32", 8193, 32, 0, 32, (DG2, WGS, RED)),
+    Bwd("dgrad2+wgrad_small_actref_32to32_stride", 8192, 32, 0, 32, (DG2, WGS), act_ref=True, dw="stride"),
+    Bwd("dgrad2+wgrad2_16+16to32", 8192, 16, 16, 32, (DG2, WG2, RED)),
+    # CUDA-core narrow backward: Cout <= 16 and C1 + C2 <= 16, input and weight gradient in one kernel
+    Bwd("narrow_gather_12+4to16_acc2", 3 * 2731, 12, 4, 16, (NB, RED), gather=True, dx2="acc"),
+    Bwd("narrow_act_8to8_acc1_stride", 8192, 8, 0, 8, (NB,), mode="act", dx1="acc", dw="stride"),
+    Bwd("narrow_wgrad_only_actref_16to16", 8192, 16, 0, 16, (NB, RED), act_ref=True, dx1=None),
+    Bwd("narrow_dgrad_only_8+8to16_dx1none", 245759, 8, 8, 16, (NB,), dx1=None, dw=None),
+    Bwd("dgrad2+wgrad_direct_16to20_plain", 8192, 16, 0, 20, (DG2, WD, RED), mode="plain"),
+    Bwd("dgrad2+wgrad_direct_16to16_dbias", 8192, 16, 0, 16, (DG2, WD, RED), mode="plain", dbias=True),
+    Bwd("generic_dgrad+wgrad_direct_16to16_M8191", 8191, 16, 0, 16, (DG, WD, RED)),
+    # relative positions: C1 <= 4
+    Bwd("wgrad_tiny_3to64_M245759", 245759, 3, 0, 64, (WT, RED), dx1=None),
+    Bwd("wgrad_tiny+generic_dgrad_gather_4to32_plain", 3 * 2731, 4, 0, 32, (DG, WT, RED), mode="plain", gather=True, slope1=None),
+    Bwd("wgrad_tiny_actref_3to16", 8192, 3, 0, 16, (WT, RED), act_ref=True, dx1=None),
+    Bwd("wgrad_direct_5to32", 8192, 5, 0, 32, (WD, RED), dx1=None),
+    Bwd("wgrad_direct_3to13_dbias", 8192, 3, 0, 13, (WD, RED), mode="plain", dx1=None, dbias=True),
+    # narrow layers over many rows / few rows
+    Bwd("wgrad_direct_128to13_dbias_M50001", 50001, 128, 0, 13, (WD,), mode="plain", dx1=None, dbias=True, slope1=None),
+    Bwd("wgrad_direct_32to64_M5000_stride", 5000, 32, 0, 64, (WD,), dx1=None, dw="stride"),
+    Bwd("dgrad_small+wgrad_rows_gather_512to256_M960", 3 * 320, 512, 0, 256, (DGS, WR), gather=True),
+    Bwd("dgrad_small+wgrad_rows_actref_64+64to64_M3000", 3000, 64, 64, 64, (DGS, WR), act_ref=True),
+    # the class head's input gradient
+    Bwd("upproj_dgrad_128to13", 8192, 128, 0, 13, (UP,), mode="plain", dw=None, slope1=None),
+    Bwd("generic_dgrad_128to13_acc1", 8192, 128, 0, 13, (DG,), mode="plain", dw=None, dx1="acc", slope1=None),
+]
+
+# Single-pass TF32 (ops.PRECISION = 1) sends these to the generic kernels, which must then miss the 3xTF32 bar.
+TF32_CASES = [
+    Fwd("tf32_fwd_64+64to64", 9000, 64, 64, 64, (FG,), prec=1),
+    Fwd("tf32_fwd_32to128", 20000, 32, 0, 128, (FG,), prec=1),
+    Bwd("tf32_bwd_64+64to64", 9000, 64, 64, 64, (DG, WG), prec=1),
+    Bwd("tf32_bwd_32to32_plain", 20000, 32, 0, 32, (DG, WG, RED), mode="plain", prec=1, dx2=None),
+]
+
+# Single-pass bf16 (ops.PRECISION = 2): the only way to reach fwd2_kernel.
+BF16_CASES = [
+    Fwd("bf16_fwd2_64to32", 9000, 64, 0, 32, (F2,), prec=2),
+    Fwd("bf16_fwd2_32+32to64_bias", 8193, 32, 32, 64, (F2,), prec=2, bias=True),
+    Bwd("bf16_dgrad2+wgrad2_32+32to32", 9000, 32, 32, 32, (DG2, WG2), prec=2),
+]
+
+CASES = FWD_CASES + FWDBN_CASES + BWD_CASES + TF32_CASES + BF16_CASES
+
+
+# ------------------------------------------------------------------------------------------------------------- helpers
+@pytest.fixture(scope="module")
+def ops():
+    from crfconv_b200 import ops as o
+    return o
+
+
+WORST = {}      # kernel -> (worst error, case)
+
+
+@pytest.fixture(scope="module", autouse=True)
+def _worst_table():
+    yield
+    if WORST:
+        print("\nworst error per kernel family (each column / row against its own maximum):")
+        for k in sorted(WORST):
+            e, c = WORST[k]
+            print(f"  {k:32s} {e:9.2e}  bar {bar(k):.0e}  ({c})")
+
+
+def _record(kernel, err, case):
+    if kernel not in WORST or err > WORST[kernel][0]:
+        WORST[kernel] = (err, case)
+
+
+_MANGLED = re.compile(r"(\d+)")
+
+
+def _qualified(name):
+    """'crf::'-relative qualified function name of a profiler kernel record, or None for other kernels."""
+    m = re.search(r"crf::((?:\w+::)*\w+_kernel)\b", name)
+    if m:
+        return m.group(1)
+    if name.startswith("_ZN3crf"):                      # not demangled: walk the <length><identifier> components
+        s, i, parts = name[3:], 0, []
+        while i < len(s) and s[i].isdigit():
+            n = _MANGLED.match(s, i).group(1)
+            i += len(n)
+            parts.append(s[i:i + int(n)])
+            i += int(n)
+        if parts and parts[0] == "crf" and parts[-1].endswith("_kernel"):
+            return "::".join(parts[1:])
+    return None
+
+
+def launched(fn):
+    """Runs fn() under the CUDA profiler; returns {qualified crf kernel name: [full names]} of what it launched."""
+    from torch.profiler import ProfilerActivity, profile
+    torch.cuda.synchronize()
+    with profile(activities=[ProfilerActivity.CUDA]) as prof:
+        fn()
+        torch.cuda.synchronize()
+    out = {}
+    for e in prof.events():
+        q = _qualified(e.name)
+        if q is not None:
+            out.setdefault(q, []).append(e.name)
+    assert out, "the profiler reported no crf:: kernel for a call that launches one"
+    return out
+
+
+def check_kernels(got, case):
+    unknown = set(got) - set(GEMM_KERNELS) - set(UTILITY_KERNELS)
+    assert not unknown, f"{case.name}: unexpected kernels {unknown}"
+    assert set(got) == set(case.kernels), f"{case.name}: ran {sorted(got)}, expected {sorted(case.kernels)}"
+
+
+class Guarded:
+    """A [rows, cols] fp32 output allocated with GUARD extra rows behind it.  fill: "nan" (overwritten outputs), "zero", or
+    the scale of random values (accumulated outputs), per column [cols] or per row [rows, 1].  .live is the view handed to
+    the kernel."""
+
+    def __init__(self, rows, cols, fill, g):
+        n = rows * cols
+        if isinstance(fill, str):
+            buf = torch.full(((rows + GUARD) * cols,), float("nan") if fill == "nan" else 0.0, device="cuda")
+        else:
+            live = torch.randn(rows, cols, generator=g, device="cuda") * fill.float()
+            buf = torch.cat([live, torch.randn(GUARD, cols, generator=g, device="cuda")]).view(-1)
+        self.buf, self.n = buf, n
+        self.live = buf[:n].view(rows, cols)
+        self.init = self.live.double().clone()
+        self.guard = buf[n:].clone()
+
+    def guard_intact(self):
+        return torch.equal(self.buf[self.n:].view(torch.int32), self.guard.view(torch.int32))
+
+
+def col_err(out, ref, base=None):
+    """Worst over columns of max|out - (base + ref)| / max|ref| of that column (NaN anywhere fails every bar)."""
+    exp = ref if base is None else base + ref
+    d = (out.double() - exp).abs().amax(0)
+    return float((d / ref.abs().amax(0).clamp_min(1e-300)).max())
+
+
+def rel_l2(out, ref):
+    return float((out.double() - ref).norm() / ref.norm())
+
+
+def lrelu(v, s):
+    return torch.where(v > 0, v, v * s)
+
+
+class Inputs:
+    """Seeded fp32 inputs of one case and the post-prologue operand A in fp64."""
+
+    def __init__(self, c):
+        self.g = g = torch.Generator(device="cuda").manual_seed(zlib.crc32(c.name.encode()))
+        self.rn = rn = lambda *s: torch.randn(*s, generator=g, device="cuda")   # noqa: E731
+        M, C1, C2, Cout = c.M, c.C1, c.C2, c.Cout
+        K = C1 + C2
+        self.idx, self.rows_dst, self.rows_src = None, 0, 0
+        if getattr(c, "gather", False):
+            assert M % 3 == 0 and (M // 3) % 128 != 0
+            self.rows_dst = M // 3
+            self.rows_src = self.rows_dst // 4 + 1
+            self.X1 = rn(3 * self.rows_src, C1) + 0.2
+            self.idx = torch.randint(0, self.rows_src, (M,), generator=g, device="cuda")
+            src = (torch.arange(M, device="cuda") // self.rows_dst) * self.rows_src + self.idx
+            A1 = self.X1.double()[src]
+        else:
+            self.X1 = rn(M, C1) + 0.2
+            A1 = self.X1.double()
+        self.X2 = rn(M, C2) - 0.1 if C2 else None
+        self.sc1 = self.sh1 = None
+        if c.slope1 is not None:
+            self.sc1, self.sh1 = 1 + 0.3 * rn(C1), 0.3 * rn(C1)
+            A1 = lrelu(A1 * self.sc1.double() + self.sh1.double(), c.slope1)
+        self.A = torch.cat([A1, self.X2.double()], 1) if C2 else A1
+        self.W = (rn(Cout, K) / math.sqrt(K) * self.scales(Cout)[:, None]).contiguous()
+
+    def scales(self, n):
+        """n factors spread log-uniformly over 1e-2 .. 1e2, in random order."""
+        s = torch.logspace(-2, 2, n, device="cuda") if n > 1 else torch.ones(1, device="cuda")
+        return s[torch.randperm(n, generator=self.g, device="cuda")]
+
+
+# ------------------------------------------------------------------------------------------------------------- forward
+def run_fwd(ops, c):
+    """Runs one forward case; returns (kernels, {output: error}, Y, Yref)."""
+    x = Inputs(c)
+    M, Cout = c.M, c.Cout
+    bias = (x.rn(Cout) * x.W.abs().amax(1)).contiguous() if c.bias else None
+    Yref = x.A @ x.W.double().t()
+    if bias is not None:
+        Yref = Yref + bias.double()
+    Y = Guarded(M, Cout, "nan", x.g)
+    st = None
+    if c.stats:
+        pre = torch.cat([Yref.abs().sum(0), (Yref ** 2).sum(0)]) * 1e-3
+        st = Guarded(ops.STAT_SLOTS, 2 * Cout, pre, x.g)
+    prev = ops.PRECISION
+    ops.PRECISION = c.prec
+    try:
+        got = launched(lambda: ops.linear_fwd(x.X1, x.W, scale1=x.sc1, shift1=x.sh1, slope1=c.slope1 if c.slope1 is not None else 1.0,
+                                              idx1=x.idx, rows_dst=x.rows_dst, rows_src=x.rows_src, X2=x.X2, bias=bias,
+                                              stats=st.live if st else None, M=M, out=Y.live))
+    finally:
+        ops.PRECISION = prev
+    check_kernels(got, c)
+    assert Y.guard_intact(), f"{c.name}: Y written past its last row"
+    errs = {"Y": col_err(Y.live, Yref)}
+    if st is not None:
+        assert st.guard_intact(), f"{c.name}: statistics written past their slots"
+        S = (st.live.double() - st.init).sum(0)              # what the kernel added, over all slots
+        Yk = Y.live.double()                                  # Σ / Σ² of the kernel's own output: the accumulation alone
+        errs["sum"] = float(((S[:Cout] - Yk.sum(0)).abs() / Yk.abs().sum(0)).max())
+        errs["sumsq"] = float(((S[Cout:] - (Yk ** 2).sum(0)).abs() / (Yk ** 2).sum(0)).max())
+    return got, errs, Y.live, Yref
+
+
+@pytest.mark.parametrize("c", FWD_CASES, ids=lambda c: c.name)
+def test_forward(ops, c):
+    got, errs, _, _ = run_fwd(ops, c)
+    (k,) = [k for k in c.kernels if k in FWD_KERNELS]
+    for e in errs.values():
+        _record(k, e, c.name)
+    bad = {n: e for n, e in errs.items() if not e < bar(k)}
+    assert not bad, f"{c.name} on {k}: {bad}"
+
+
+@pytest.mark.parametrize("c", FWDBN_CASES, ids=lambda c: c.name)
+def test_forward_bn(ops, c):
+    x = Inputs(c)
+    M, Cout, eps, mom = c.M, c.Cout, 1e-5, 0.1
+    bnm = torch.nn.BatchNorm1d(Cout, eps=eps, momentum=mom).cuda()
+    with torch.no_grad():
+        bnm.weight.copy_(0.5 + torch.rand(Cout, generator=x.g, device="cuda"))
+        bnm.bias.copy_(0.3 * x.rn(Cout))
+        bnm.running_mean.copy_(x.rn(Cout))
+        bnm.running_var.copy_(1 + torch.rand(Cout, generator=x.g, device="cuda"))
+    rm0, rv0 = bnm.running_mean.double().clone(), bnm.running_var.double().clone()
+    stats = Guarded(ops.STAT_SLOTS, 2 * Cout, "zero", x.g)
+    st = ops.BN(Cout, x.X1.device, stats=stats.live)
+    counter = torch.zeros(ops.counter_ints(), dtype=torch.int32, device="cuda")
+    Y = Guarded(M, Cout, "nan", x.g)
+    got = launched(lambda: ops.linear_fwd_bn(x.X1, x.W, st, bnm, counter, scale1=x.sc1, shift1=x.sh1,
+                                             slope1=c.slope1 if c.slope1 is not None else 1.0, X2=x.X2, out=Y.live))
+    check_kernels(got, c)
+    assert Y.guard_intact() and stats.guard_intact(), f"{c.name}: written past the live rows"
+    assert int(counter.abs().sum()) == 0, "the arrival counter must be left at zero"
+    Yref = x.A @ x.W.double().t()
+    Yk = Y.live.double()
+    mu, var = Yk.mean(0), Yk.var(0, unbiased=False)
+    istd = (var + eps).rsqrt()
+    sd = var.sqrt()
+    gm, bt = bnm.weight.double(), bnm.bias.double()
+
+    def err(out, ref, scale):
+        return float(((out.double() - ref).abs() / scale).max())
+
+    errs = {"Y": col_err(Y.live, Yref),
+            "mean": err(st.mean, mu, sd), "invstd": err(st.invstd, istd, istd), "scale": err(st.scale, gm * istd, gm * istd),
+            "shift": err(st.shift, bt - mu * gm * istd, bt.abs() + (mu * gm * istd).abs()),
+            "running_mean": err(bnm.running_mean, (1 - mom) * rm0 + mom * mu, rm0.abs() + sd),
+            "running_var": err(bnm.running_var, (1 - mom) * rv0 + mom * var * M / (M - 1), rv0 + var)}
+    gemm = [k for k in c.kernels if k in FWD_KERNELS][0]
+    _record(gemm, errs["Y"], c.name)
+    bad = {n: e for n, e in errs.items() if not e < (bar(gemm) if n == "Y" else BAR_BN_FINALIZE)}
+    assert not bad, f"{c.name}: {bad}"
+
+
+# ------------------------------------------------------------------------------------------------------------- backward
+def run_bwd(ops, c):
+    """Runs one backward case; returns (kernels, {output: (error, producing kernel)}, {output: (out, ref)})."""
+    x = Inputs(c)
+    M, C1, C2, Cout = c.M, c.C1, c.C2, c.Cout
+    K = C1 + C2
+    slope = 0.1
+    dY = x.rn(M, Cout) * x.scales(Cout)
+    H = bn = act_ref = None
+    if c.mode == "plain":
+        if c.dbias:
+            # column sums (dbias) well away from zero.  Only here: an offset also makes every dW entry grow like M while the
+            # rounding errors grow like sqrt(M), which would hide a weight-gradient error (single-pass TF32 then meets 2e-5)
+            dY = dY + 0.3 * dY.abs().amax(0)
+        dH = dY.double()
+        slope = 1.0
+    else:
+        H = (x.rn(M, Cout) + 0.8 * (torch.rand(Cout, generator=x.g, device="cuda") - 0.5)) * x.scales(Cout)
+        bn = ops.BN(Cout, dY.device, alloc_stats=False)
+        if c.mode == "act":                               # LeakyReLU of H itself: identity affine, k1 = k2 = 0
+            H = torch.where(H.abs() < KINK, torch.where(H >= 0, 2 * KINK, -2 * KINK), H)
+            bn.scale.fill_(1.0); bn.shift.zero_(); bn.mean.zero_(); bn.invstd.fill_(1.0); bn.k1.zero_(); bn.k2.zero_()
+            dH = lrelu_grad(H.double(), dY.double(), slope)
+        else:
+            gamma = 0.5 + torch.rand(Cout, generator=x.g, device="cuda", dtype=torch.float64)
+            beta = 0.3 * x.rn(Cout).double()
+            for _ in range(4):                            # move every V = Ĥ·γ + β out of (-KINK, KINK)
+                Hd = H.double()
+                mu, var = Hd.mean(0), Hd.var(0, unbiased=False)
+                istd = (var + 1e-5).rsqrt()
+                Hh = (Hd - mu) * istd
+                V = Hh * gamma + beta
+                near = V.abs() < KINK
+                if not bool(near.any()):
+                    break
+                Vt = torch.where(V >= 0, 2 * KINK, -2 * KINK)
+                H = torch.where(near, mu + (Vt - beta) / gamma / istd, Hd).float()
+            assert not bool(near.any())
+            bn.mean.copy_(mu.float()); bn.invstd.copy_(istd.float())
+            bn.scale.copy_((gamma * istd).float()); bn.shift.copy_((beta - mu * gamma * istd).float())
+            if c.act_ref:
+                act_ref = x.rn(M, Cout)
+                pre = act_ref.double()
+            else:
+                pre = V
+            dV = torch.where(pre > 0, dY.double(), dY.double() * slope)
+            k1, k2 = dV.mean(0), (dV * Hh).mean(0)
+            bn.k1.copy_(k1.float()); bn.k2.copy_(k2.float())
+            dH = gamma * istd * (dV - k1 - Hh * k2)
+        bn.count, bn.training = M, True
+    dA = dH @ x.W.double()
+    refs = {"dX1": dA[:, :C1], "dX2": dA[:, C1:], "dW": dH.t() @ x.A, "dbias": dH.sum(0, keepdim=True)}
+
+    def out(rows, cols, how, ref):
+        return Guarded(rows, cols, "nan" if how == "new" else ref.abs().amax(0), x.g)
+
+    o = {}
+    if c.dx1:
+        o["dX1"] = out(M, C1, c.dx1, refs["dX1"])
+    if C2 and c.dx2:
+        o["dX2"] = out(M, C2, c.dx2, refs["dX2"])
+    if c.dw:
+        o["dW"] = Guarded(Cout, K, refs["dW"].abs().amax(1, keepdim=True), x.g)     # random, at each row's own scale
+    if c.dbias:
+        o["dbias"] = out(1, Cout, "acc", refs["dbias"])
+    scratch, stride = None, 0
+    if c.dw == "stride":
+        n = Cout * K
+        stride = (n + 63) // 64 * 64 + 64
+        scratch = Guarded(ops.GRAD_SLOTS, stride, "zero", x.g)
+    prev = ops.PRECISION
+    ops.PRECISION = c.prec
+    try:
+        got = launched(lambda: ops.linear_bwd(
+            dY, H, bn, slope, x.X1, x.W, scale1=x.sc1, shift1=x.sh1, slope1=c.slope1 if c.slope1 is not None else 1.0,
+            idx1=x.idx, rows_dst=x.rows_dst, rows_src=x.rows_src, X2=x.X2,
+            dX1=o["dX1"].live if "dX1" in o else None, acc1=c.dx1 == "acc",
+            dX2=o["dX2"].live if "dX2" in o else None, acc2=c.dx2 == "acc",
+            dW=o["dW"].live if "dW" in o else None, dbias=o["dbias"].live.view(-1) if "dbias" in o else None,
+            act_ref=act_ref, scratch=scratch.live if scratch else None, scratch_stride=stride))
+    finally:
+        ops.PRECISION = prev
+    check_kernels(got, c)
+    if scratch is not None:
+        n = Cout * K
+        assert scratch.guard_intact() and bool((scratch.live[:, n:] == 0).all()), f"{c.name}: weight-gradient slot written past its end"
+        ops.grad_slots_reduce(scratch.live, o["dW"].live.view(-1), n, stride)
+        torch.cuda.synchronize()
+    for name, buf in o.items():
+        assert buf.guard_intact(), f"{c.name}: {name} written past its live part"
+    dg = [k for k in c.kernels if k in DGRAD_KERNELS + BOTH_KERNELS]
+    wg = [k for k in c.kernels if k in WGRAD_KERNELS + BOTH_KERNELS]
+    errs, pairs = {}, {}
+    for name, buf in o.items():
+        ref = refs[name]
+        base = None if (name in ("dX1", "dX2") and getattr(c, name.lower()) == "new") else buf.init
+        if name == "dW":
+            e = col_err(buf.live.t(), ref.t(), base.t())
+        else:
+            e = col_err(buf.live, ref, base)
+        errs[name] = (e, (dg if name.startswith("dX") else wg)[0])
+        pairs[name] = (buf.live.double() - (0 if base is None else base), ref)
+    return got, errs, pairs
+
+
+def lrelu_grad(pre, dy, slope):
+    return torch.where(pre > 0, dy, dy * slope)
+
+
+@pytest.mark.parametrize("c", BWD_CASES, ids=lambda c: c.name)
+def test_backward(ops, c):
+    got, errs, _ = run_bwd(ops, c)
+    for e, k in errs.values():
+        _record(k, e, c.name)
+    bad = {n: (e, k) for n, (e, k) in errs.items() if not e < bar(k)}
+    assert not bad, f"{c.name}: {bad}"
+
+
+# ------------------------------------------------------------------------------------------------------------- precision modes
+@pytest.mark.parametrize("c", TF32_CASES, ids=lambda c: c.name)
+def test_single_pass_tf32_misses_the_3xtf32_bar(ops, c):
+    """The generic kernels in single-pass TF32 (the `false` instantiations) must miss the bar the 3xTF32 kernels meet."""
+    if isinstance(c, Fwd):
+        got, errs, _, _ = run_fwd(ops, c)
+        errs = {"Y": errs["Y"]}
+    else:
+        got, errs, _ = run_bwd(ops, c)
+        errs = {n: e for n, (e, _) in errs.items()}
+    for q, names in got.items():
+        if q in GEMM_KERNELS:
+            assert all(re.search(r"_kernel<[^>]*false>", s) for s in names), f"{c.name}: not the single-pass instantiation: {names}"
+    good = {n: e for n, e in errs.items() if not e > BAR_X3}
+    assert not good, f"{c.name}: single-pass TF32 met the 3xTF32 bar {BAR_X3}: {good}"
+
+
+@pytest.mark.parametrize("c", BF16_CASES, ids=lambda c: c.name)
+def test_single_pass_bf16_within_stated_bound(ops, c):
+    if isinstance(c, Fwd):
+        _, errs, Y, Yref = run_fwd(ops, c)
+        e = rel_l2(Y, Yref)
+        assert e < BF16_FWD_L2, f"{c.name}: {e}"
+    else:
+        _, _, pairs = run_bwd(ops, c)
+        worst = {n: rel_l2(a, b) for n, (a, b) in pairs.items()}
+        assert all(v < BF16_GRAD_L2 for v in worst.values()), f"{c.name}: {worst}"
