@@ -28,8 +28,6 @@ constexpr int BM = 128;      // rows per CTA tile (fwd / dgrad)
 constexpr int BK = 32;       // reduction chunk
 constexpr int AS = BK + 4;   // smem row stride for [row][k] operands read as (g, t): bank = 4g + t
 
-__device__ __forceinline__ float lrelu(float v, float slope) { return v > 0.0f ? v : v * slope; }
-
 // ------------------------------------------------------------------------------------------ forward
 
 
@@ -570,16 +568,13 @@ __global__ void __launch_bounds__(256) wgrad_tiny_kernel(const WgradArgs a) {
     }
 }
 
-inline bool try_wgrad_tiny(const WgradArgs& a, cudaStream_t st, int* rc) {
-    if (a.C2 != 0 || a.C1 < 1 || a.C1 > 4 || a.dbias || (a.Cout & 3) || a.Cout > 1024 || (256 % (a.Cout >> 2)) != 0) return false;
-    if ((reinterpret_cast<uintptr_t>(a.dY) & 15) || (a.bn.scale && (reinterpret_cast<uintptr_t>(a.H) & 15))) return false;
-    if (a.bn.scale && a.bn.act_ref && (reinterpret_cast<uintptr_t>(a.bn.act_ref) & 15)) return false;
+inline int try_wgrad_tiny(const WgradArgs& a, cudaStream_t st) {
+    if (a.C2 != 0 || a.C1 < 1 || a.C1 > 4 || a.dbias || (a.Cout & 3) || a.Cout > 1024 || (256 % (a.Cout >> 2)) != 0) return kDeclined;
+    if (!aligned16(a.dY) || (a.bn.scale && !aligned16(a.H))) return kDeclined;
+    if (a.bn.scale && a.bn.act_ref && !aligned16(a.bn.act_ref)) return kDeclined;
     const int rows_per_it = 256 / (a.Cout >> 2);
     const unsigned grid = (unsigned)std::min<int64_t>(ceil_div(a.M, (int64_t)rows_per_it * 4), (int64_t)kNumSMs * 8);
-    wgrad_tiny_kernel<4><<<grid, 256, 0, st>>>(a);
-    cudaError_t e = cudaPeekAtLastError();
-    *rc = e == cudaSuccess ? CRF_OK : (int)e;
-    return true;
+    return launch<false>(wgrad_tiny_kernel<4>, dim3(grid), dim3(256), 0, st, a);
 }
 
 // dW[co, k] += Σ_m dH[m, co] · A[m, k],  A = [prologue(X1) | X2].  Output tile 64 (co) × 64 (k) per CTA; CTAs along
@@ -702,6 +697,33 @@ inline int dispatch_bn(int n, F&& f) {
     return f(std::integral_constant<int, 8>{});
 }
 
+// The generic kernels take every shape: x3 = 3xTF32, else single-pass TF32.
+inline int fwd_generic(const FwdArgs& a, bool x3, cudaStream_t st) {
+    return dispatch_bn(a.Cout, [&](auto bn) {
+        constexpr int BN = decltype(bn)::value;
+        const dim3 grid((unsigned)ceil_div(a.M, BM), (unsigned)ceil_div(a.Cout, BN));
+        return launch<false>(x3 ? fwd_kernel<BN, true> : fwd_kernel<BN, false>, grid, dim3(kThreads), 0, st, a);
+    });
+}
+
+inline int dgrad_generic(const DgradArgs& a, bool x3, cudaStream_t st) {
+    const int Ktot = a.C1 + a.C2;
+    return dispatch_bn(Ktot, [&](auto bn) {
+        constexpr int BN = decltype(bn)::value;
+        const dim3 grid((unsigned)ceil_div(a.M, BM), (unsigned)ceil_div(Ktot, BN));
+        return launch<false>(x3 ? dgrad_kernel<BN, true> : dgrad_kernel<BN, false>, grid, dim3(kThreads), 0, st, a);
+    });
+}
+
+inline int wgrad_generic(WgradArgs a, bool x3, cudaStream_t st) {
+    const int ty = (int)ceil_div(a.Cout, 64), tz = (int)ceil_div(a.C1 + a.C2, 64);
+    int64_t splits = std::max<int64_t>(1, std::min<int64_t>(ceil_div(a.M, 256), (int64_t)(2 * kNumSMs) / (ty * tz) + 1));
+    a.rows_per_cta = ceil_div(ceil_div(a.M, splits), WR) * WR;
+    splits = ceil_div(a.M, a.rows_per_cta);
+    const dim3 grid((unsigned)splits, (unsigned)ty, (unsigned)tz);
+    return launch<false>(x3 ? wgrad_kernel<true> : wgrad_kernel<false>, grid, dim3(kThreads), 0, st, a);
+}
+
 }  // namespace lin
 }  // namespace crf
 
@@ -719,36 +741,26 @@ int crfconv_set_fast_path(int mode) {
 
 // Y[M,Cout] = [lrelu(X1*scale1+shift1) | X2] · Wᵀ (+ bias);  stats[0:Cout] += Σ_rows Y, stats[Cout:2Cout] += Σ_rows Y².
 // X1 rows may be gathered: source row of output row m = (m / rows_dst) * rows_src + idx1[m]   (idx1 null ⇒ identity).
-// precision: 0 = 3xTF32 (fp32-grade), 1 = single-pass TF32.
+// precision: 0 = 3xTF32 (fp32-grade), 1 = single-pass TF32, 2 = single-pass bf16 where the persistent kernels take the shape
+// (single-pass TF32 elsewhere).  Families in the order of DESIGN.md §4.3; the first that takes the call launches one kernel.
 int crfconv_linear_fwd(const float* X1, int C1, const float* scale1, const float* shift1, float slope1, const int64_t* idx1,
                        int64_t rows_dst, int64_t rows_src, const float* X2, int C2, const float* W, const float* bias, float* Y,
                        float* stats, int64_t M, int Cout, int precision, void* stream) {
-    if (M < 0 || Cout <= 0 || C1 < 0 || C2 < 0 || C1 + C2 <= 0) return CRF_ERR_INVALID_ARG;
+    if (M < 0 || Cout <= 0 || C1 < 0 || C2 < 0 || C1 + C2 <= 0 || precision < 0 || precision > 2) return CRF_ERR_INVALID_ARG;
     if (M == 0) return CRF_OK;
     if ((C1 > 0 && !X1) || (C2 > 0 && !X2) || !W || !Y) return CRF_ERR_INVALID_ARG;
     if (idx1 && (rows_dst <= 0 || rows_src <= 0)) return CRF_ERR_INVALID_ARG;
-    lin::FwdArgs a{X1, C1, scale1, shift1, slope1, idx1, rows_dst, rows_src, X2, C2, W, bias, Y, stats, M, Cout};
+    const lin::FwdArgs a{X1, C1, scale1, shift1, slope1, idx1, rows_dst, rows_src, X2, C2, W, bias, Y, stats, M, Cout};
     cudaStream_t st = (cudaStream_t)stream;
-    if (lin::use_fast(M)) {
-        int rc2 = CRF_OK;
-        if (lin::try_fwd3(a, precision, st, &rc2)) return rc2;      // tcgen05: also faster than the CUDA-core kernel for 16→16 (17 vs 24 us)
-        if (lin::try_narrow_fwd(a, st, &rc2)) return rc2;
-        if (lin::try_fwd2(a, precision, st, &rc2)) return rc2;
-    }
-    if (precision == 0) {
-        int rc2 = CRF_OK;
-        if (lin::try_fwd_small(a, st, &rc2)) return rc2;
-        if (lin::try_upproj_fwd(a, st, &rc2)) return rc2;
-    }
-    if (precision == 2) precision = 1;     // generic kernels: single-pass TF32 stands in for single-pass bf16
-    return lin::dispatch_bn(Cout, [&](auto bn) {
-        constexpr int BN = decltype(bn)::value;
-        dim3 grid((unsigned)ceil_div(M, lin::BM), (unsigned)ceil_div(Cout, BN));
-        if (precision == 0) lin::fwd_kernel<BN, true><<<grid, lin::kThreads, 0, st>>>(a);
-        else lin::fwd_kernel<BN, false><<<grid, lin::kThreads, 0, st>>>(a);
-        CRF_LAUNCH_CHECK();
-        return CRF_OK;
-    });
+    const bool fast = lin::use_fast(M), x3 = precision == 0;
+    int rc = lin::kDeclined;
+    if (rc == lin::kDeclined && fast) rc = lin::try_fwd3(a, precision, st);      // tcgen05: also faster than the CUDA-core kernel for 16→16 (17 vs 24 us)
+    if (rc == lin::kDeclined && fast) rc = lin::try_narrow_fwd(a, st);
+    if (rc == lin::kDeclined && fast) rc = lin::try_fwd2(a, precision, st);
+    if (rc == lin::kDeclined && x3) rc = lin::try_fwd_small(a, st);
+    if (rc == lin::kDeclined && x3) rc = lin::try_upproj_fwd(a, st);
+    if (rc == lin::kDeclined) rc = lin::fwd_generic(a, x3, st);
+    return rc;
 }
 
 int crfconv_bn_finalize_fwd(const float* stats, int64_t count, const float* gamma, const float* beta, float eps, float momentum,
@@ -808,89 +820,63 @@ int crfconv_linear_bwd_launches(void) { return lin::t_bwd_launches; }
 
 // Gradient of crfconv_linear_fwd wrt its (post-prologue) inputs and its weight.  The upstream gradient is given wrt the
 // layer's ACTIVATION output (dY); the BN(+LeakyReLU) backward transform is applied on the fly (scale == NULL ⇒ the layer
-// had no BN: dH = dY).   dX1 / dX2 may be NULL (not needed); acc ⇒ accumulate into the destination.
+// had no BN: dH = dY).   dX1 / dX2 may be NULL (not needed); acc ⇒ accumulate into the destination.  With idx1, dX1 is the
+// gradient wrt the GATHERED rows [M, C1]; scatter it with crfconv_scatter_add_rows.
+// Families in the order of DESIGN.md §4.3: a one-pass kernel for both gradients, else one kernel per requested gradient.
 int crfconv_linear_bwd(const float* dY, const float* H, const float* act_ref, const float* scale, const float* shift,
                        const float* mean, const float* invstd, const float* k1, const float* k2, float slope,
                        const float* X1, int C1, const float* scale1, const float* shift1, float slope1, const int64_t* idx1,
                        int64_t rows_dst, int64_t rows_src, const float* X2, int C2, const float* W, float* dX1, int acc1,
                        float* dX2, int acc2, float* dW, float* dbias, float* dW_scratch, int64_t dW_scratch_stride, int64_t M, int Cout, int precision,
                        void* stream) {
-    lin::t_bwd_launches = 0;
-    if (M < 0 || Cout <= 0 || C1 < 0 || C2 < 0 || C1 + C2 <= 0 || !dY || !W) return CRF_ERR_INVALID_ARG;
+    int& launches = lin::t_bwd_launches;
+    launches = 0;
+    if (M < 0 || Cout <= 0 || C1 < 0 || C2 < 0 || C1 + C2 <= 0 || !dY || !W || precision < 0 || precision > 2) return CRF_ERR_INVALID_ARG;
     if (M == 0) return CRF_OK;
     if (scale && (Cout & 3)) return CRF_ERR_UNSUPPORTED;
     cudaStream_t st = (cudaStream_t)stream;
-    const int n_reduce = (dW && dW_scratch && dW_scratch_stride <= 0) ? 1 : 0;
-    lin::t_bwd_launches = int(dX1 || dX2) + int(dW != nullptr) + n_reduce;     // one kernel each, unless a one-pass kernel takes both
-    lin::BnBwd bn{scale, shift, mean, invstd, k1, k2, act_ref, slope};
+    const bool fast = lin::use_fast(M), x3 = precision == 0;
     const int Ktot = C1 + C2;
-    const int gprec = precision == 2 ? 1 : precision;    // precision seen by the generic (TF32) kernels
     // weight-gradient partial slots: CTAs add into dW_scratch[slot] (zero-initialised by the caller), reduced into dW afterwards
-    float* wdst = (dW && dW_scratch) ? dW_scratch : dW;
-    const int64_t wstride = (dW && dW_scratch) ? (dW_scratch_stride > 0 ? dW_scratch_stride : (int64_t)Cout * Ktot) : 0;
-    auto reduce_slots = [&]() -> int {
-        if (dW && dW_scratch && dW_scratch_stride <= 0) {      // stride given ⇒ the caller reduces all its layers at once
-            lin::grad_slots_reduce_kernel<<<(unsigned)ceil_div((int64_t)Cout * Ktot, 256), 256, 0, st>>>(dW_scratch, dW, Cout * Ktot, (int64_t)Cout * Ktot);
-            CRF_LAUNCH_CHECK();
-        }
-        return CRF_OK;
+    // here, or by the caller when it gives the slot stride (it reduces all its layers at once)
+    const bool slots = dW && dW_scratch;
+    const int64_t wstride = slots ? (dW_scratch_stride > 0 ? dW_scratch_stride : (int64_t)Cout * Ktot) : 0;
+    const lin::BnBwd bn{scale, shift, mean, invstd, k1, k2, act_ref, slope};
+    const lin::DgradArgs d{dY, H, bn, W, dX1, C1, acc1, dX2, C2, acc2, M, Cout};
+    const lin::WgradArgs w{dY, H, bn, X1, C1, scale1, shift1, slope1, idx1, rows_dst, rows_src, X2, C2, slots ? dW_scratch : dW, dbias, M, Cout, 0, wstride};
+    auto finish = [&](int rc) -> int {
+        if (rc != CRF_OK || !slots || dW_scratch_stride > 0) return rc;
+        ++launches;
+        return lin::launch<false>(lin::grad_slots_reduce_kernel, dim3((unsigned)ceil_div((int64_t)Cout * Ktot, 256)), dim3(256), 0, st,
+                                  dW_scratch, dW, Cout * Ktot, (int64_t)Cout * Ktot);
     };
-    if (lin::use_fast(M)) {                               // hidden-width layers: one fused dgrad + wgrad CUDA-core kernel
-        lin::DgradArgs d{dY, H, bn, W, dX1, C1, acc1, dX2, C2, acc2, M, Cout};
-        lin::WgradArgs w{dY, H, bn, X1, C1, scale1, shift1, slope1, idx1, rows_dst, rows_src, X2, C2, wdst, dbias, M, Cout, 0, wstride};
-        int rc2 = CRF_OK;
-        if (dW && lin::try_bwd3(d, w, precision, st, &rc2)) {
-            lin::t_bwd_launches = 1 + n_reduce;
-            return rc2 != CRF_OK ? rc2 : reduce_slots();
-        }
-        if (lin::try_narrow_bwd(d, dW ? &w : nullptr, st, &rc2)) {
-            lin::t_bwd_launches = 1 + n_reduce;
-            return rc2 != CRF_OK ? rc2 : reduce_slots();
-        }
+
+    int rc = lin::kDeclined;                                                      // input and weight gradient in one kernel
+    if (rc == lin::kDeclined && fast) rc = lin::try_bwd3(d, w, precision, st);
+    if (rc == lin::kDeclined && fast) rc = lin::try_narrow_bwd(d, dW ? &w : nullptr, st);
+    if (rc != lin::kDeclined) {
+        ++launches;
+        return finish(rc);
     }
-    if (dX1 || dX2) {
-        // with idx1, dX1 is the gradient wrt the GATHERED rows [M, C1]; scatter it with crfconv_scatter_add_rows
-        lin::DgradArgs a{dY, H, bn, W, dX1, C1, acc1, dX2, C2, acc2, M, Cout};
-        int rc = CRF_OK;
-        if (!(lin::use_fast(M) && (lin::try_dgrad3(a, precision, st, &rc) || lin::try_dgrad2(a, precision, st, &rc))) &&
-            !(gprec == 0 && (lin::try_dgrad_small(a, st, &rc) || lin::try_upproj_dgrad(a, st, &rc))))
-        rc = lin::dispatch_bn(Ktot, [&](auto bnv) {
-            constexpr int BN = decltype(bnv)::value;
-            dim3 grid((unsigned)ceil_div(M, lin::BM), (unsigned)ceil_div(Ktot, BN));
-            if (gprec == 0) lin::dgrad_kernel<BN, true><<<grid, lin::kThreads, 0, st>>>(a);
-            else lin::dgrad_kernel<BN, false><<<grid, lin::kThreads, 0, st>>>(a);
-            CRF_LAUNCH_CHECK();
-            return CRF_OK;
-        });
+    if (dX1 || dX2) {                                                             // input gradient
+        if (rc == lin::kDeclined && fast) rc = lin::try_dgrad3(d, precision, st);
+        if (rc == lin::kDeclined && fast) rc = lin::try_dgrad2(d, precision, st);
+        if (rc == lin::kDeclined && x3) rc = lin::try_dgrad_small(d, st);
+        if (rc == lin::kDeclined && x3) rc = lin::try_upproj_dgrad(d, st);
+        if (rc == lin::kDeclined) rc = lin::dgrad_generic(d, x3, st);
+        ++launches;
         if (rc != CRF_OK) return rc;
     }
-    if (dW) {
-        lin::WgradArgs a{dY, H, bn, X1, C1, scale1, shift1, slope1, idx1, rows_dst, rows_src, X2, C2, wdst, dbias, M, Cout, 0, wstride};
-        {
-            int rc2 = CRF_OK;
-            if (lin::try_wgrad_tiny(a, st, &rc2)) return rc2 != CRF_OK ? rc2 : reduce_slots();
-        }
-        if (lin::use_fast(M)) {
-            int rc2 = CRF_OK;
-            if (lin::try_wgrad3(a, precision, st, &rc2)) return rc2 != CRF_OK ? rc2 : reduce_slots();
-            if (lin::try_wgrad2(a, precision, st, &rc2)) return rc2 != CRF_OK ? rc2 : reduce_slots();
-        }
-        {
-            int rc2 = CRF_OK;
-            if (gprec == 0 && lin::try_wgrad_direct(a, st, &rc2)) return rc2 != CRF_OK ? rc2 : reduce_slots();
-            if (gprec == 0 && lin::try_wgrad_rows(a, st, &rc2)) return rc2 != CRF_OK ? rc2 : reduce_slots();
-        }
-        const int ty = (int)ceil_div(Cout, 64), tz = (int)ceil_div(Ktot, 64);
-        int64_t splits = std::max<int64_t>(1, std::min<int64_t>(ceil_div(M, 256), (int64_t)(2 * kNumSMs) / (ty * tz) + 1));
-        a.rows_per_cta = ceil_div(ceil_div(M, splits), lin::WR) * lin::WR;
-        splits = ceil_div(M, a.rows_per_cta);
-        dim3 grid((unsigned)splits, (unsigned)ty, (unsigned)tz);
-        if (gprec == 0) lin::wgrad_kernel<true><<<grid, lin::kThreads, 0, st>>>(a);
-        else lin::wgrad_kernel<false><<<grid, lin::kThreads, 0, st>>>(a);
-        CRF_LAUNCH_CHECK();
-        return reduce_slots();
-    }
-    return CRF_OK;
+    if (!dW) return CRF_OK;
+    rc = lin::kDeclined;                                                          // weight gradient
+    if (rc == lin::kDeclined) rc = lin::try_wgrad_tiny(w, st);
+    if (rc == lin::kDeclined && fast) rc = lin::try_wgrad3(w, precision, st);
+    if (rc == lin::kDeclined && fast) rc = lin::try_wgrad2(w, precision, st);
+    if (rc == lin::kDeclined && x3) rc = lin::try_wgrad_direct(w, st);
+    if (rc == lin::kDeclined && x3) rc = lin::try_wgrad_rows(w, st);
+    if (rc == lin::kDeclined) rc = lin::wgrad_generic(w, x3, st);
+    ++launches;
+    return finish(rc);
 }
 
 // crfconv_linear_fwd + training-mode BatchNorm finalize of its output (what crfconv_bn_finalize_fwd computes from `stats`), in ONE
@@ -901,12 +887,12 @@ int crfconv_linear_fwd_bn(const float* X1, int C1, const float* scale1, const fl
                           const float* gamma, const float* beta, float* running_mean, float* running_var, float eps, float momentum,
                           float* scale, float* shift, float* mean, float* invstd, void* stream) {
     if (M <= 0 || Cout <= 0 || C1 <= 0 || C2 < 0 || !X1 || (C2 > 0 && !X2) || !W || !Y || !stats || !counter || !scale || !shift) return CRF_ERR_INVALID_ARG;
+    if (precision < 0 || precision > 2) return CRF_ERR_INVALID_ARG;
     lin::FwdArgs a{X1, C1, scale1, shift1, slope1, nullptr, 0, 0, X2, C2, W, nullptr, Y, stats, M, Cout};
     a.fin = cl::FwdFin{stats, counter, gamma, beta, running_mean, running_var, eps, momentum, (double)M, scale, shift, mean, invstd};
-    cudaStream_t st = (cudaStream_t)stream;
     if (lin::use_fast(M)) {
-        int rc2 = CRF_OK;
-        if (lin::try_fwd3(a, precision, st, &rc2)) return rc2;
+        const int rc = lin::try_fwd3(a, precision, (cudaStream_t)stream);
+        if (rc != lin::kDeclined) return rc;
     }
     const int rc = crfconv_linear_fwd(X1, C1, scale1, shift1, slope1, nullptr, 0, 0, X2, C2, W, nullptr, Y, stats, M, Cout, precision, stream);
     if (rc != CRF_OK) return rc;

@@ -15,14 +15,15 @@ using lin::BnBwd;
 using lin::DgradArgs;
 using lin::FwdArgs;
 using lin::WgradArgs;
+using lin::lrelu;
 
 constexpr int BK = 32;     // reduction chunk (floats) per pipeline stage
 constexpr int AS = 40;     // smem row stride (floats) of staged fp32 tiles: 40 ≡ 8 (mod 32) ⇒ conflict-free LDS.64 at (g, 2t)
 constexpr int NST = 3;     // cp.async ring depth
 
 // ===================================================================================================== forward
-// Y[M, Cout] = [ lrelu(X1*scale+shift) | X2 ] · Wᵀ (+bias), Σ/Σ² epilogue.   BN = padded Cout tile (8..64).
-template <int BN, bool X3>
+// Y[M, Cout] = [ lrelu(X1*scale+shift) | X2 ] · Wᵀ (+bias), Σ/Σ² epilogue, single bf16 pass.   BN = padded Cout tile (8..64).
+template <int BN>
 __global__ void __launch_bounds__(kThreads, 2) fwd2_kernel(const FwdArgs a, const int ntiles) {
     constexpr int BM = 128;
     extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -131,7 +132,7 @@ __global__ void __launch_bounds__(kThreads, 2) fwd2_kernel(const FwdArgs a, cons
 #pragma unroll
                 for (int nt = 0; nt < BN / 8; ++nt) {
                     const int wi = (nt * 8 + g) * WS2 + wb;
-                    mma3<X3>(acc[nt], ah, al, Wh[wi], Wh[wi + 4], Wl[wi], Wl[wi + 4]);
+                    mma3<false>(acc[nt], ah, al, Wh[wi], Wh[wi + 4], Wl[wi], Wl[wi + 4]);
                 }
             }
         }
@@ -389,15 +390,7 @@ __global__ void __launch_bounds__(kThreads, (BN >= 128 || REF) ? 1 : 2) dgrad2_k
         Wh[n * WS2 + kp / 2] = hi;
         Wl[n * WS2 + kp / 2] = lo;
     }
-    for (int k = tid; k < Kpad; k += kThreads) {
-        float4 pr = make_float4(1.f, 0.f, 0.f, 0.f);
-        if (!plain && k < C) {
-            const float sc = __ldg(a.bn.scale + k), sh = __ldg(a.bn.shift + k), mu = __ldg(a.bn.mean + k), is = __ldg(a.bn.invstd + k);
-            const float k1 = __ldg(a.bn.k1 + k), k2 = __ldg(a.bn.k2 + k);
-            pr = make_float4(sc, sh, -sc * is * k2, -sc * k1 + sc * is * k2 * mu);
-        }
-        s_par[k] = pr;
-    }
+    for (int k = tid; k < Kpad; k += kThreads) s_par[k] = (!plain && k < C) ? a.bn.coef(k) : make_float4(1.f, 0.f, 0.f, 0.f);
 
     const int my_tiles = (ntiles - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x;
     const int Q = my_tiles * nch;
@@ -541,15 +534,7 @@ __global__ void __launch_bounds__(kThreads, 2) wgrad2_kernel(const WgradArgs a, 
     const int Ktot = a.C1 + a.C2, C = a.Cout;
     const int wco = w % WCO, wci = w / WCO;
 
-    for (int k = tid; k < CO; k += kThreads) {
-        float4 pr = make_float4(1.f, 0.f, 0.f, 0.f);
-        if (!plain && k < C) {
-            const float sc = __ldg(a.bn.scale + k), sh = __ldg(a.bn.shift + k), mu = __ldg(a.bn.mean + k), is = __ldg(a.bn.invstd + k);
-            const float k1 = __ldg(a.bn.k1 + k), k2 = __ldg(a.bn.k2 + k);
-            pr = make_float4(sc, sh, -sc * is * k2, -sc * k1 + sc * is * k2 * mu);
-        }
-        s_par[k] = pr;
-    }
+    for (int k = tid; k < CO; k += kThreads) s_par[k] = (!plain && k < C) ? a.bn.coef(k) : make_float4(1.f, 0.f, 0.f, 0.f);
     for (int k = tid; k < KP; k += kThreads) {
         float2 pr = make_float2(1.f, 0.f);
         if (a.scale1 && k < a.C1) pr = make_float2(__ldg(a.scale1 + k), __ldg(a.shift1 + k));
@@ -689,7 +674,7 @@ size_t wgrad2_smem() {
     return (size_t)2 * RAW * 4 + (size_t)2 * (CO + KP) * TS * 4 + (size_t)CO * 16 + (size_t)KP * 8;
 }
 
-// ---- F×F (F <= 32) weight gradients on CUDA cores: dW[a][b] += Σ_m dH[m][a]·X[m][b].  Each thread owns a 4×4 block of the
+// ---- F×F weight gradients on CUDA cores (launched for F = 32; F = 8 / 16 are narrow_bwd's): dW[a][b] += Σ_m dH[m][a]·X[m][b].  Each thread owns a 4×4 block of the
 // output; the (F/4)² block owners are replicated over 256/(F/4)² row groups that take interleaved rows of a 128-row tile.
 template <int F, bool REF>
 __global__ void __launch_bounds__(kThreads) wgrad_small_kernel(const WgradArgs a, const int ntiles) {
@@ -765,43 +750,24 @@ __global__ void __launch_bounds__(kThreads) wgrad_small_kernel(const WgradArgs a
     for (int i = tid; i < F * F; i += kThreads) atomicAdd(a.dW + a.slot_stride * (blockIdx.x % kGradSlots) + i, red[i]);
 }
 
-inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
-
 }  // namespace lin2
 
 namespace lin {
 
-#define CRF_SET_SMEM(kern, bytes)                                                                            \
-    do {                                                                                                     \
-        cudaError_t _e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(bytes)); \
-        if (_e != cudaSuccess) { *rc = (int)_e; return true; }                                               \
-    } while (0)
-
-bool try_fwd2(const FwdArgs& a, int precision, cudaStream_t st, int* rc) {
+int try_fwd2(const FwdArgs& a, int precision, cudaStream_t st) {
     using namespace lin2;
     const int Ktot = a.C1 + a.C2;
-    if (precision == 1) return false;                          // explicit TF32 request → generic kernels
-    if (a.Cout > 64 || (a.Cout & 3) || Ktot > 128 || (a.C1 & 3) || (a.C2 & 3) || a.C1 == 0) return false;
-    if (!aligned16(a.X1) || (a.C2 && !aligned16(a.X2)) || (reinterpret_cast<uintptr_t>(a.Y) & 7)) return false;
+    if (precision == 1) return kDeclined;                      // explicit TF32 request → generic kernels
+    if (a.Cout > 64 || (a.Cout & 3) || Ktot > 128 || (a.C1 & 3) || (a.C2 & 3) || a.C1 == 0) return kDeclined;
+    if (!aligned16(a.X1) || (a.C2 && !aligned16(a.X2)) || (reinterpret_cast<uintptr_t>(a.Y) & 7)) return kDeclined;
     const int nch = (a.C1 + BK - 1) / BK + (a.C2 + BK - 1) / BK, Kpad = nch * BK;
-    if (Kpad > 160) return false;
+    if (Kpad > 160) return kDeclined;
     const int ntiles = (int)ceil_div(a.M, 128);
-    const int grid = std::min(ntiles, 2 * kNumSMs);
-    *rc = CRF_OK;
     auto go = [&](auto bnv) {
         constexpr int BN = decltype(bnv)::value;
-        if (precision == 0) {            // fp32-grade forward (3xTF32)
-            const size_t smem = fwd2t_smem<BN>(Kpad);
-            CRF_SET_SMEM((fwd2t_kernel<BN>), smem);
-            fwd2t_kernel<BN><<<std::min(ntiles, FwdT<BN>::CTAS * kNumSMs), kThreads, smem, st>>>(a, ntiles);
-        } else {
-            const size_t smem = fwd2_smem<BN>(Kpad);
-            if (precision == 3) { CRF_SET_SMEM((fwd2_kernel<BN, true>), smem); fwd2_kernel<BN, true><<<grid, kThreads, smem, st>>>(a, ntiles); }
-            else                { CRF_SET_SMEM((fwd2_kernel<BN, false>), smem); fwd2_kernel<BN, false><<<grid, kThreads, smem, st>>>(a, ntiles); }
-        }
-        cudaError_t e = cudaPeekAtLastError();
-        if (e != cudaSuccess) *rc = (int)e;
-        return true;
+        if (precision == 0)              // fp32-grade forward (3xTF32)
+            return launch<false>(fwd2t_kernel<BN>, dim3(std::min(ntiles, FwdT<BN>::CTAS * kNumSMs)), dim3(kThreads), fwd2t_smem<BN>(Kpad), st, a, ntiles);
+        return launch<false>(fwd2_kernel<BN>, dim3(std::min(ntiles, 2 * kNumSMs)), dim3(kThreads), fwd2_smem<BN>(Kpad), st, a, ntiles);
     };
     if (a.Cout > 32) return go(std::integral_constant<int, 64>{});
     if (a.Cout > 16) return go(std::integral_constant<int, 32>{});
@@ -809,29 +775,24 @@ bool try_fwd2(const FwdArgs& a, int precision, cudaStream_t st, int* rc) {
     return go(std::integral_constant<int, 8>{});
 }
 
-bool try_dgrad2(const DgradArgs& a, int precision, cudaStream_t st, int* rc) {
+int try_dgrad2(const DgradArgs& a, int precision, cudaStream_t st) {
     using namespace lin2;
     const int Ktot = a.C1 + a.C2;
-    if (precision == 1) return false;
-    if (a.Cout > 64 || (a.Cout & 3) || Ktot > 128 || Ktot < 8 || (a.C1 & 3) || (a.C2 & 3)) return false;
-    if (!aligned16(a.dY) || (a.bn.scale && !aligned16(a.H)) || (a.bn.act_ref && !aligned16(a.bn.act_ref))) return false;
-    if ((a.dX1 && (reinterpret_cast<uintptr_t>(a.dX1) & 7)) || (a.dX2 && (reinterpret_cast<uintptr_t>(a.dX2) & 7))) return false;
+    if (precision == 1) return kDeclined;
+    if (a.Cout > 64 || (a.Cout & 3) || Ktot > 128 || Ktot < 8 || (a.C1 & 3) || (a.C2 & 3)) return kDeclined;
+    if (!aligned16(a.dY) || (a.bn.scale && !aligned16(a.H)) || (a.bn.act_ref && !aligned16(a.bn.act_ref))) return kDeclined;
+    if ((a.dX1 && (reinterpret_cast<uintptr_t>(a.dX1) & 7)) || (a.dX2 && (reinterpret_cast<uintptr_t>(a.dX2) & 7))) return kDeclined;
     const int Kpad = (int)ceil_div(a.Cout, BK) * BK;
     const bool x3 = precision != 2, ref = a.bn.scale && a.bn.act_ref;
-    *rc = CRF_OK;
     auto go = [&](auto bnv) {
         constexpr int BN = decltype(bnv)::value;
         constexpr int BM = 16 * (8 / (BN >= 64 ? 2 : 1));
         const int ntiles = (int)ceil_div(a.M, BM);
-        const int grid = std::min(ntiles, 2 * kNumSMs);
-        auto run = [&](auto kern, size_t smem) {
-            cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-            if (e == cudaSuccess) { kern<<<grid, kThreads, smem, st>>>(a, ntiles); e = cudaPeekAtLastError(); }
-            if (e != cudaSuccess) *rc = (int)e;
-        };
-        if (ref) { if (x3) run(dgrad2_kernel<BN, true, true>, dgrad2_smem<BN, true>(Kpad)); else run(dgrad2_kernel<BN, false, true>, dgrad2_smem<BN, true>(Kpad)); }
-        else     { if (x3) run(dgrad2_kernel<BN, true, false>, dgrad2_smem<BN, false>(Kpad)); else run(dgrad2_kernel<BN, false, false>, dgrad2_smem<BN, false>(Kpad)); }
-        return true;
+        const dim3 grid(std::min(ntiles, 2 * kNumSMs));
+        if (ref) return x3 ? launch<false>(dgrad2_kernel<BN, true, true>, grid, dim3(kThreads), dgrad2_smem<BN, true>(Kpad), st, a, ntiles)
+                           : launch<false>(dgrad2_kernel<BN, false, true>, grid, dim3(kThreads), dgrad2_smem<BN, true>(Kpad), st, a, ntiles);
+        return x3 ? launch<false>(dgrad2_kernel<BN, true, false>, grid, dim3(kThreads), dgrad2_smem<BN, false>(Kpad), st, a, ntiles)
+                  : launch<false>(dgrad2_kernel<BN, false, false>, grid, dim3(kThreads), dgrad2_smem<BN, false>(Kpad), st, a, ntiles);
     };
     if (Ktot > 64) return go(std::integral_constant<int, 128>{});
     if (Ktot > 32) return go(std::integral_constant<int, 64>{});
@@ -840,49 +801,37 @@ bool try_dgrad2(const DgradArgs& a, int precision, cudaStream_t st, int* rc) {
     return go(std::integral_constant<int, 8>{});
 }
 
-bool try_wgrad2(const WgradArgs& a, int precision, cudaStream_t st, int* rc) {
+int try_wgrad2(const WgradArgs& a, int precision, cudaStream_t st) {
     using namespace lin2;
     const int Ktot = a.C1 + a.C2;
-    if (precision == 1 || a.dbias) return false;
-    if (a.Cout > 64 || (a.Cout & 3) || Ktot > 128 || (a.C1 & 3) || (a.C2 & 3) || a.C1 == 0) return false;
-    if (!aligned16(a.dY) || (a.bn.scale && !aligned16(a.H)) || !aligned16(a.X1) || (a.C2 && !aligned16(a.X2))) return false;
-    if (a.bn.act_ref && !aligned16(a.bn.act_ref)) return false;
+    if (precision == 1 || a.dbias) return kDeclined;
+    if (a.Cout > 64 || (a.Cout & 3) || Ktot > 128 || (a.C1 & 3) || (a.C2 & 3) || a.C1 == 0) return kDeclined;
+    if (!aligned16(a.dY) || (a.bn.scale && !aligned16(a.H)) || !aligned16(a.X1) || (a.C2 && !aligned16(a.X2))) return kDeclined;
+    if (a.bn.act_ref && !aligned16(a.bn.act_ref)) return kDeclined;
     const bool x3 = precision != 2, ref = a.bn.scale && a.bn.act_ref;
-    *rc = CRF_OK;
     // square hidden-width products (GC, GM, second MLP layers): CUDA-core kernel
-    if (a.Cout == Ktot && a.C2 == 0 && (Ktot == 8 || Ktot == 16 || Ktot == 32)) {
+    if (a.Cout == 32 && Ktot == 32 && a.C2 == 0) {
         const int ntiles = (int)ceil_div(a.M, 128);
-        const int grid = std::min(ntiles, 4 * kNumSMs);
-        auto run = [&](auto kern) {
-            kern<<<grid, kThreads, 0, st>>>(a, ntiles);
-            cudaError_t e = cudaPeekAtLastError();
-            if (e != cudaSuccess) *rc = (int)e;
-        };
-        if (Ktot == 8) { if (ref) run(wgrad_small_kernel<8, true>); else run(wgrad_small_kernel<8, false>); }
-        else if (Ktot == 16) { if (ref) run(wgrad_small_kernel<16, true>); else run(wgrad_small_kernel<16, false>); }
-        else { if (ref) run(wgrad_small_kernel<32, true>); else run(wgrad_small_kernel<32, false>); }
-        return true;
+        const dim3 grid(std::min(ntiles, 4 * kNumSMs));
+        return ref ? launch<false>(wgrad_small_kernel<32, true>, grid, dim3(kThreads), 0, st, a, ntiles)
+                   : launch<false>(wgrad_small_kernel<32, false>, grid, dim3(kThreads), 0, st, a, ntiles);
     }
     const int CO = a.Cout <= 16 ? 16 : (a.Cout <= 32 ? 32 : 64);
     const int KP = Ktot <= 16 ? 16 : (Ktot <= 32 ? 32 : (Ktot <= 64 ? 64 : 128));
     const int ntiles = (int)ceil_div(a.M, RT);
-    const int grid = std::min(ntiles, 2 * kNumSMs);
-    auto run = [&](auto kern, size_t smem) {
-        cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e == cudaSuccess) { kern<<<grid, kThreads, smem, st>>>(a, ntiles); e = cudaPeekAtLastError(); }
-        if (e != cudaSuccess) *rc = (int)e;
-    };
-#define CRF_WG(co, kp)                                                                                                  \
-    if (CO == co && KP == kp) {                                                                                         \
-        if (ref) { if (x3) run(wgrad2_kernel<co, kp, true, true>, wgrad2_smem<co, kp, true>()); else run(wgrad2_kernel<co, kp, false, true>, wgrad2_smem<co, kp, true>()); } \
-        else     { if (x3) run(wgrad2_kernel<co, kp, true, false>, wgrad2_smem<co, kp, false>()); else run(wgrad2_kernel<co, kp, false, false>, wgrad2_smem<co, kp, false>()); } \
-        return true;                                                                                                    \
+    const dim3 grid(std::min(ntiles, 2 * kNumSMs));
+#define CRF_WG(co, kp)                                                                                                                       \
+    if (CO == co && KP == kp) {                                                                                                              \
+        if (ref) return x3 ? launch<false>(wgrad2_kernel<co, kp, true, true>, grid, dim3(kThreads), wgrad2_smem<co, kp, true>(), st, a, ntiles)     \
+                           : launch<false>(wgrad2_kernel<co, kp, false, true>, grid, dim3(kThreads), wgrad2_smem<co, kp, true>(), st, a, ntiles);   \
+        return x3 ? launch<false>(wgrad2_kernel<co, kp, true, false>, grid, dim3(kThreads), wgrad2_smem<co, kp, false>(), st, a, ntiles)            \
+                  : launch<false>(wgrad2_kernel<co, kp, false, false>, grid, dim3(kThreads), wgrad2_smem<co, kp, false>(), st, a, ntiles);          \
     }
     CRF_WG(64, 128) CRF_WG(64, 64) CRF_WG(64, 32) CRF_WG(64, 16)
     CRF_WG(32, 128) CRF_WG(32, 64) CRF_WG(32, 32)
     CRF_WG(16, 128) CRF_WG(16, 64)
 #undef CRF_WG
-    return false;
+    return kDeclined;
 }
 
 }  // namespace lin

@@ -8,7 +8,8 @@
 //   * contractions on mma.sync m16n8k16 bf16 with bf16x3 error compensation: a·b ≈ a_hi·b_hi + a_hi·b_lo + a_lo·b_hi,
 //     16 mantissa bits per operand → relative error ≈ 2^-16, well inside the 1e-3 parity budget, at twice the MAC rate of
 //     3xTF32 on this part (measured: 557 vs 278 TFLOP/s dense for single-pass bf16 / tf32 mma.sync, profiles/).
-//     PREC = 1 selects a single bf16 pass (stated tolerance 2e-2, see DESIGN.md).
+//     precision 2 selects a single bf16 pass (stated tolerance 2e-2, see DESIGN.md §5); fwd2_kernel exists only in that form,
+//     the fp32-grade forward is the 3xTF32 fwd2t_kernel.
 #pragma once
 #include <cuda_bf16.h>
 
@@ -52,8 +53,6 @@ __device__ __forceinline__ void mma3(float (&d)[4], const uint32_t (&ah)[4], con
     }
     mma_bf16(d, ah, bh0, bh1);
 }
-
-__device__ __forceinline__ float lrelu(float v, float slope) { return v > 0.0f ? v : v * slope; }
 
 }  // namespace lin2
 }  // namespace crf

@@ -17,7 +17,6 @@
 // HBM (rows × (Ktot + Cout) × 4 bytes); the MMAs of a tile take ≈0.8 us of the ≈1.9 us the tile's bytes need.
 #include <algorithm>
 #include <cstdlib>
-#include <type_traits>
 
 #include "common.cuh"
 #include "linear_args.cuh"
@@ -54,8 +53,6 @@ __device__ __forceinline__ void trace(int ev, int idx) {      // fixed record sl
 #else
 #define CRF_TRACE(ev, idx)
 #endif
-
-__device__ __forceinline__ float lrelu(float v, float slope) { return v > 0.0f ? v : v * slope; }
 
 template <int BN>
 struct Layout {
@@ -369,8 +366,6 @@ __global__ void __launch_bounds__(kThreads, 1) fwd3_kernel(const FwdArgs a, cons
     }
 }
 
-inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
-
 }  // namespace lin3
 
 #ifdef CRF_FWD3_TRACE
@@ -388,31 +383,21 @@ extern "C" int crfconv_debug_fwd3_trace(long long* out, int max_records, int res
 namespace lin {
 
 // tcgen05 forward: fp32-grade precision only (3xTF32); shapes of the hot path (Cout <= 64, <= 4 slabs of 32 input channels)
-bool try_fwd3(const FwdArgs& a, int precision, cudaStream_t st, int* rc) {
+int try_fwd3(const FwdArgs& a, int precision, cudaStream_t st) {
     using namespace lin3;
-    if (precision != 0) return false;
-    if (a.idx1 || (a.scale1 && !(a.slope1 >= 0.f && a.slope1 <= 1.f))) return false;   // gathered rows / expanding slopes: older kernels
-    if (a.Cout > 64 || (a.Cout & 3) || (a.C1 & 3) || (a.C2 & 3) || a.C1 <= 0) return false;
+    if (precision != 0) return kDeclined;
+    if (a.idx1 || (a.scale1 && !(a.slope1 >= 0.f && a.slope1 <= 1.f))) return kDeclined;   // gathered rows / expanding slopes: older kernels
+    if (a.Cout > 64 || (a.Cout & 3) || (a.C1 & 3) || (a.C2 & 3) || a.C1 <= 0) return kDeclined;
     const int nch = (a.C1 + BK - 1) / BK + (a.C2 + BK - 1) / BK;
-    if (nch > 4) return false;
-    if (!aligned16(a.X1) || (a.C2 && !aligned16(a.X2)) || !aligned16(a.Y)) return false;
+    if (nch > 4) return kDeclined;
+    if (!aligned16(a.X1) || (a.C2 && !aligned16(a.X2)) || !aligned16(a.Y)) return kDeclined;
     const int ntiles = (int)ceil_div(a.M, BM);
-    if (ntiles <= 0) return false;
-    *rc = CRF_OK;
-    auto go = [&](auto bnv) {
-        constexpr int BN = decltype(bnv)::value;
-        const size_t smem = Layout<BN>::bytes(nch);
-        cudaError_t e = cudaFuncSetAttribute(fwd3_kernel<BN>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e == cudaSuccess) {
-            e = launch_k(fwd3_kernel<BN>, dim3(std::min(ntiles, kNumSMs)), dim3(kThreads), smem, st, a, ntiles);
-        }
-        if (e != cudaSuccess) *rc = (int)e;
-        return true;
-    };
-    if (a.fin.part && (a.fin.part != a.stats || (a.Cout != 64 && a.Cout != 32 && a.Cout != 16))) return false;   // fused finalize: Cout == BN only
-    if (a.Cout > 32) return go(std::integral_constant<int, 64>{});
-    if (a.Cout > 16) return go(std::integral_constant<int, 32>{});
-    return go(std::integral_constant<int, 16>{});
+    if (ntiles <= 0) return kDeclined;
+    if (a.fin.part && (a.fin.part != a.stats || (a.Cout != 64 && a.Cout != 32 && a.Cout != 16))) return kDeclined;   // fused finalize: Cout == BN only
+    const dim3 grid(std::min(ntiles, kNumSMs));
+    if (a.Cout > 32) return launch<true>(fwd3_kernel<64>, grid, dim3(kThreads), Layout<64>::bytes(nch), st, a, ntiles);
+    if (a.Cout > 16) return launch<true>(fwd3_kernel<32>, grid, dim3(kThreads), Layout<32>::bytes(nch), st, a, ntiles);
+    return launch<true>(fwd3_kernel<16>, grid, dim3(kThreads), Layout<16>::bytes(nch), st, a, ntiles);
 }
 
 }  // namespace lin

@@ -33,6 +33,7 @@ namespace lin3b {
 
 using lin::DgradArgs;
 using lin::WgradArgs;
+using lin::lrelu;
 using namespace umma;
 
 // 13 warps: 4 of them on one SM sub-partition leave 128 registers per thread (17 warps would leave 96, and the producers spill)
@@ -53,17 +54,6 @@ constexpr uint32_t kTmemCols = 256;
 static_assert(2 * BN + kStages * 2 * RS <= (int)kTmemCols, "TMEM columns");
 constexpr size_t kSmemBytes = (size_t)kStages * kStageBytes + kWBytes + (size_t)(4 * BN + 2 * 128) * 4 + (2 * kStages + 2 * kStages) * 8 + 16;
 static_assert(kSmemBytes <= 227 * 1024, "shared memory");
-
-__device__ __forceinline__ float lrelu(float v, float slope) { return v > 0.0f ? v : v * slope; }
-
-// byte offset of the 16-byte chunk c16 (0..7) of line r inside a SWIZZLE_128B_BASE32B block (32-byte chunks XOR (r & 3))
-__device__ __forceinline__ uint32_t blk_off(int r, int c16) { return (uint32_t)(r * 128 + ((((c16 >> 1) ^ (r & 3)) << 5) | ((c16 & 1) << 4))); }
-
-// MN-major SWIZZLE_128B_BASE32B descriptor: LBO = stride between 32-channel blocks, SBO = 512 B between 4-line atoms
-__device__ __forceinline__ uint64_t desc_mn(uint32_t saddr, uint32_t lbo_bytes) {
-    return (uint64_t)((saddr >> 4) & 0x3FFF) | ((uint64_t)((lbo_bytes >> 4) & 0x3FFF) << 16) | ((uint64_t)(512 >> 4) << 32) | ((uint64_t)1 << 46) |
-           ((uint64_t)1 << 61);
-}
 
 __global__ void __launch_bounds__(kThreads, 1) bwd3_kernel(const DgradArgs d, const WgradArgs a, const int ntiles) {
     extern __shared__ __align__(1024) uint8_t smem[];
@@ -118,14 +108,8 @@ __global__ void __launch_bounds__(kThreads, 1) bwd3_kernel(const DgradArgs d, co
     }
     pdl_wait();
     for (int k = tid; k < BN; k += kThreads) {
-        float sc = 1.f, sh = 0.f, pz = 0.f, pw = 0.f;
-        if (!plain && k < C) {
-            sc = __ldg(a.bn.scale + k); sh = __ldg(a.bn.shift + k);
-            const float mu = __ldg(a.bn.mean + k), is = __ldg(a.bn.invstd + k), k1 = __ldg(a.bn.k1 + k), k2 = __ldg(a.bn.k2 + k);
-            pz = -sc * is * k2;
-            pw = -sc * k1 + sc * is * k2 * mu;
-        }
-        s_par[k] = sc; s_par[BN + k] = sh; s_par[2 * BN + k] = pz; s_par[3 * BN + k] = pw;
+        const float4 p = (!plain && k < C) ? a.bn.coef(k) : make_float4(1.f, 0.f, 0.f, 0.f);
+        s_par[k] = p.x; s_par[BN + k] = p.y; s_par[2 * BN + k] = p.z; s_par[3 * BN + k] = p.w;
     }
     for (int k = tid; k < 128; k += kThreads) {
         float sc = 1.f, sh = 0.f;
@@ -389,28 +373,23 @@ __global__ void __launch_bounds__(kThreads, 1) bwd3_kernel(const DgradArgs d, co
     if (warp == 0) tmem_dealloc(tmem, kTmemCols);
 }
 
-inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
-
 }  // namespace lin3b
 
 namespace lin {
 
-bool try_bwd3(const DgradArgs& d, const WgradArgs& w, int precision, cudaStream_t st, int* rc) {
+int try_bwd3(const DgradArgs& d, const WgradArgs& w, int precision, cudaStream_t st) {
     using namespace lin3b;
-    if (precision != 0) return false;
-    if (!w.dW || (!d.dX1 && !d.dX2)) return false;
-    if (w.idx1 || w.dbias || w.bn.act_ref) return false;
-    if (w.Cout <= 32 || w.Cout > BN || (w.Cout & 3) || (w.C1 & 3) || (w.C2 & 3) || w.C1 <= 0) return false;
+    if (precision != 0) return kDeclined;
+    if (!w.dW || (!d.dX1 && !d.dX2)) return kDeclined;
+    if (w.idx1 || w.dbias || w.bn.act_ref) return kDeclined;
+    if (w.Cout <= 32 || w.Cout > BN || (w.Cout & 3) || (w.C1 & 3) || (w.C2 & 3) || w.C1 <= 0) return kDeclined;
     const int Ktot = w.C1 + w.C2;
-    if (Ktot <= 64 || Ktot > 128 || (w.C1 + 31) / 32 + (w.C2 + 31) / 32 > kXBlocks) return false;
-    if (!aligned16(w.dY) || !aligned16(w.X1) || (w.C2 && !aligned16(w.X2)) || (w.bn.scale && !aligned16(w.H))) return false;
-    if ((d.dX1 && !aligned16(d.dX1)) || (d.dX2 && !aligned16(d.dX2))) return false;
+    if (Ktot <= 64 || Ktot > 128 || (w.C1 + 31) / 32 + (w.C2 + 31) / 32 > kXBlocks) return kDeclined;
+    if (!aligned16(w.dY) || !aligned16(w.X1) || (w.C2 && !aligned16(w.X2)) || (w.bn.scale && !aligned16(w.H))) return kDeclined;
+    if ((d.dX1 && !aligned16(d.dX1)) || (d.dX2 && !aligned16(d.dX2))) return kDeclined;
     const int ntiles = (int)ceil_div(w.M, RS);
-    if (ntiles <= 0) return false;
-    cudaError_t e = cudaFuncSetAttribute(bwd3_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemBytes);
-    if (e == cudaSuccess) e = launch_k(bwd3_kernel, dim3(std::min(ntiles, kNumSMs)), dim3(kThreads), kSmemBytes, st, d, w, ntiles);
-    *rc = e == cudaSuccess ? CRF_OK : (int)e;
-    return true;
+    if (ntiles <= 0) return kDeclined;
+    return launch<true>(bwd3_kernel, dim3(std::min(ntiles, kNumSMs)), dim3(kThreads), kSmemBytes, st, d, w, ntiles);
 }
 
 }  // namespace lin

@@ -9,7 +9,6 @@
 // What bounds it: rows × (2·Cout + Ktot) × 4 bytes of HBM traffic (dY, H read; dX written).
 #include <algorithm>
 #include <cstdlib>
-#include <type_traits>
 
 #include "common.cuh"
 #include "linear_args.cuh"
@@ -29,18 +28,13 @@ constexpr int BM = 128, BK = 32, RING = 3;
 static_assert(kGroups == RING, "group g owns ring slot g");
 constexpr int kSlabBytes = BM * 128, kSlotBytes = 2 * kSlabBytes;
 constexpr int kStageCols = 64, kStageLd = kStageCols + 4;        // the epilogue handles the accumulator in column blocks of 64
+constexpr int BN = 128;                                          // N = input channels, padded (64 < Ktot <= 128)
+constexpr uint32_t kTmemCols = 2 * BN;
+inline size_t smem_bytes(int nch) {
+    return (size_t)RING * kSlotBytes + (size_t)2 * nch * BN * 128 + (size_t)BM * kStageLd * 4 + (size_t)4 * nch * BK * 4 + (size_t)(2 * RING + 4) * 8 + 16;
+}
 
-template <int BN>
-struct Layout {
-    static constexpr uint32_t kTmemCols = 2 * BN < 32 ? 32 : 2 * BN;
-    static size_t bytes(int nch) {
-        return (size_t)RING * kSlotBytes + (size_t)2 * nch * BN * 128 + (size_t)BM * kStageLd * 4 + (size_t)4 * nch * BK * 4 + (size_t)(2 * RING + 4) * 8 + 16;
-    }
-};
-
-template <int BN>
 __global__ void __launch_bounds__(kThreads, 1) dgrad3_kernel(const DgradArgs a, const int ntiles) {
-    using L = Layout<BN>;
     extern __shared__ __align__(1024) uint8_t smem[];
     const int C = a.Cout, Ktot = a.C1 + a.C2;
     const int nch = (C + BK - 1) / BK, Kpad = nch * BK;               // K dimension = output channels of the layer
@@ -58,7 +52,7 @@ __global__ void __launch_bounds__(kThreads, 1) dgrad3_kernel(const DgradArgs a, 
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const bool plain = a.bn.scale == nullptr;
     pdl_trigger();
-    if (warp == 0) tmem_alloc(tmem_slot, L::kTmemCols);
+    if (warp == 0) tmem_alloc(tmem_slot, kTmemCols);
     if (tid == kEpiWarps * 32) {
         for (int i = 0; i < RING; ++i) { mbar_init(full + i, 1); mbar_init(empty + i, 1); }
         for (int i = 0; i < 2; ++i) { mbar_init(tfull + i, 1); mbar_init(tempty + i, kEpiWarps); }
@@ -93,14 +87,8 @@ __global__ void __launch_bounds__(kThreads, 1) dgrad3_kernel(const DgradArgs a, 
     }
     pdl_wait();                                                    // W is a parameter; the BatchNorm constants, dY and H are upstream results
     for (int k = tid; k < Kpad; k += kThreads) {
-        float sc = 1.f, sh = 0.f, pz = 0.f, pw = 0.f;
-        if (!plain && k < C) {
-            sc = __ldg(a.bn.scale + k); sh = __ldg(a.bn.shift + k);
-            const float mu = __ldg(a.bn.mean + k), is = __ldg(a.bn.invstd + k), k1 = __ldg(a.bn.k1 + k), k2 = __ldg(a.bn.k2 + k);
-            pz = -sc * is * k2;
-            pw = -sc * k1 + sc * is * k2 * mu;
-        }
-        s_par[k] = sc; s_par[Kpad + k] = sh; s_par[2 * Kpad + k] = pz; s_par[3 * Kpad + k] = pw;
+        const float4 p = (!plain && k < C) ? a.bn.coef(k) : make_float4(1.f, 0.f, 0.f, 0.f);
+        s_par[k] = p.x; s_par[Kpad + k] = p.y; s_par[2 * Kpad + k] = p.z; s_par[3 * Kpad + k] = p.w;
     }
     fence_async_smem();
     tc_fence_before();
@@ -246,42 +234,25 @@ __global__ void __launch_bounds__(kThreads, 1) dgrad3_kernel(const DgradArgs a, 
     }
     tc_fence_before();
     __syncthreads();
-    if (warp == 0) tmem_dealloc(tmem, L::kTmemCols);
+    if (warp == 0) tmem_dealloc(tmem, kTmemCols);
 }
-
-inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
 
 }  // namespace lin3d
 
 namespace lin {
 
-bool try_dgrad3(const DgradArgs& a, int precision, cudaStream_t st, int* rc) {
+int try_dgrad3(const DgradArgs& a, int precision, cudaStream_t st) {
     using namespace lin3d;
-    if (precision != 0) return false;
+    if (precision != 0) return kDeclined;
     const int Ktot = a.C1 + a.C2;
-    if (a.Cout > 64 || (a.Cout & 3) || Ktot > 128 || Ktot < 16 || (a.C1 & 3) || (a.C2 & 3) || a.bn.act_ref) return false;
-    if (!aligned16(a.dY) || (a.bn.scale && !aligned16(a.H))) return false;
-    if ((a.dX1 && !aligned16(a.dX1)) || (a.dX2 && !aligned16(a.dX2))) return false;
-    if (!a.dX1 && !a.dX2) return false;
-    if (Ktot <= 64 || a.Cout <= 32) return false;      // narrower products: the mma.sync kernel is as fast or faster (measured)
+    if (a.Cout > 64 || (a.Cout & 3) || Ktot > BN || (a.C1 & 3) || (a.C2 & 3) || a.bn.act_ref) return kDeclined;
+    if (!aligned16(a.dY) || (a.bn.scale && !aligned16(a.H))) return kDeclined;
+    if ((a.dX1 && !aligned16(a.dX1)) || (a.dX2 && !aligned16(a.dX2))) return kDeclined;
+    if (!a.dX1 && !a.dX2) return kDeclined;
+    if (Ktot <= 64 || a.Cout <= 32) return kDeclined;  // narrower products: the mma.sync kernel is as fast or faster (measured)
     const int ntiles = (int)ceil_div(a.M, BM);
-    if (ntiles <= 0) return false;
-    const int nch = (a.Cout + BK - 1) / BK;
-    *rc = CRF_OK;
-    auto go = [&](auto bnv) {
-        constexpr int BN = decltype(bnv)::value;
-        const size_t smem = Layout<BN>::bytes(nch);
-        cudaError_t e = cudaFuncSetAttribute(dgrad3_kernel<BN>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e == cudaSuccess) {
-            e = launch_k(dgrad3_kernel<BN>, dim3(std::min(ntiles, kNumSMs)), dim3(kThreads), smem, st, a, ntiles);
-        }
-        if (e != cudaSuccess) *rc = (int)e;
-        return true;
-    };
-    if (Ktot > 64) return go(std::integral_constant<int, 128>{});
-    if (Ktot > 32) return go(std::integral_constant<int, 64>{});
-    if (Ktot > 16) return go(std::integral_constant<int, 32>{});
-    return go(std::integral_constant<int, 16>{});
+    if (ntiles <= 0) return kDeclined;
+    return launch<true>(dgrad3_kernel, dim3(std::min(ntiles, kNumSMs)), dim3(kThreads), smem_bytes((a.Cout + BK - 1) / BK), st, a, ntiles);
 }
 
 }  // namespace lin

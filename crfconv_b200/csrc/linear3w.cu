@@ -17,7 +17,6 @@
 //   warps 0..3   epilogue  : once per CTA, tcgen05.ld of dWᵀ and atomic adds into dW[slot][co][k].
 // What bounds it: reading dY, H and X once from HBM (rows × (2·Cout + Ktot) × 4 bytes).
 #include <algorithm>
-#include <type_traits>
 
 #include "common.cuh"
 #include "linear_args.cuh"
@@ -27,6 +26,7 @@ namespace crf {
 namespace lin3w {
 
 using lin::WgradArgs;
+using lin::lrelu;
 using namespace umma;
 
 constexpr int kEpiWarps = 4, kProdWarps = 12, kGroupWarps = 2, kGroups = kProdWarps / kGroupWarps;
@@ -34,17 +34,6 @@ constexpr int kThreads = (kEpiWarps + 1 + kProdWarps) * 32;      // 544
 constexpr int RS = 64;                                           // rows per stage
 constexpr int kBlockBytes = RS * 128;                            // one [64 rows × 32 channels] fp32 block
 constexpr int kXBlocks = 4;                                      // M = 128 input channels (zero blocks beyond Ktot)
-
-__device__ __forceinline__ float lrelu(float v, float slope) { return v > 0.0f ? v : v * slope; }
-
-// byte offset of the 16-byte chunk c16 (0..7) of row r inside a block (SWIZZLE_128B_BASE32B: 32-byte chunks XOR (r & 3))
-__device__ __forceinline__ uint32_t blk_off(int r, int c16) { return (uint32_t)(r * 128 + ((((c16 >> 1) ^ (r & 3)) << 5) | ((c16 & 1) << 4))); }
-
-// MN-major SWIZZLE_128B_BASE32B descriptor: LBO = stride between 32-channel blocks, SBO = 512 B between 4-row atoms
-__device__ __forceinline__ uint64_t desc_mn(uint32_t saddr, uint32_t lbo_bytes) {
-    return (uint64_t)((saddr >> 4) & 0x3FFF) | ((uint64_t)((lbo_bytes >> 4) & 0x3FFF) << 16) | ((uint64_t)(512 >> 4) << 32) | ((uint64_t)1 << 46) |
-           ((uint64_t)1 << 61);
-}
 
 template <int BN>
 struct Layout {
@@ -83,14 +72,8 @@ __global__ void __launch_bounds__(kThreads, 1) wgrad3_kernel(const WgradArgs a, 
     }
     pdl_wait();
     for (int k = tid; k < BN; k += kThreads) {
-        float sc = 1.f, sh = 0.f, pz = 0.f, pw = 0.f;
-        if (!plain && k < C) {
-            sc = __ldg(a.bn.scale + k); sh = __ldg(a.bn.shift + k);
-            const float mu = __ldg(a.bn.mean + k), is = __ldg(a.bn.invstd + k), k1 = __ldg(a.bn.k1 + k), k2 = __ldg(a.bn.k2 + k);
-            pz = -sc * is * k2;
-            pw = -sc * k1 + sc * is * k2 * mu;
-        }
-        s_par[k] = sc; s_par[BN + k] = sh; s_par[2 * BN + k] = pz; s_par[3 * BN + k] = pw;
+        const float4 p = (!plain && k < C) ? a.bn.coef(k) : make_float4(1.f, 0.f, 0.f, 0.f);
+        s_par[k] = p.x; s_par[BN + k] = p.y; s_par[2 * BN + k] = p.z; s_par[3 * BN + k] = p.w;
     }
     for (int k = tid; k < 128; k += kThreads) {
         float sc = 1.f, sh = 0.f;
@@ -262,36 +245,24 @@ __global__ void __launch_bounds__(kThreads, 1) wgrad3_kernel(const WgradArgs a, 
     if (warp == 0) tmem_dealloc(tmem, L::kTmemCols);
 }
 
-inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
-
 }  // namespace lin3w
 
 namespace lin {
 
-bool try_wgrad3(const WgradArgs& a, int precision, cudaStream_t st, int* rc) {
+int try_wgrad3(const WgradArgs& a, int precision, cudaStream_t st) {
     using namespace lin3w;
-    if (precision != 0) return false;
-    if (a.idx1 || a.dbias || a.bn.act_ref) return false;
-    if (a.Cout > 64 || (a.Cout & 3) || (a.C1 & 3) || (a.C2 & 3) || a.C1 <= 0) return false;
-    if ((a.C1 + 31) / 32 + (a.C2 + 31) / 32 > kXBlocks) return false;
-    if (a.C1 + a.C2 <= 64) return false;        // narrow inputs: M is padded to 128 anyway and the mma.sync kernels are as fast (measured)
-    if (!aligned16(a.dY) || !aligned16(a.X1) || (a.C2 && !aligned16(a.X2))) return false;
-    if (a.bn.scale && !aligned16(a.H)) return false;
+    if (precision != 0) return kDeclined;
+    if (a.idx1 || a.dbias || a.bn.act_ref) return kDeclined;
+    if (a.Cout > 64 || (a.Cout & 3) || (a.C1 & 3) || (a.C2 & 3) || a.C1 <= 0) return kDeclined;
+    if ((a.C1 + 31) / 32 + (a.C2 + 31) / 32 > kXBlocks) return kDeclined;
+    if (a.C1 + a.C2 <= 64) return kDeclined;    // narrow inputs: M is padded to 128 anyway and the mma.sync kernels are as fast (measured)
+    if (!aligned16(a.dY) || !aligned16(a.X1) || (a.C2 && !aligned16(a.X2))) return kDeclined;
+    if (a.bn.scale && !aligned16(a.H)) return kDeclined;
     const int ntiles = (int)ceil_div(a.M, RS);
-    if (ntiles <= 0) return false;
-    *rc = CRF_OK;
-    auto go = [&](auto bnv) {
-        constexpr int BN = decltype(bnv)::value;
-        const size_t smem = Layout<BN>::bytes();
-        cudaError_t e = cudaFuncSetAttribute(wgrad3_kernel<BN>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e == cudaSuccess) {
-            e = launch_k(wgrad3_kernel<BN>, dim3(std::min(ntiles, kNumSMs)), dim3(kThreads), smem, st, a, ntiles);
-        }
-        if (e != cudaSuccess) *rc = (int)e;
-        return true;
-    };
-    if (a.Cout > 32) return go(std::integral_constant<int, 64>{});
-    return go(std::integral_constant<int, 32>{});
+    if (ntiles <= 0) return kDeclined;
+    const dim3 grid(std::min(ntiles, kNumSMs));
+    if (a.Cout > 32) return launch<true>(wgrad3_kernel<64>, grid, dim3(kThreads), Layout<64>::bytes(), st, a, ntiles);
+    return launch<true>(wgrad3_kernel<32>, grid, dim3(kThreads), Layout<32>::bytes(), st, a, ntiles);
 }
 
 }  // namespace lin

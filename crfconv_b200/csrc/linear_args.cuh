@@ -1,4 +1,4 @@
-// Argument blocks shared by the generic (linear.cu) and fast-path (linear2.cu) Linear kernels.
+// Argument blocks, device helpers and the launcher protocol shared by the Linear kernel families (linear*.cu).
 #pragma once
 #include <cstdint>
 
@@ -6,6 +6,9 @@
 
 namespace crf {
 namespace lin {
+
+__device__ __forceinline__ float lrelu(float v, float slope) { return v > 0.0f ? v : v * slope; }
+inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
 
 struct FwdArgs {
     const float* X1; int C1;                      // segment 1: [M, C1] (row-gathered through idx1 when given)
@@ -30,6 +33,14 @@ struct BnBwd {
     const float* k2;       // mean over rows of dV·Ĥ
     const float* act_ref;  // [M, C] saved activation output whose sign selects the LeakyReLU branch (null ⇒ use V)
     float slope;           // 1 ⇒ no activation
+
+    // Channel c's constants of dH = sc·dV + pz·H + pw, returned as (sc, sh, pz, pw):
+    // pz = −sc·istd·k2, pw = −sc·k1 + sc·istd·k2·mean; the LeakyReLU branch of dV is selected by sc·H + sh.
+    __device__ __forceinline__ float4 coef(int c) const {
+        const float sc = __ldg(scale + c), sh = __ldg(shift + c), mu = __ldg(mean + c), is = __ldg(invstd + c);
+        const float q1 = __ldg(k1 + c), q2 = __ldg(k2 + c);
+        return make_float4(sc, sh, -sc * is * q2, -sc * q1 + sc * is * q2 * mu);
+    }
 };
 
 struct DgradArgs {
@@ -52,27 +63,49 @@ struct WgradArgs {
     int64_t slot_stride;  // 0, or Cout·Ktot when dW points at [kGradSlots][Cout·Ktot] partial slots
 };
 
-// fast-path launchers (linear2.cu); return true when the shape was handled
-bool try_fwd2(const FwdArgs& a, int precision, cudaStream_t st, int* rc);
-bool try_dgrad2(const DgradArgs& a, int precision, cudaStream_t st, int* rc);
-bool try_wgrad2(const WgradArgs& a, int precision, cudaStream_t st, int* rc);
-// tcgen05 / TMEM forward (linear3.cu)
-bool try_fwd3(const FwdArgs& a, int precision, cudaStream_t st, int* rc);
-bool try_wgrad3(const WgradArgs& a, int precision, cudaStream_t st, int* rc);   // linear3w.cu
-bool try_dgrad3(const DgradArgs& a, int precision, cudaStream_t st, int* rc);   // linear3d.cu
+// Launchers.  Each try_* returns kDeclined when the call is outside its family's shape range (the dispatch in linear.cu then
+// tries the next family), else the status of its launch: CRF_OK or a cudaError_t.
+constexpr int kDeclined = -1000;   // below every CRF_ERR_* code; cudaError_t values are >= 0
+
+// Raises kernel's dynamic shared-memory limit to smem (when smem > 0), launches it and returns CRF_OK or the CUDA error.
+// PDL = true launches through launch_k (common.cuh): only for kernels that execute pdl_wait().  The others are launched
+// plainly and must never carry the programmatic-serialization attribute.
+template <bool PDL, typename... KArgs, typename... Args>
+inline int launch(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args&&... args) {
+    cudaError_t e = cudaSuccess;
+    if (smem > 0) e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e == cudaSuccess) {
+        if constexpr (PDL) {
+            e = launch_k(kernel, grid, block, smem, st, static_cast<Args&&>(args)...);
+        } else {
+            kernel<<<grid, block, smem, st>>>(static_cast<KArgs>(args)...);
+            e = cudaPeekAtLastError();
+        }
+    }
+    return e == cudaSuccess ? CRF_OK : (int)e;
+}
+
+// tcgen05 / TMEM (linear3*.cu): forward, weight gradient, input gradient
+int try_fwd3(const FwdArgs& a, int precision, cudaStream_t st);
+int try_wgrad3(const WgradArgs& a, int precision, cudaStream_t st);
+int try_dgrad3(const DgradArgs& a, int precision, cudaStream_t st);
 // input and weight gradient in one pass (linear3b.cu); needs dW and at least one of dX1 / dX2
-bool try_bwd3(const DgradArgs& d, const WgradArgs& w, int precision, cudaStream_t st, int* rc);
+int try_bwd3(const DgradArgs& d, const WgradArgs& w, int precision, cudaStream_t st);
+// persistent cp.async kernels (linear2.cu)
+int try_fwd2(const FwdArgs& a, int precision, cudaStream_t st);
+int try_dgrad2(const DgradArgs& a, int precision, cudaStream_t st);
+int try_wgrad2(const WgradArgs& a, int precision, cudaStream_t st);
 // narrow layers over many rows: operands straight from global memory in fragment order (linear_direct.cu)
-bool try_wgrad_direct(const WgradArgs& a, cudaStream_t st, int* rc);
-bool try_upproj_fwd(const FwdArgs& a, cudaStream_t st, int* rc);      // narrow input → wide output (output-bound streams)
-bool try_upproj_dgrad(const DgradArgs& a, cudaStream_t st, int* rc);
+int try_wgrad_direct(const WgradArgs& a, cudaStream_t st);
+int try_upproj_fwd(const FwdArgs& a, cudaStream_t st);      // narrow input → wide output (output-bound streams)
+int try_upproj_dgrad(const DgradArgs& a, cudaStream_t st);
 // few rows, wide channels (deep levels): 32-row tiles with register prefetch (linear_small.cu)
-bool try_fwd_small(const FwdArgs& a, cudaStream_t st, int* rc);
-bool try_dgrad_small(const DgradArgs& a, cudaStream_t st, int* rc);
-bool try_wgrad_rows(WgradArgs a, cudaStream_t st, int* rc);
+int try_fwd_small(const FwdArgs& a, cudaStream_t st);
+int try_dgrad_small(const DgradArgs& a, cudaStream_t st);
+int try_wgrad_rows(WgradArgs a, cudaStream_t st);
 // CUDA-core kernels for hidden-width layers (linear_narrow.cu); w == nullptr ⇒ dgrad only
-bool try_narrow_fwd(const FwdArgs& a, cudaStream_t st, int* rc);
-bool try_narrow_bwd(const DgradArgs& d, const WgradArgs* w, cudaStream_t st, int* rc);
+int try_narrow_fwd(const FwdArgs& a, cudaStream_t st);
+int try_narrow_bwd(const DgradArgs& d, const WgradArgs* w, cudaStream_t st);
 
 }  // namespace lin
 }  // namespace crf

@@ -38,13 +38,7 @@ __global__ void __launch_bounds__(kThreads, MB * NB > 4 ? 1 : 2) wgrad_direct_ke
     const bool plain = a.bn.scale == nullptr;
     for (int i = tid; i < CO * KP; i += kThreads) s_w[i] = 0.f;
     for (int k = tid; k < CO; k += kThreads) {
-        float4 pr = make_float4(1.f, 0.f, 0.f, 0.f);
-        if (!plain && k < C) {
-            const float sc = __ldg(a.bn.scale + k), sh = __ldg(a.bn.shift + k), mu = __ldg(a.bn.mean + k), is = __ldg(a.bn.invstd + k);
-            const float k1 = __ldg(a.bn.k1 + k), k2 = __ldg(a.bn.k2 + k);
-            pr = make_float4(sc, sh, -sc * is * k2, -sc * k1 + sc * is * k2 * mu);
-        }
-        s_par[k] = pr;
+        s_par[k] = (!plain && k < C) ? a.bn.coef(k) : make_float4(1.f, 0.f, 0.f, 0.f);
         s_b[k] = 0.f;
     }
     for (int k = tid; k < KP; k += kThreads) {
@@ -176,35 +170,30 @@ __global__ void __launch_bounds__(kThreads, MB * NB > 4 ? 1 : 2) wgrad_direct_ke
 }
 
 template <int MB, int NB>
-inline int launch(const WgradArgs& a, cudaStream_t st) {
+inline int run(const WgradArgs& a, cudaStream_t st) {
     constexpr int per_sm = MB * NB > 4 ? 1 : 2;
     const int64_t tiles = ceil_div(a.M, 16);
     const unsigned grid = (unsigned)std::max<int64_t>(1, std::min<int64_t>(ceil_div(tiles, kWarps), (int64_t)kNumSMs * per_sm));
-    wgrad_direct_kernel<MB, NB><<<grid, kThreads, 0, st>>>(a);
-    const cudaError_t e = cudaPeekAtLastError();
-    return e == cudaSuccess ? CRF_OK : (int)e;
+    return launch<false>(wgrad_direct_kernel<MB, NB>, dim3(grid), dim3(kThreads), 0, st, a);
 }
 
 }  // namespace dw
 
-bool try_wgrad_direct(const WgradArgs& a, cudaStream_t st, int* rc) {
+int try_wgrad_direct(const WgradArgs& a, cudaStream_t st) {
     const int Ktot = a.C1 + a.C2;
-    if (a.bn.scale && a.bn.act_ref) return false;               // saved-activation branch selection: tiled kernels
-    if (a.Cout < 1 || a.Cout > 128 || Ktot < 1 || Ktot > 128 || a.C1 < 1 || a.M < 1) return false;
+    if (a.bn.scale && a.bn.act_ref) return kDeclined;           // saved-activation branch selection: tiled kernels
+    if (a.Cout < 1 || a.Cout > 128 || Ktot < 1 || Ktot > 128 || a.C1 < 1 || a.M < 1) return kDeclined;
     const int mb = a.Cout <= 16 ? 1 : (a.Cout <= 32 ? 2 : (a.Cout <= 64 ? 4 : 8));
     const int nb = Ktot <= 8 ? 1 : (Ktot <= 16 ? 2 : (Ktot <= 32 ? 4 : (Ktot <= 64 ? 8 : 16)));
-    if (mb * nb > 32) return false;
-#define CRF_DW(m, n)                         \
-    if (mb == m && nb == n) {                \
-        *rc = dw::launch<m, n>(a, st);       \
-        return true;                         \
-    }
+    if (mb * nb > 32) return kDeclined;
+#define CRF_DW(m, n) \
+    if (mb == m && nb == n) return dw::run<m, n>(a, st);
     CRF_DW(1, 1) CRF_DW(1, 2) CRF_DW(1, 4) CRF_DW(1, 8) CRF_DW(1, 16)
     CRF_DW(2, 1) CRF_DW(2, 2) CRF_DW(2, 4) CRF_DW(2, 8) CRF_DW(2, 16)
     CRF_DW(4, 1) CRF_DW(4, 2) CRF_DW(4, 4) CRF_DW(4, 8)
     CRF_DW(8, 1) CRF_DW(8, 2) CRF_DW(8, 4)
 #undef CRF_DW
-    return false;
+    return kDeclined;
 }
 
 }  // namespace lin
@@ -354,46 +343,41 @@ __global__ void __launch_bounds__(kThreads, NP > 64 ? 1 : 2) upproj_kernel(const
 }
 
 template <int KP, int NP>
-inline int launch(const UpArgs& a, cudaStream_t st) {
+inline int run(const UpArgs& a, cudaStream_t st) {
     const int64_t tiles = ceil_div(a.M, (int64_t)16);
     const unsigned grid = (unsigned)std::max<int64_t>(1, std::min<int64_t>(ceil_div(tiles, (int64_t)kWarps), (int64_t)kNumSMs * (NP > 64 ? 1 : 2)));
-    upproj_kernel<KP, NP><<<grid, kThreads, 0, st>>>(a);
-    const cudaError_t e = cudaPeekAtLastError();
-    return e == cudaSuccess ? CRF_OK : (int)e;
+    return launch<false>(upproj_kernel<KP, NP>, dim3(grid), dim3(kThreads), 0, st, a);
 }
 
-inline bool dispatch(const UpArgs& a, cudaStream_t st, int* rc) {
+inline int dispatch(const UpArgs& a, cudaStream_t st) {
     const int kp = a.K <= 8 ? 8 : (a.K <= 16 ? 16 : 32);
     const int np = a.N <= 32 ? 32 : (a.N <= 64 ? 64 : 128);
-#define CRF_UP(k, n)                      \
-    if (kp == k && np == n) {             \
-        *rc = launch<k, n>(a, st);        \
-        return true;                      \
-    }
+#define CRF_UP(k, n) \
+    if (kp == k && np == n) return run<k, n>(a, st);
     CRF_UP(8, 32) CRF_UP(8, 64) CRF_UP(8, 128) CRF_UP(16, 32) CRF_UP(16, 64) CRF_UP(16, 128) CRF_UP(32, 64) CRF_UP(32, 128)
 #undef CRF_UP
-    return false;
+    return kDeclined;
 }
 
 }  // namespace up
 
 // forward: wide output, narrow plain input
-bool try_upproj_fwd(const FwdArgs& a, cudaStream_t st, int* rc) {
-    if (a.idx1 || a.C2 != 0 || a.C1 < 1 || a.C1 > 32 || a.Cout < 32 || a.Cout > 128 || (a.Cout & 3) || a.M < 8192) return false;
-    if (a.Cout <= 2 * a.C1) return false;                      // only when the output dominates the traffic
-    if ((reinterpret_cast<uintptr_t>(a.Y) & 15) || (a.bias && (reinterpret_cast<uintptr_t>(a.bias) & 15))) return false;
+int try_upproj_fwd(const FwdArgs& a, cudaStream_t st) {
+    if (a.idx1 || a.C2 != 0 || a.C1 < 1 || a.C1 > 32 || a.Cout < 32 || a.Cout > 128 || (a.Cout & 3) || a.M < 8192) return kDeclined;
+    if (a.Cout <= 2 * a.C1) return kDeclined;                  // only when the output dominates the traffic
+    if (!aligned16(a.Y) || (a.bias && !aligned16(a.bias))) return kDeclined;
     up::UpArgs u{a.X1, a.C1, a.C1, a.scale1, a.shift1, a.slope1, a.W, a.C1, 1, a.bias, a.Y, a.Cout, a.stats, a.M};
-    return up::dispatch(u, st, rc);
+    return up::dispatch(u, st);
 }
 
 // input gradient of a plain Linear with few outputs: dX[M, Ktot] = dY[M, Cout]·W[Cout, Ktot]   (the 13-class head)
-bool try_upproj_dgrad(const DgradArgs& a, cudaStream_t st, int* rc) {
+int try_upproj_dgrad(const DgradArgs& a, cudaStream_t st) {
     const int Ktot = a.C1 + a.C2;
-    if (a.bn.scale || a.C2 != 0 || !a.dX1 || a.acc1 || a.Cout < 1 || a.Cout > 32 || Ktot < 32 || Ktot > 128 || (Ktot & 3) || a.M < 8192) return false;
-    if (Ktot <= 2 * a.Cout) return false;
-    if (reinterpret_cast<uintptr_t>(a.dX1) & 15) return false;
+    if (a.bn.scale || a.C2 != 0 || !a.dX1 || a.acc1 || a.Cout < 1 || a.Cout > 32 || Ktot < 32 || Ktot > 128 || (Ktot & 3) || a.M < 8192) return kDeclined;
+    if (Ktot <= 2 * a.Cout) return kDeclined;
+    if (!aligned16(a.dX1)) return kDeclined;
     up::UpArgs u{a.dY, a.Cout, a.Cout, nullptr, nullptr, 1.f, a.W, 1, Ktot, nullptr, a.dX1, Ktot, nullptr, a.M};
-    return up::dispatch(u, st, rc);
+    return up::dispatch(u, st);
 }
 
 }  // namespace lin

@@ -8,12 +8,11 @@
 // 2-3 CTAs per SM overlap one CTA's copy with another's math (no ring needed: compute per tile is short).
 //   narrow_fwd : Y = [lrelu(X1*sc+sh) | X2]·Wᵀ (+bias), Σ/Σ² epilogue
 //   narrow_bwd : dH on the fly; dX = dH·W (split into the two segments, optional +=); dW += dHᵀ·A
-// The templates are written for Cout <= 64 if Cin <= 16, else Cout <= 16, but the dispatch (narrow_shape below) sends them only
-// Cout <= 16 AND C1 + C2 <= 16, every count a multiple of 4, no dbias; at >= 8,192 rows, and the forward only when the tcgen05
-// kernel turns the call down (gathered rows, slope1 outside [0, 1]).
+// The dispatch (narrow_shape below) sends them Cout <= 16 AND C1 + C2 <= 16, every count a multiple of 4, no dbias; at >= 8,192
+// rows, and the forward only when the tcgen05 kernel turns the call down (gathered rows, slope1 outside [0, 1]).  So the kernels
+// are instantiated for a padded Cout of 8 / 16 and, in backward, a padded Ktot of 16.
 #include <algorithm>
 #include <cstdlib>
-#include <type_traits>
 
 #include "common.cuh"
 #include "linear2.cuh"
@@ -29,7 +28,7 @@ using lin::WgradArgs;
 using lin2::cp_async16;
 using lin2::cp_async_commit;
 using lin2::cp_async_wait;
-using lin2::lrelu;
+using lin::lrelu;
 
 constexpr int TR = 128;          // rows per tile = threads per CTA
 
@@ -172,15 +171,7 @@ __global__ void __launch_bounds__(TR) bwd_kernel(const BwdArgs b, const int ntil
         const int co = e / KT, k = e % KT;
         Ws[e] = (co < C && k < Ktot) ? __ldg(a.W + (int64_t)co * Ktot + k) : 0.f;
     }
-    for (int k = tid; k < CO; k += TR) {
-        float4 pr = make_float4(1.f, 0.f, 0.f, 0.f);
-        if (!plain && k < C) {
-            const float sc = __ldg(a.bn.scale + k), sh = __ldg(a.bn.shift + k), mu = __ldg(a.bn.mean + k), is = __ldg(a.bn.invstd + k);
-            const float k1 = __ldg(a.bn.k1 + k), k2 = __ldg(a.bn.k2 + k);
-            pr = make_float4(sc, sh, -sc * is * k2, -sc * k1 + sc * is * k2 * mu);
-        }
-        s_par[k] = pr;
-    }
+    for (int k = tid; k < CO; k += TR) s_par[k] = (!plain && k < C) ? a.bn.coef(k) : make_float4(1.f, 0.f, 0.f, 0.f);
     for (int k = tid; k < KT; k += TR) {
         float2 pr = make_float2(1.f, 0.f);
         if (b.scale1 && k < a.C1) pr = make_float2(__ldg(b.scale1 + k), __ldg(b.shift1 + k));
@@ -344,49 +335,40 @@ __global__ void __launch_bounds__(TR) bwd_kernel(const BwdArgs b, const int ntil
 template <int CO, int KT, bool REF>
 size_t bwd_smem() { return (size_t)(TR * (CO + 4) * (REF ? 3 : 2) + TR * (KT + 4) + CO * KT) * 4 + (size_t)CO * 16 + (size_t)KT * 8; }
 
-inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
-
 }  // namespace narrow
 
 namespace lin {
 
-// Shapes routed to the CUDA-core kernels.  The kernels are written for Cout <= 16 (Cin <= 128) and Cin <= 16 (Cout <= 64), but
-// measured against the tensor-core kernels on B200 (profiles/README_r01.md) they only win for hidden×hidden layers
+// Shapes routed to the CUDA-core kernels.  Measured against the tensor-core kernels on B200 (profiles/README_r01.md), one thread
+// per row only wins for hidden×hidden layers
 // (16→16 forward 25 vs 28 µs, backward 29 vs 45 µs, GC/GM 27 vs 33 µs per call at 245,760 rows): with one thread per row the
 // per-element BN+LeakyReLU prologue and the per-channel butterfly statistics cost more issue slots than the FFMAs they feed.
 static inline bool narrow_shape(int Cout, int Ktot) { return Cout <= 16 && Ktot <= 16; }
 
-bool try_narrow_fwd(const FwdArgs& a, cudaStream_t st, int* rc) {
+// CTAs per SM that fit in 200 KB of shared memory (1 KB reserved per CTA), at most 8
+static inline int ctas_per_sm(size_t smem) { return (int)std::max<size_t>(1, std::min<size_t>(8, (200 * 1024) / (smem + 1024))); }
+
+int try_narrow_fwd(const FwdArgs& a, cudaStream_t st) {
     using namespace narrow;
     const int Ktot = a.C1 + a.C2;
-    if (!narrow_shape(a.Cout, Ktot) || (a.Cout & 3) || (a.C1 & 3) || (a.C2 & 3) || a.C1 == 0) return false;
-    if (!aligned16(a.X1) || (a.C2 && !aligned16(a.X2)) || !aligned16(a.Y)) return false;
+    if (!narrow_shape(a.Cout, Ktot) || (a.Cout & 3) || (a.C1 & 3) || (a.C2 & 3) || a.C1 == 0) return kDeclined;
+    if (!aligned16(a.X1) || (a.C2 && !aligned16(a.X2)) || !aligned16(a.Y)) return kDeclined;
     const int ntiles = (int)ceil_div(a.M, TR);
-    *rc = CRF_OK;
-    auto go = [&](auto cov) {
-        constexpr int CO = decltype(cov)::value;
-        const size_t smem = fwd_smem<CO>(Ktot);
-        const int per_sm = (int)std::max<size_t>(1, std::min<size_t>(8, (200 * 1024) / (smem + 1024)));
-        const int grid = std::min(ntiles, per_sm * kNumSMs);
-        cudaError_t e = cudaFuncSetAttribute(fwd_kernel<CO>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e == cudaSuccess) { fwd_kernel<CO><<<grid, TR, smem, st>>>(a, ntiles); e = cudaPeekAtLastError(); }
-        if (e != cudaSuccess) *rc = (int)e;
-        return true;
+    auto go = [&](auto kern, size_t smem) {
+        return launch<false>(kern, dim3(std::min(ntiles, ctas_per_sm(smem) * kNumSMs)), dim3(TR), smem, st, a, ntiles);
     };
-    if (a.Cout > 32) return go(std::integral_constant<int, 64>{});
-    if (a.Cout > 16) return go(std::integral_constant<int, 32>{});
-    if (a.Cout > 8) return go(std::integral_constant<int, 16>{});
-    return go(std::integral_constant<int, 8>{});
+    if (a.Cout > 8) return go(fwd_kernel<16>, fwd_smem<16>(Ktot));
+    return go(fwd_kernel<8>, fwd_smem<8>(Ktot));
 }
 
-bool try_narrow_bwd(const DgradArgs& d, const WgradArgs* w, cudaStream_t st, int* rc) {
+int try_narrow_bwd(const DgradArgs& d, const WgradArgs* w, cudaStream_t st) {
     using namespace narrow;
     const int Ktot = d.C1 + d.C2, C = d.Cout;
-    if (!narrow_shape(C, Ktot) || (C & 3) || (d.C1 & 3) || (d.C2 & 3) || d.C1 == 0) return false;
-    if (w && w->dbias) return false;
-    if (!aligned16(d.dY) || (d.bn.scale && !aligned16(d.H)) || (d.bn.act_ref && !aligned16(d.bn.act_ref))) return false;
-    if ((d.dX1 && !aligned16(d.dX1)) || (d.dX2 && !aligned16(d.dX2))) return false;
-    if (w && (!aligned16(w->X1) || (d.C2 && !aligned16(w->X2)))) return false;
+    if (!narrow_shape(C, Ktot) || (C & 3) || (d.C1 & 3) || (d.C2 & 3) || d.C1 == 0) return kDeclined;
+    if (w && w->dbias) return kDeclined;
+    if (!aligned16(d.dY) || (d.bn.scale && !aligned16(d.H)) || (d.bn.act_ref && !aligned16(d.bn.act_ref))) return kDeclined;
+    if ((d.dX1 && !aligned16(d.dX1)) || (d.dX2 && !aligned16(d.dX2))) return kDeclined;
+    if (w && (!aligned16(w->X1) || (d.C2 && !aligned16(w->X2)))) return kDeclined;
     BwdArgs b{};
     b.d = d;
     b.need_dx = (d.dX1 || d.dX2) ? 1 : 0;
@@ -396,27 +378,11 @@ bool try_narrow_bwd(const DgradArgs& d, const WgradArgs* w, cudaStream_t st, int
     }
     const bool ref = d.bn.scale && d.bn.act_ref;
     const int ntiles = (int)ceil_div(d.M, TR);
-    *rc = CRF_OK;
-    auto run = [&](auto kern, size_t smem) {
-        const int per_sm = (int)std::max<size_t>(1, std::min<size_t>(8, (200 * 1024) / (smem + 1024)));
-        const int grid = std::min(ntiles, per_sm * kNumSMs);
-        cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e == cudaSuccess) { kern<<<grid, TR, smem, st>>>(b, ntiles); e = cudaPeekAtLastError(); }
-        if (e != cudaSuccess) *rc = (int)e;
+    auto go = [&](auto kern, size_t smem) {
+        return launch<false>(kern, dim3(std::min(ntiles, ctas_per_sm(smem) * kNumSMs)), dim3(TR), smem, st, b, ntiles);
     };
-    const int CO = C <= 8 ? 8 : (C <= 16 ? 16 : (C <= 32 ? 32 : 64));
-    const int KT = Ktot <= 16 ? 16 : (Ktot <= 32 ? 32 : (Ktot <= 64 ? 64 : 128));
-#define CRF_NB(co, kt)                                                                                             \
-    if (CO == co && KT == kt) {                                                                                    \
-        if (ref) run(bwd_kernel<co, kt, true>, bwd_smem<co, kt, true>());                                          \
-        else run(bwd_kernel<co, kt, false>, bwd_smem<co, kt, false>());                                            \
-        return true;                                                                                               \
-    }
-    CRF_NB(8, 16) CRF_NB(8, 32) CRF_NB(8, 64) CRF_NB(8, 128)
-    CRF_NB(16, 16) CRF_NB(16, 32) CRF_NB(16, 64) CRF_NB(16, 128)
-    CRF_NB(32, 16) CRF_NB(64, 16)
-#undef CRF_NB
-    return false;
+    if (C > 8) return ref ? go(bwd_kernel<16, 16, true>, bwd_smem<16, 16, true>()) : go(bwd_kernel<16, 16, false>, bwd_smem<16, 16, false>());
+    return ref ? go(bwd_kernel<8, 16, true>, bwd_smem<8, 16, true>()) : go(bwd_kernel<8, 16, false>, bwd_smem<8, 16, false>());
 }
 
 }  // namespace lin

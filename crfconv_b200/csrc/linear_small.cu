@@ -20,7 +20,6 @@ namespace sm {
 constexpr int kThreads = 256;
 constexpr int BM = 32, BK = 32, AS = BK + 4;
 
-__device__ __forceinline__ float lrelu(float v, float slope) { return v > 0.0f ? v : v * slope; }
 __device__ __forceinline__ float4 ldg4(const float* p) { return __ldg(reinterpret_cast<const float4*>(p)); }
 
 // ------------------------------------------------------------------------------------------------------------------ forward
@@ -150,11 +149,7 @@ __global__ void __launch_bounds__(kThreads) dgrad_small_kernel(const DgradArgs a
     const int Ktot = a.C1 + a.C2, C = a.Cout;
     const bool plain = a.bn.scale == nullptr;
     if (!plain)
-        for (int k = tid; k < C; k += kThreads) {
-            const float sc = __ldg(a.bn.scale + k), sh = __ldg(a.bn.shift + k), mu = __ldg(a.bn.mean + k), is = __ldg(a.bn.invstd + k);
-            const float k1 = __ldg(a.bn.k1 + k), k2 = __ldg(a.bn.k2 + k);
-            s_par[k] = make_float4(sc, sh, -sc * is * k2, -sc * k1 + sc * is * k2 * mu);
-        }
+        for (int k = tid; k < C; k += kThreads) s_par[k] = a.bn.coef(k);
     const int c4 = tid & 7, r = tid >> 3;
     const int64_t m = m0 + r;
     const int nch = (C + BK - 1) / BK;
@@ -263,14 +258,8 @@ __global__ void __launch_bounds__(kThreads) wgrad_rows_kernel(const WgradArgs a)
     const int64_t mbeg = (int64_t)blockIdx.x * a.rows_per_cta, mend = min(a.M, mbeg + a.rows_per_cta);
     const bool plain = a.bn.scale == nullptr;
     if (tid < 64) {
-        float4 pr = make_float4(1.f, 0.f, 0.f, 0.f);
         const int k = co0 + tid;
-        if (!plain && k < C) {
-            const float sc = __ldg(a.bn.scale + k), sh = __ldg(a.bn.shift + k), mu = __ldg(a.bn.mean + k), is = __ldg(a.bn.invstd + k);
-            const float k1 = __ldg(a.bn.k1 + k), k2 = __ldg(a.bn.k2 + k);
-            pr = make_float4(sc, sh, -sc * is * k2, -sc * k1 + sc * is * k2 * mu);
-        }
-        s_par[tid] = pr;
+        s_par[tid] = (!plain && k < C) ? a.bn.coef(k) : make_float4(1.f, 0.f, 0.f, 0.f);
         float2 pp = make_float2(1.f, 0.f);
         const int kk = k0 + tid;
         if (a.scale1 && kk < a.C1) pp = make_float2(__ldg(a.scale1 + kk), __ldg(a.shift1 + kk));
@@ -366,63 +355,53 @@ __global__ void __launch_bounds__(kThreads) wgrad_rows_kernel(const WgradArgs a)
         }
 }
 
-inline bool al16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
 // rows at which the 128-row tiling of the generic kernels still fills the machine
 inline bool few_rows(int64_t M, int ntiles_n) { return ceil_div(M, (int64_t)128) * ntiles_n < 2 * kNumSMs; }
 
 }  // namespace sm
 
-bool try_fwd_small(const FwdArgs& a, cudaStream_t st, int* rc) {
+int try_fwd_small(const FwdArgs& a, cudaStream_t st) {
     using namespace sm;
     const int Ktot = a.C1 + a.C2;
-    if (a.Cout < 32 || (a.Cout & 3) || (a.C1 & 3) || (a.C2 & 3) || a.C1 <= 0 || Ktot < 32) return false;
-    if (!al16(a.X1) || (a.C2 && !al16(a.X2)) || !al16(a.W) || !al16(a.Y) || (a.scale1 && (!al16(a.scale1) || !al16(a.shift1)))) return false;
+    if (a.Cout < 32 || (a.Cout & 3) || (a.C1 & 3) || (a.C2 & 3) || a.C1 <= 0 || Ktot < 32) return kDeclined;
+    if (!aligned16(a.X1) || (a.C2 && !aligned16(a.X2)) || !aligned16(a.W) || !aligned16(a.Y) ||
+        (a.scale1 && (!aligned16(a.scale1) || !aligned16(a.shift1)))) return kDeclined;
     const int BN = a.Cout > 32 ? 64 : 32;
     const int tn = (int)ceil_div(a.Cout, BN);
-    if (!few_rows(a.M, tn)) return false;
-    dim3 grid((unsigned)ceil_div(a.M, (int64_t)BM), (unsigned)tn);
-    if (BN == 64) fwd_small_kernel<64><<<grid, kThreads, 0, st>>>(a);
-    else fwd_small_kernel<32><<<grid, kThreads, 0, st>>>(a);
-    const cudaError_t e = cudaPeekAtLastError();
-    *rc = e == cudaSuccess ? CRF_OK : (int)e;
-    return true;
+    if (!few_rows(a.M, tn)) return kDeclined;
+    const dim3 grid((unsigned)ceil_div(a.M, (int64_t)BM), (unsigned)tn);
+    return launch<false>(BN == 64 ? fwd_small_kernel<64> : fwd_small_kernel<32>, grid, dim3(kThreads), 0, st, a);
 }
 
-bool try_dgrad_small(const DgradArgs& a, cudaStream_t st, int* rc) {
+int try_dgrad_small(const DgradArgs& a, cudaStream_t st) {
     using namespace sm;
     const int Ktot = a.C1 + a.C2;
-    if (Ktot < 32 || (a.Cout & 3) || (a.C1 & 3) || (a.C2 & 3) || a.Cout < 32 || a.Cout > 1024) return false;
-    if (!al16(a.dY) || !al16(a.W) || (a.bn.scale && !al16(a.H)) || (a.bn.scale && a.bn.act_ref && !al16(a.bn.act_ref))) return false;
-    if ((a.dX1 && (reinterpret_cast<uintptr_t>(a.dX1) & 7)) || (a.dX2 && (reinterpret_cast<uintptr_t>(a.dX2) & 7))) return false;
+    if (Ktot < 32 || (a.Cout & 3) || (a.C1 & 3) || (a.C2 & 3) || a.Cout < 32 || a.Cout > 1024) return kDeclined;
+    if (!aligned16(a.dY) || !aligned16(a.W) || (a.bn.scale && !aligned16(a.H)) || (a.bn.scale && a.bn.act_ref && !aligned16(a.bn.act_ref))) return kDeclined;
+    if ((a.dX1 && (reinterpret_cast<uintptr_t>(a.dX1) & 7)) || (a.dX2 && (reinterpret_cast<uintptr_t>(a.dX2) & 7))) return kDeclined;
     const int BN = Ktot > 32 ? 64 : 32;
     const int tn = (int)ceil_div(Ktot, BN);
-    if (!few_rows(a.M, tn)) return false;
-    dim3 grid((unsigned)ceil_div(a.M, (int64_t)BM), (unsigned)tn);
+    if (!few_rows(a.M, tn)) return kDeclined;
+    const dim3 grid((unsigned)ceil_div(a.M, (int64_t)BM), (unsigned)tn);
     const size_t smem = a.bn.scale ? (size_t)a.Cout * sizeof(float4) : 0;
     const bool ref = a.bn.scale && a.bn.act_ref;
-    if (BN == 64) { if (ref) dgrad_small_kernel<64, true><<<grid, kThreads, smem, st>>>(a); else dgrad_small_kernel<64, false><<<grid, kThreads, smem, st>>>(a); }
-    else          { if (ref) dgrad_small_kernel<32, true><<<grid, kThreads, smem, st>>>(a); else dgrad_small_kernel<32, false><<<grid, kThreads, smem, st>>>(a); }
-    const cudaError_t e = cudaPeekAtLastError();
-    *rc = e == cudaSuccess ? CRF_OK : (int)e;
-    return true;
+    if (BN == 64) return launch<false>(ref ? dgrad_small_kernel<64, true> : dgrad_small_kernel<64, false>, grid, dim3(kThreads), smem, st, a);
+    return launch<false>(ref ? dgrad_small_kernel<32, true> : dgrad_small_kernel<32, false>, grid, dim3(kThreads), smem, st, a);
 }
 
-bool try_wgrad_rows(WgradArgs a, cudaStream_t st, int* rc) {
+int try_wgrad_rows(WgradArgs a, cudaStream_t st) {
     using namespace sm;
     const int Ktot = a.C1 + a.C2;
-    if (a.dbias || (a.Cout & 3) || (a.C1 & 3) || (a.C2 & 3) || a.C1 <= 0 || a.Cout < 32 || Ktot < 32) return false;
-    if (!al16(a.dY) || !al16(a.X1) || (a.C2 && !al16(a.X2)) || (a.bn.scale && !al16(a.H)) || (a.bn.scale && a.bn.act_ref && !al16(a.bn.act_ref))) return false;
+    if (a.dbias || (a.Cout & 3) || (a.C1 & 3) || (a.C2 & 3) || a.C1 <= 0 || a.Cout < 32 || Ktot < 32) return kDeclined;
+    if (!aligned16(a.dY) || !aligned16(a.X1) || (a.C2 && !aligned16(a.X2)) || (a.bn.scale && !aligned16(a.H)) ||
+        (a.bn.scale && a.bn.act_ref && !aligned16(a.bn.act_ref))) return kDeclined;
     const int ty = (int)ceil_div(a.Cout, 64), tz = (int)ceil_div(Ktot, 64);
-    if (!few_rows(a.M, 1)) return false;
+    if (!few_rows(a.M, 1)) return kDeclined;
     int64_t splits = std::max<int64_t>(1, std::min<int64_t>(ceil_div(a.M, (int64_t)BM), (int64_t)(3 * kNumSMs) / (ty * tz) + 1));
     a.rows_per_cta = ceil_div(ceil_div(a.M, splits), (int64_t)BM) * BM;
     splits = ceil_div(a.M, a.rows_per_cta);
-    dim3 grid((unsigned)splits, (unsigned)ty, (unsigned)tz);
-    if (a.bn.scale && a.bn.act_ref) wgrad_rows_kernel<true><<<grid, kThreads, 0, st>>>(a);
-    else wgrad_rows_kernel<false><<<grid, kThreads, 0, st>>>(a);
-    const cudaError_t e = cudaPeekAtLastError();
-    *rc = e == cudaSuccess ? CRF_OK : (int)e;
-    return true;
+    const dim3 grid((unsigned)splits, (unsigned)ty, (unsigned)tz);
+    return launch<false>(a.bn.scale && a.bn.act_ref ? wgrad_rows_kernel<true> : wgrad_rows_kernel<false>, grid, dim3(kThreads), 0, st, a);
 }
 
 }  // namespace lin

@@ -3,6 +3,9 @@
 //   * operands live in shared memory in the K-major SWIZZLE_128B canonical layout: a "slab" is [rows][32 floats], one
 //     128-byte line per row, the 16-byte chunk c of row r stored at chunk position c ^ (r & 7); 8-row groups are 1024 B
 //     apart (the descriptor's stride byte offset); slabs are 1024-byte aligned;
+//   * MN-major tf32 operands (the contraction runs along the rows, linear3w.cu / linear3b.cu) exist only in the
+//     SWIZZLE_128B_BASE32B layout: a block is [rows][32 channels], one 128-byte line per row, the 32-byte chunk c of row r
+//     stored at chunk position c ^ (r & 3); 4-row atoms are 512 B apart (descriptor SBO), 32-channel blocks LBO bytes apart;
 //   * one thread issues tcgen05.mma (kind::tf32, M = 128, N = 16..256, K = 8 per instruction); the fp32 accumulator lives in
 //     TMEM: row i of D on lane i, column j at column base + j;
 //   * completion is tracked with tcgen05.commit → mbarrier; every wait is bounded and traps instead of hanging the GPU.
@@ -93,6 +96,13 @@ __device__ __forceinline__ void tmem_dealloc(uint32_t taddr, uint32_t ncols) {
 // K-major SWIZZLE_128B shared-memory matrix descriptor (descriptor version 1 = sm_100)
 __device__ __forceinline__ uint64_t smem_desc_k128(uint32_t saddr) {
     return (uint64_t)((saddr >> 4) & 0x3FFF) | ((uint64_t)(1024 >> 4) << 32) | ((uint64_t)1 << 46) | ((uint64_t)2 << 61);
+}
+// byte offset of the 16-byte chunk c16 (0..7) of row r inside a SWIZZLE_128B_BASE32B block (32-byte chunks XOR (r & 3))
+__device__ __forceinline__ uint32_t blk_off(int r, int c16) { return (uint32_t)(r * 128 + ((((c16 >> 1) ^ (r & 3)) << 5) | ((c16 & 1) << 4))); }
+// MN-major SWIZZLE_128B_BASE32B descriptor: LBO = stride between 32-channel blocks, SBO = 512 B between 4-row atoms
+__device__ __forceinline__ uint64_t desc_mn(uint32_t saddr, uint32_t lbo_bytes) {
+    return (uint64_t)((saddr >> 4) & 0x3FFF) | ((uint64_t)((lbo_bytes >> 4) & 0x3FFF) << 16) | ((uint64_t)(512 >> 4) << 32) | ((uint64_t)1 << 46) |
+           ((uint64_t)1 << 61);
 }
 // instruction descriptor: D f32, A and B tf32, both K-major
 __host__ __device__ constexpr uint32_t idesc_tf32(int M, int N) {

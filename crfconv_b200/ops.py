@@ -9,7 +9,8 @@ import torch
 
 from . import _lib
 
-# 0 = 3xTF32 (fp32-grade, default: matches the fp32 reference to ~1e-6), 1 = single-pass TF32
+# 0 = 3xTF32 (fp32-grade, default: matches the fp32 reference to ~1e-6), 1 = single-pass TF32, 2 = single-pass bf16 in the
+# persistent kernels (single-pass TF32 elsewhere; DESIGN.md §5).  The Linear entry points refuse any other value.
 PRECISION = int(os.environ.get("CRFCONV_PRECISION", "0"))
 STAT_SLOTS = 64      # include/crfconv_b200.h: CRFCONV_STAT_SLOTS
 GRAD_SLOTS = 32      # CRFCONV_GRAD_SLOTS

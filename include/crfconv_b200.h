@@ -88,7 +88,8 @@ int crfconv_grid_subsample_host(const float* points, int64_t N, const float* fea
 /* ------------------------------------------------------------- Linear + BatchNorm + LeakyReLU chains (MLP)
  * Replaces models/common.py:26-40 (MLP = nn.Linear(bias = not bn) → FastBatchNorm1d → activation) as it is used by
  * models/continuous_crf_conv_big.py:20-29 and models/point_conv_big.py:20-23,65-70.  All pointers are device
- * pointers, tensors are row-major [rows, channels] f32.  precision: 0 = 3xTF32 (fp32-grade), 1 = one TF32 pass.  */
+ * pointers, tensors are row-major [rows, channels] f32.  precision: 0 = 3xTF32 (fp32-grade), 1 = one TF32 pass, 2 = one bf16
+ * pass in the persistent kernels (one TF32 pass elsewhere); any other value is refused with CRF_ERR_INVALID_ARG.  */
 
 /* Kernel selection knob for tests / experiments: -1 = default rule (persistent bf16x3 kernels for large row counts,
  * generic 3xTF32 kernels otherwise), 0 = generic only, 1 = fast whenever the shape allows.  Returns the previous mode. */

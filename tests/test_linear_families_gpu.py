@@ -19,7 +19,7 @@ Run with `-s` to see the worst error per kernel family."""
 import math
 import re
 import zlib
-from dataclasses import dataclass
+from dataclasses import dataclass, replace
 from typing import Optional
 
 import pytest
@@ -589,3 +589,26 @@ def test_single_pass_bf16_within_stated_bound(ops, c):
         _, _, pairs = run_bwd(ops, c)
         worst = {n: rel_l2(a, b) for n, (a, b) in pairs.items()}
         assert all(v < BF16_GRAD_L2 for v in worst.values()), f"{c.name}: {worst}"
+
+
+def test_precision_3_is_refused(ops):
+    """precision is 0 (3xTF32), 1 (single-pass TF32) or 2 (single-pass bf16): crfconv_linear_fwd, crfconv_linear_bwd and
+    crfconv_linear_fwd_bn refuse any other value with CRF_ERR_INVALID_ARG instead of running some mix of the kernels."""
+    def refused():
+        return pytest.raises(RuntimeError, match=r"\(status -1\)$")
+    with refused():
+        run_fwd(ops, replace(FWD_CASES[0], prec=3))
+    with refused():
+        run_bwd(ops, replace(BWD_CASES[0], prec=3))
+    c = FWDBN_CASES[0]
+    x = Inputs(c)
+    st = ops.BN(c.Cout, x.X1.device, stats=torch.zeros(ops.STAT_SLOTS, 2 * c.Cout, device="cuda"))
+    counter = torch.zeros(ops.counter_ints(), dtype=torch.int32, device="cuda")
+    prev = ops.PRECISION
+    ops.PRECISION = 3
+    try:
+        with refused():
+            ops.linear_fwd_bn(x.X1, x.W, st, torch.nn.BatchNorm1d(c.Cout).cuda(), counter, scale1=x.sc1, shift1=x.sh1, X2=x.X2,
+                              out=torch.empty(c.M, c.Cout, device="cuda"))
+    finally:
+        ops.PRECISION = prev
