@@ -56,8 +56,7 @@ SIGNATURES = {
     "crfconv_fused_part_floats": (_int, []),
     "crfconv_fused_counter_ints": (_int, []),
     "crfconv_out_bwd_part_floats": (_int, []),
-    "crfconv_fused_tune": (_int, [_int, _int]),
-    "crfconv_lin16_fwd": (_int, [_vp, _int, _vp, _vp, _vp, _f32, _vp, _vp, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _f32, _f32, _vp, _vp, _vp, _vp, _vp]),
+    "crfconv_lin16_fwd": (_int, [_vp, _int, _vp, _vp, _vp, _f32, _vp, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _f32, _f32, _vp, _vp, _vp, _vp, _vp]),
     "crfconv_up16_fwd": (_int, [_vp, _vp, _int, _vp, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _f32, _f32, _vp, _vp, _vp, _vp, _vp]),
     "crfconv_linear_fwd_bn": (_int, [_vp, _int, _vp, _vp, _f32, _vp, _int, _vp, _vp, _vp, _i64, _int, _int, _vp, _vp, _vp, _vp, _vp, _f32, _f32,
                                      _vp, _vp, _vp, _vp, _vp]),
@@ -66,7 +65,7 @@ SIGNATURES = {
     "crfconv_in16_dgrad": (_int, [_vp] * 8 + [_int, _vp, _int, _i64, _vp]),
     "crfconv_in16_wgrad": (_int, [_vp] * 8 + [_int, _vp, _i64, _i64, _vp]),
     "crfconv_out16_bwd": (_int, [_vp] * 6 + [_f32, _vp, _vp, _vp, _i64] + [_vp] * 10),
-    "crfconv_crf_step_bwd_fused": (_int, [_vp] * 12 + [_int, _vp, _vp, _vp, _vp, _i64, _vp, _i64, _i64, _int, _int, _int, _int] + [_vp] * 7),
+    "crfconv_crf_step_bwd_fused": (_int, [_vp] * 12 + [_int, _vp, _vp, _vp, _vp, _i64, _vp, _i64, _i64, _int, _int, _int] + [_vp] * 7),
     "crfconv_crf_upsample_bwd_fused": (_int, [_vp] * 7 + [_i64, _i64, _i64] + [_vp] * 7),
     "crfconv_crf_compat_fwd": (_int, [_vp, _vp, _vp, _vp, _int, _vp]),
     "crfconv_crf_compat_bwd": (_int, [_vp, _vp, _vp, _vp, _vp, _vp, _int, _vp]),
@@ -83,8 +82,6 @@ SIGNATURES = {
     "crfconv_pcf_param_grads": (_int, [_vp] * 18 + [_int, _vp]),
     "crfconv_cross_entropy_fwd": (_int, [_vp, _vp, _vp, _i64, _int, _i64, _vp, _vp]),
     "crfconv_cross_entropy_bwd": (_int, [_vp, _vp, _vp, _i64, _int, _i64, _vp, _vp, _int, _vp, _vp]),
-    "crfconv_crf_upsample_fwd_packed": (_int, [_vp, _vp, _vp, _vp, _vp, _i64, _i64, _i64, _vp]),
-    "crfconv_crf_step_fwd_packed": (_int, [_vp, _vp, _vp, _vp, _vp, _vp, _i64, _i64, _vp]),
     "crfconv_crf_upsample_bwd": (_int, [_vp, _vp, _vp, _vp, _i64, _i64, _i64, _int, _vp]),
     "crfconv_crf_step_fwd": (_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _i64, _int, _int, _vp]),
     "crfconv_pack_index_host": (_int, [_vp, _i64, _int, _vp, _int]),

@@ -238,7 +238,6 @@ class _CRFConvFunction(torch.autograd.Function):
                 None, None, *_param_grads(ctx.gbuf, [Gc, *grads]))
 
 
-PACKED = False         # measured experiment, off (module attribute, no environment switch; steps = 1): mean-field operands {Hy | z} interleaved into 128-byte rows (crf.cu); measured: no gain
 _THIRD = {}
 
 
@@ -317,19 +316,13 @@ class _CRFConvFusedFunction(torch.autograd.Function):
             ops.lin16_fwd(H1u, W2u, s2u, bns[1], parts[1], cnt[1], pre=s1u, pslope=sl[0], out=H2u)
             join.record(side)
         ops.lin16_fwd(P, W1p, s1p, bns[2], parts[2], cnt[2], out=H1p)          # pairwise_nn (:59)
-        packed = PACKED and steps == 1
-        YX = torch.empty((M, 2 * F), dtype=torch.float32, device=dev) if packed else None
-        ops.lin16_fwd(H1p, W2p, s2p, bns[3], parts[3], cnt[3], pre=s1p, pslope=sl[2], out=H2p, packed_out=YX)
+        ops.lin16_fwd(H1p, W2p, s2p, bns[3], parts[3], cnt[3], pre=s1p, pslope=sl[2], out=H2p)
         main.wait_event(join)
         main.wait_event(join_aux)
-        if packed:                                                                # one 128-byte row {Hy | z} per gathered neighbour
-            ops.crf_upsample_fwd_packed(H2u, s2u, up, YX, B, N, Nc)               # (:60)
-            xs = [None, ops.crf_step_fwd_packed(YX, s2p.scale, nbr, Cm, Minv, B, N)]   # (:68-72)
-        else:
-            z = ops.crf_upsample_fwd(H2u, s2u, up, B, N, Nc)                      # (:60)
-            xs = [z]
-            for _ in range(steps):                                                # (:68-72)
-                xs.append(ops.crf_step_fwd(H2p, s2p.scale, z, xs[-1], nbr, Cm, Minv, B, N, K))
+        z = ops.crf_upsample_fwd(H2u, s2u, up, B, N, Nc)                          # (:60)
+        xs = [z]
+        for _ in range(steps):                                                    # (:68-72)
+            xs.append(ops.crf_step_fwd(H2p, s2p.scale, z, xs[-1], nbr, Cm, Minv, B, N, K))
         H3 = ops.up16_fwd(xs[-1], Wo, so, bns[4], cnt[4])                       # out_nn (:74)
         Hf = ops.linear_fwd_bn(H3, Wf, sf, bns[5], cnt[5], scale1=so.scale, shift1=so.shift, slope1=sl[4], X2=P)   # fusion_nn (:76)
         out = ops.bn_act_fwd(Hf, sf, sl[5])
@@ -344,14 +337,13 @@ class _CRFConvFusedFunction(torch.autograd.Function):
         ctx.bn = (s1u, s2u, s1p, s2p, so, sf)
         ctx.sl = sl
         ctx.gamma_y = bns[3].weight.detach() if bns[3].weight is not None else torch.ones(F, dtype=torch.float32, device=dev)
-        ctx.save_for_backward(U, P, up, nbr, H1u, H2u, H1p, H2p, H3, Hf, Cm, Minv, cc, W1u, W2u, W1p, W2p, Wo, Wf, YX, *xs)
+        ctx.save_for_backward(U, P, up, nbr, H1u, H2u, H1p, H2p, H3, Hf, Cm, Minv, cc, W1u, W2u, W1p, W2p, Wo, Wf, *xs)
         return out.view(B, N, Co)
 
     @staticmethod
     def backward(ctx, gout):
-        (U, P, up, nbr, H1u, H2u, H1p, H2p, H3, Hf, Cm, Minv, cc, W1u, W2u, W1p, W2p, Wo, Wf, YX, *xs) = ctx.saved_tensors
+        (U, P, up, nbr, H1u, H2u, H1p, H2p, H3, Hf, Cm, Minv, cc, W1u, W2u, W1p, W2p, Wo, Wf, *xs) = ctx.saved_tensors
         B, N, Nc, K, F, Co, Cu, Cp, steps = ctx.dims
-        packed = YX is not None
         s1u, s2u, s1p, s2p, so, sf = ctx.bn
         sl = ctx.sl
         dev = gout.device
@@ -410,9 +402,9 @@ class _CRFConvFusedFunction(torch.autograd.Function):
         for t in range(steps, 0, -1):
             gprev = big.take(M, F)
             first = t == steps
-            ops.crf_step_bwd_fused(YX if packed else H2p, s2p, z, xs[t - 1], nbr, Cm, Minv, g, xs[-1] if first else None, Q if first else None,
+            ops.crf_step_bwd_fused(H2p, s2p, z, xs[t - 1], nbr, Cm, Minv, g, xs[-1] if first else None, Q if first else None,
                                    a0 if first else None, Gz, not first, gprev, Gy, scr(GC), scr(GM), n_small, ysum, B, N, K,
-                                   t == 1, cnt[2], ctx.gamma_y, dg["2p"], db["2p"], packed=packed)
+                                   t == 1, cnt[2], ctx.gamma_y, dg["2p"], db["2p"])
             g = gprev
         Gc = take_small(F, F)
         aux = _aux_stream(dev)

@@ -51,54 +51,7 @@ struct Carver {
     }
 };
 
-
-// ---- programmatic dependent launch (PDL) ------------------------------------------------------------------------------
-// A CRF layer step is ≈25 dependent kernels of 6-170 us; between two of them the GPU drains, launches, and runs the next kernel's
-// prologue (weight staging, TMEM allocation) before the first useful byte moves.  With PDL every kernel of the chain
-//   * calls pdl_trigger() first: the NEXT kernel in the stream may be scheduled as soon as all CTAs of this one have started and
-//     SM resources free up, so its launch latency and prologue overlap this kernel's tail (slow CTAs, last-CTA finalize);
-//   * calls pdl_wait() before it touches ANY global memory written by an earlier kernel of the stream (and before any global write):
-//     it returns once the preceding kernel has completed and its writes are visible.  Everything before the wait may only read
-//     parameters (weights) and write shared memory.
-// Every kernel launched through launch_k() executes pdl_wait(), which makes completion transitive along the chain.  Both
-// instructions are no-ops when the kernel was launched without the attribute.
-// MEASURED AND REJECTED (round 2, profiles/README_r02.md): with the attribute on, the S1 step went from 0.775 to 0.812 ms — the CTAs
-// of the next kernel sit on the SMs spinning in griddepcontrol.wait and crowd out the kernels of the parallel graph branches (unary
-// chain, compatibility algebra).  Kept as an experiment knob only: crfconv_fused_tune(1, 1); off by default.
-inline int& pdl_flag() { static int v = 0; return v; }
-__device__ __forceinline__ void pdl_trigger() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
-__device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-
-template <typename... KArgs, typename... Args>
-inline cudaError_t launch_k(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args&&... args) {
-    cudaLaunchConfig_t cfg{};
-    cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = smem; cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = pdl_flag() ? 1 : 0;
-    return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
-}
-
 __device__ __forceinline__ int lane_id() { return threadIdx.x & 31; }
-
-// ---- 256-bit global loads (sm_100: LDG.E.256) ---------------------------------------------------------------------------
-// The L1 data pipe is charged per 128-byte line an instruction touches (≈2 cycles per line inside one instruction).  A gather of
-// 64-byte rows with 128-bit loads touches 8 lines per warp instruction and uses half of each; with the two 64-byte rows an edge
-// needs (y_j, x_j) interleaved into ONE 128-byte row ("packed" layout, crf.cu) and 256-bit loads, 4 lanes fetch a whole line
-// and the line count per edge halves.
-__device__ __forceinline__ void ldg8(const float* p, float4& a, float4& b) {
-    asm("ld.global.nc.v8.f32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];"
-        : "=f"(a.x), "=f"(a.y), "=f"(a.z), "=f"(a.w), "=f"(b.x), "=f"(b.y), "=f"(b.z), "=f"(b.w)
-        : "l"(p));
-}
-// 4 consecutive int64 (one quarter of a K = 16 neighbour row) as ints
-__device__ __forceinline__ void ldg_idx4(const long long* p, int (&r)[4]) {
-    long long a, b, c, d;
-    asm("ld.global.nc.v4.b64 {%0, %1, %2, %3}, [%4];" : "=l"(a), "=l"(b), "=l"(c), "=l"(d) : "l"(p));
-    r[0] = (int)a; r[1] = (int)b; r[2] = (int)c; r[3] = (int)d;
-}
 
 __device__ __forceinline__ float warp_sum(float v) {
 #pragma unroll

@@ -88,8 +88,6 @@ __device__ __forceinline__ float dot4(float4 a, float4 b) { return a.x * b.x + a
 __global__ void __launch_bounds__(256) upsample_affine_kernel(const float* __restrict__ Hu, const float* __restrict__ scale,
                                                               const float* __restrict__ shift, const int64_t* __restrict__ up,
                                                               float* __restrict__ z, int64_t total, int64_t N, int64_t Nc, int F4) {
-    pdl_trigger();
-    pdl_wait();
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= total * F4) return;
     const int64_t m = i / F4;
@@ -143,8 +141,6 @@ __global__ void __launch_bounds__(256, F == 16 ? 5 : 1) step_fwd_kernel(const St
     __shared__ __align__(16) float Cs[TC ? 4 : F * F];
     __shared__ __align__(16) float Ms[TC ? 4 : F * F];
     __shared__ __align__(16) float4 fC[TC ? 128 : 1], fM[TC ? 128 : 1];
-    pdl_trigger();
-    pdl_wait();
     if constexpr (TC) {
         cl::stage_mat16(fC, [&](int k, int n) { return a.Cm[k * 16 + n]; }, threadIdx.x, blockDim.x);
         cl::stage_mat16(fM, [&](int k, int n) { return a.Minv[k * 16 + n]; }, threadIdx.x, blockDim.x);
@@ -209,73 +205,6 @@ __global__ void __launch_bounds__(256, F == 16 ? 5 : 1) step_fwd_kernel(const St
         gather_full<F>(v, full, lane);
         x = rowvec_mat<F>(full, Ms, c0);
     }
-    if (valid) *reinterpret_cast<float4*>(a.xout + p * F + c0) = x;
-}
-
-// ---- packed layout (F = 16, K = 16, first mean-field step: x^0 = z) ---------------------------------------------------------
-// YX[m][32]: lane slice s (channels 4s..4s+3) of point m owns floats [8s, 8s+8) = { Hy[m][4s..4s+3], z[m][4s..4s+3] }: the two rows an
-// edge gathers are ONE 128-byte line fetched by the point's 4 lanes with one 256-bit load each (see ldg8, common.cuh).
-__global__ void __launch_bounds__(256) upsample_affine_packed_kernel(const float* __restrict__ Hu, const float* __restrict__ scale,
-                                                                     const float* __restrict__ shift, const int64_t* __restrict__ up,
-                                                                     float* __restrict__ YX, int64_t total, int64_t N, int64_t Nc) {
-    pdl_trigger();
-    pdl_wait();
-    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= total * 4) return;
-    const int64_t m = i >> 2;
-    const int s = (int)(i & 3), c = 4 * s;
-    const int64_t src = (m / N) * Nc + __ldg(up + m);
-    const float4 h = ld4(Hu + src * 16 + c), sc = ld4(scale + c), sh = ld4(shift + c);
-    *reinterpret_cast<float4*>(YX + m * 32 + 8 * s + 4) =
-        make_float4(fmaf(h.x, sc.x, sh.x), fmaf(h.y, sc.y, sh.y), fmaf(h.z, sc.z, sh.z), fmaf(h.w, sc.w, sh.w));
-}
-
-struct StepPackedArgs {
-    const float* YX; const float* scale_y; const int64_t* nbr; const float* Cm; const float* Minv;
-    float* xout; int64_t total, N;
-};
-
-__global__ void __launch_bounds__(256) step_fwd_packed_kernel(const StepPackedArgs a) {
-    constexpr int F = 16;
-    __shared__ __align__(16) float4 fC[128], fM[128];
-    pdl_trigger();
-    pdl_wait();
-    cl::stage_mat16(fC, [&](int k, int n) { return a.Cm[k * 16 + n]; }, threadIdx.x, blockDim.x);
-    cl::stage_mat16(fM, [&](int k, int n) { return a.Minv[k * 16 + n]; }, threadIdx.x, blockDim.x);
-    __syncthreads();
-    const int lane = lane_id(), sub = lane & 3, c0 = 4 * sub, gb = lane & ~3;
-    const int64_t warp = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-    int64_t p = warp * 8 + (lane >> 2);
-    const bool valid = p < a.total;
-    if (!valid) p = a.total - 1;
-    const int64_t base = (p / a.N) * a.N;
-    int r[4];                                              // lane s of the point holds indices 4s..4s+3
-    ldg_idx4(reinterpret_cast<const long long*>(a.nbr + p * 16) + 4 * sub, r);
-    const float4 sc = ld4(a.scale_y + c0);
-    float4 hyi, zi;
-    ldg8(a.YX + p * 32 + 8 * sub, hyi, zi);
-    const float4 yi = mul4(hyi, sc);
-    float mx = -INFINITY, l = 0.f;
-    float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
-#pragma unroll
-    for (int k = 1; k < 16; ++k) {                         // online softmax: the compiler keeps a handful of gathers in flight (56 registers)
-        const int64_t row = base + __shfl_sync(0xffffffffu, r[k & 3], gb + (k >> 2));
-        float4 hj, xj;
-        ldg8(a.YX + row * 32 + 8 * sub, hj, xj);
-        const float4 df = sub4(yi, mul4(hj, sc));
-        const float al = -group_sum<4>(dot4(df, df));
-        const float nm = fmaxf(mx, al);
-        const float corr = __expf(mx - nm), pj = __expf(al - nm);
-        l = l * corr + pj;
-        acc.x = acc.x * corr + pj * xj.x; acc.y = acc.y * corr + pj * xj.y;
-        acc.z = acc.z * corr + pj * xj.z; acc.w = acc.w * corr + pj * xj.w;
-        mx = nm;
-    }
-    const float inv_l = 1.0f / l;
-    const float4 msg = make_float4(acc.x * inv_l, acc.y * inv_l, acc.z * inv_l, acc.w * inv_l);
-    float4 v = cl::rows8_mat16(msg, fC, lane);
-    v.x += zi.x; v.y += zi.y; v.z += zi.z; v.w += zi.w;
-    const float4 x = cl::rows8_mat16(v, fM, lane);
     if (valid) *reinterpret_cast<float4*>(a.xout + p * F + c0) = x;
 }
 
@@ -472,8 +401,6 @@ __global__ void __launch_bounds__(128) step_bwd_reg_kernel(const StepArgs a) {
 // Cm = cᵀc ; Minv = (I + Cm)^{-1} by Gauss-Jordan (I + cᵀc is SPD with eigenvalues >= 1: no pivoting needed).
 __global__ void __launch_bounds__(256) compat_fwd_kernel(const float* __restrict__ c, float* __restrict__ Cm, float* __restrict__ Minv,
                                                          double* scratch, int F) {
-    pdl_trigger();
-    pdl_wait();
     __shared__ double colp[128];
     __shared__ double piv;
     double* aug = scratch;   // [F][2F]
@@ -507,8 +434,6 @@ __global__ void __launch_bounds__(256) compat_fwd_kernel(const float* __restrict
 __global__ void __launch_bounds__(256) compat_bwd_kernel(const float* __restrict__ c, const float* __restrict__ Minv,
                                                          const float* __restrict__ GC, const float* __restrict__ GM, float* Gc,
                                                          double* scratch, int F) {
-    pdl_trigger();
-    pdl_wait();
     double* T = scratch;            // T = Minvᵀ·GM
     double* G = scratch + F * F;    // G = GC − T·Minvᵀ
     const int tid = threadIdx.x, nt = blockDim.x;
@@ -540,8 +465,6 @@ __global__ void __launch_bounds__(256) compat_bwd_kernel(const float* __restrict
 __global__ void __launch_bounds__(1024) compat_fwd_smem_kernel(const float* __restrict__ c, float* __restrict__ Cm, float* __restrict__ Minv,
                                                                int F) {
     extern __shared__ __align__(16) double sm_d[];              // aug [F][2F] | colp [F] | c as doubles [F][F]
-    pdl_trigger();
-    pdl_wait();
     double* aug = sm_d;
     double* colp = aug + F * 2 * F;
     double* cs = colp + F;
@@ -577,8 +500,6 @@ __global__ void __launch_bounds__(1024) compat_fwd_smem_kernel(const float* __re
 __global__ void __launch_bounds__(1024) compat_bwd_smem_kernel(const float* __restrict__ c, const float* __restrict__ Minv,
                                                                const float* __restrict__ GC, const float* __restrict__ GM, float* Gc, int F) {
     extern __shared__ __align__(16) double sm_d[];              // T [F][F+1] | G [F][F+1] | then floats: Minv [F][F+1], GM / c [F][F+1]
-    pdl_trigger();
-    pdl_wait();
     const int L = F + 1;                                        // odd pitch: column walks (stride L) are bank-conflict free
     double* T = sm_d;
     double* G = T + F * L;
@@ -635,11 +556,11 @@ int crfconv_crf_compat_fwd(const float* c, float* Cm, float* Minv, double* scrat
         const size_t smem = ((size_t)F * 2 * F + F + (size_t)F * F) * sizeof(double);
         static bool attr = false;
         if (!attr) { CRF_CUDA(cudaFuncSetAttribute(mf::compat_fwd_smem_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 112 * 1024)); attr = true; }
-        CRF_CUDA(launch_k(mf::compat_fwd_smem_kernel, dim3(1), dim3(F >= 32 ? 1024 : 256), smem, (cudaStream_t)stream, c, Cm, Minv, F));
+        mf::compat_fwd_smem_kernel<<<1, F >= 32 ? 1024 : 256, smem, (cudaStream_t)stream>>>(c, Cm, Minv, F);
         CRF_LAUNCH_CHECK();
         return CRF_OK;
     }
-    CRF_CUDA(launch_k(mf::compat_fwd_kernel, dim3(1), dim3(256), 0, (cudaStream_t)stream, c, Cm, Minv, scratch, F));
+    mf::compat_fwd_kernel<<<1, 256, 0, (cudaStream_t)stream>>>(c, Cm, Minv, scratch, F);
     CRF_LAUNCH_CHECK();
     return CRF_OK;
 }
@@ -651,11 +572,11 @@ int crfconv_crf_compat_bwd(const float* c, const float* Minv, const float* GC, c
         const size_t smem = (size_t)2 * F * (F + 1) * sizeof(double) + (size_t)2 * F * (F + 1) * sizeof(float);
         static bool attr = false;
         if (!attr) { CRF_CUDA(cudaFuncSetAttribute(mf::compat_bwd_smem_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 112 * 1024)); attr = true; }
-        CRF_CUDA(launch_k(mf::compat_bwd_smem_kernel, dim3(1), dim3(F >= 32 ? 1024 : 256), smem, (cudaStream_t)stream, c, Minv, GC, GM, Gc, F));
+        mf::compat_bwd_smem_kernel<<<1, F >= 32 ? 1024 : 256, smem, (cudaStream_t)stream>>>(c, Minv, GC, GM, Gc, F);
         CRF_LAUNCH_CHECK();
         return CRF_OK;
     }
-    CRF_CUDA(launch_k(mf::compat_bwd_kernel, dim3(1), dim3(256), 0, (cudaStream_t)stream, c, Minv, GC, GM, Gc, scratch, F));
+    mf::compat_bwd_kernel<<<1, 256, 0, (cudaStream_t)stream>>>(c, Minv, GC, GM, Gc, scratch, F);
     CRF_LAUNCH_CHECK();
     return CRF_OK;
 }
@@ -666,8 +587,8 @@ int crfconv_crf_upsample_fwd(const float* Hu, const float* scale, const float* s
     if (B < 0 || N < 0 || Nc <= 0 || F <= 0 || (F & 3)) return CRF_ERR_INVALID_ARG;
     const int64_t total = B * N;
     if (total == 0) return CRF_OK;
-    CRF_CUDA(launch_k(mf::upsample_affine_kernel, dim3((unsigned)ceil_div(total * (F / 4), 256)), dim3(256), 0, (cudaStream_t)stream, Hu, scale, shift,
-                      up_idx, z, total, N, Nc, F / 4));
+    mf::upsample_affine_kernel<<<(unsigned)ceil_div(total * (F / 4), 256), 256, 0, (cudaStream_t)stream>>>(Hu, scale, shift, up_idx, z, total,
+                                                                                                    N, Nc, F / 4);
     CRF_LAUNCH_CHECK();
     return CRF_OK;
 }
@@ -696,31 +617,10 @@ int crfconv_crf_step_fwd(const float* Hy, const float* scale_y, const float* z, 
         constexpr int FF = decltype(f)::value;
         constexpr int PPW = 32 / (FF / 4);
         const int64_t warps = ceil_div(a.total, PPW);
-        CRF_CUDA(launch_k(mf::step_fwd_kernel<FF>, dim3((unsigned)ceil_div(warps, 8)), dim3(256), 0, (cudaStream_t)stream, a));
+        mf::step_fwd_kernel<FF><<<(unsigned)ceil_div(warps, 8), 256, 0, (cudaStream_t)stream>>>(a);
         CRF_LAUNCH_CHECK();
         return CRF_OK;
     });
-}
-
-// Packed variants (F = 16, K = 16, step 1 only): YX[B*N, 32] holds Hy (written by crfconv_lin16_fwd's Ypk output) and z interleaved.
-int crfconv_crf_upsample_fwd_packed(const float* Hu, const float* scale, const float* shift, const int64_t* up_idx, float* YX, int64_t B,
-                                    int64_t N, int64_t Nc, void* stream) {
-    if (B <= 0 || N <= 0 || Nc <= 0 || !Hu || !scale || !shift || !up_idx || !YX) return CRF_ERR_INVALID_ARG;
-    const int64_t total = B * N;
-    CRF_CUDA(launch_k(mf::upsample_affine_packed_kernel, dim3((unsigned)ceil_div(total * 4, 256)), dim3(256), 0, (cudaStream_t)stream, Hu, scale,
-                      shift, up_idx, YX, total, N, Nc));
-    CRF_LAUNCH_CHECK();
-    return CRF_OK;
-}
-
-int crfconv_crf_step_fwd_packed(const float* YX, const float* scale_y, const int64_t* neighbor_idx, const float* Cm, const float* Minv,
-                                float* xout, int64_t B, int64_t N, void* stream) {
-    if (B <= 0 || N <= 0 || !YX || !scale_y || !neighbor_idx || !Cm || !Minv || !xout) return CRF_ERR_INVALID_ARG;
-    if ((reinterpret_cast<uintptr_t>(YX) & 31) || (reinterpret_cast<uintptr_t>(neighbor_idx) & 31)) return CRF_ERR_INVALID_ARG;
-    mf::StepPackedArgs a{YX, scale_y, neighbor_idx, Cm, Minv, xout, B * N, N};
-    CRF_CUDA(launch_k(mf::step_fwd_packed_kernel, dim3((unsigned)ceil_div(ceil_div(a.total, 8), 8)), dim3(256), 0, (cudaStream_t)stream, a));
-    CRF_LAUNCH_CHECK();
-    return CRF_OK;
 }
 
 // Backward of one step.  g = dL/dx^t.  Gz = h, or += h when gz_acc (owner rows), gprev += Σ s_ij q_i (must be zero-initialised),

@@ -78,7 +78,7 @@ using namespace crf;
 
 extern "C" {
 
-int crfconv_abi_version(void) { return 1; }
+int crfconv_abi_version(void) { return 2; }
 
 const char* crfconv_status_string(int status) {
     switch (status) {

@@ -233,8 +233,6 @@ __global__ void __launch_bounds__(128) bn_finalize_fwd_kernel(const float* __res
 __global__ void __launch_bounds__(256) bn_act_fwd_kernel(const float* __restrict__ H, const float* __restrict__ scale,
                                                          const float* __restrict__ shift, const float* __restrict__ R,
                                                          float slope, float* __restrict__ Y, int64_t total4, int C4) {
-    pdl_trigger();
-    pdl_wait();
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total4; i += (int64_t)gridDim.x * blockDim.x) {
         const int c = (int)(i % C4) * 4;
         const float4 h = __ldg(reinterpret_cast<const float4*>(H) + i);
@@ -264,8 +262,6 @@ template <bool REF>
 __global__ void __launch_bounds__(256, REF ? 3 : 4) bn_bwd_reduce_kernel(const float* __restrict__ dY, const float* __restrict__ H, BnBwd bn,
                                                             float* __restrict__ sums, int64_t M, int C, const cl::BwdFin fin) {
     __shared__ float red[256 * 8];
-    pdl_trigger();
-    pdl_wait();
     const int C4 = C >> 2;
     const int tpr = C4;                           // threads per row
     const int rows_per_it = 256 / tpr;            // C4 divides 256 for C in {8,...,1024}
@@ -354,8 +350,6 @@ __global__ void __launch_bounds__(128) bn_finalize_bwd_kernel(const float* __res
 
 // dW[i] += Σ_slots scratch[slot][i]   (fixed order ⇒ deterministic for a given launch configuration)
 __global__ void __launch_bounds__(256) grad_slots_reduce_kernel(const float* __restrict__ scratch, float* dW, int n, int64_t stride) {
-    pdl_trigger();
-    pdl_wait();
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
     float s = 0.f;
@@ -574,7 +568,7 @@ inline int try_wgrad_tiny(const WgradArgs& a, cudaStream_t st) {
     if (a.bn.scale && a.bn.act_ref && !aligned16(a.bn.act_ref)) return kDeclined;
     const int rows_per_it = 256 / (a.Cout >> 2);
     const unsigned grid = (unsigned)std::min<int64_t>(ceil_div(a.M, (int64_t)rows_per_it * 4), (int64_t)kNumSMs * 8);
-    return launch<false>(wgrad_tiny_kernel<4>, dim3(grid), dim3(256), 0, st, a);
+    return launch(wgrad_tiny_kernel<4>, dim3(grid), dim3(256), 0, st, a);
 }
 
 // dW[co, k] += Σ_m dH[m, co] · A[m, k],  A = [prologue(X1) | X2].  Output tile 64 (co) × 64 (k) per CTA; CTAs along
@@ -702,7 +696,7 @@ inline int fwd_generic(const FwdArgs& a, bool x3, cudaStream_t st) {
     return dispatch_bn(a.Cout, [&](auto bn) {
         constexpr int BN = decltype(bn)::value;
         const dim3 grid((unsigned)ceil_div(a.M, BM), (unsigned)ceil_div(a.Cout, BN));
-        return launch<false>(x3 ? fwd_kernel<BN, true> : fwd_kernel<BN, false>, grid, dim3(kThreads), 0, st, a);
+        return launch(x3 ? fwd_kernel<BN, true> : fwd_kernel<BN, false>, grid, dim3(kThreads), 0, st, a);
     });
 }
 
@@ -711,7 +705,7 @@ inline int dgrad_generic(const DgradArgs& a, bool x3, cudaStream_t st) {
     return dispatch_bn(Ktot, [&](auto bn) {
         constexpr int BN = decltype(bn)::value;
         const dim3 grid((unsigned)ceil_div(a.M, BM), (unsigned)ceil_div(Ktot, BN));
-        return launch<false>(x3 ? dgrad_kernel<BN, true> : dgrad_kernel<BN, false>, grid, dim3(kThreads), 0, st, a);
+        return launch(x3 ? dgrad_kernel<BN, true> : dgrad_kernel<BN, false>, grid, dim3(kThreads), 0, st, a);
     });
 }
 
@@ -721,7 +715,7 @@ inline int wgrad_generic(WgradArgs a, bool x3, cudaStream_t st) {
     a.rows_per_cta = ceil_div(ceil_div(a.M, splits), WR) * WR;
     splits = ceil_div(a.M, a.rows_per_cta);
     const dim3 grid((unsigned)splits, (unsigned)ty, (unsigned)tz);
-    return launch<false>(x3 ? wgrad_kernel<true> : wgrad_kernel<false>, grid, dim3(kThreads), 0, st, a);
+    return launch(x3 ? wgrad_kernel<true> : wgrad_kernel<false>, grid, dim3(kThreads), 0, st, a);
 }
 
 }  // namespace lin
@@ -780,7 +774,7 @@ int crfconv_bn_act_fwd(const float* H, const float* scale, const float* shift, c
     if (M == 0) return CRF_OK;
     const int64_t total4 = M * (C / 4);
     const unsigned grid = (unsigned)std::min<int64_t>(ceil_div(total4, 256), (int64_t)kNumSMs * 16);
-    CRF_CUDA(launch_k(lin::bn_act_fwd_kernel, dim3(grid), dim3(256), 0, (cudaStream_t)stream, H, scale, shift, R, slope, Y, total4, C / 4));
+    lin::bn_act_fwd_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(H, scale, shift, R, slope, Y, total4, C / 4);
     CRF_LAUNCH_CHECK();
     return CRF_OK;
 }
@@ -811,7 +805,7 @@ int crfconv_bn_finalize_bwd(const float* sums, int64_t count, float* k1, float* 
 int crfconv_grad_slots_reduce(const float* scratch, float* dW, int64_t n, int64_t stride, void* stream) {
     if (n < 0 || !scratch || !dW || stride < n) return CRF_ERR_INVALID_ARG;
     if (n == 0) return CRF_OK;
-    CRF_CUDA(launch_k(lin::grad_slots_reduce_kernel, dim3((unsigned)ceil_div(n, 256)), dim3(256), 0, (cudaStream_t)stream, scratch, dW, (int)n, stride));
+    lin::grad_slots_reduce_kernel<<<(unsigned)ceil_div(n, 256), 256, 0, (cudaStream_t)stream>>>(scratch, dW, (int)n, stride);
     CRF_LAUNCH_CHECK();
     return CRF_OK;
 }
@@ -847,7 +841,7 @@ int crfconv_linear_bwd(const float* dY, const float* H, const float* act_ref, co
     auto finish = [&](int rc) -> int {
         if (rc != CRF_OK || !slots || dW_scratch_stride > 0) return rc;
         ++launches;
-        return lin::launch<false>(lin::grad_slots_reduce_kernel, dim3((unsigned)ceil_div((int64_t)Cout * Ktot, 256)), dim3(256), 0, st,
+        return lin::launch(lin::grad_slots_reduce_kernel, dim3((unsigned)ceil_div((int64_t)Cout * Ktot, 256)), dim3(256), 0, st,
                                   dW_scratch, dW, Cout * Ktot, (int64_t)Cout * Ktot);
     };
 
@@ -914,8 +908,8 @@ int crfconv_bn_bwd_reduce_fin(const float* dY, const float* H, const float* act_
     // exactly one resident wave: 3 (REF, 84 registers) or 4 (64 registers) CTAs per SM
     const cl::BwdFin fin{sums, counter, (double)M, k1, k2, dgamma, dbeta};
     const unsigned grid = (unsigned)std::min<int64_t>(ceil_div(M, rows_per_it * 8), (int64_t)kNumSMs * (act_ref ? 3 : 4));   // <= cl::kMaxTicketGrid
-    if (act_ref) CRF_CUDA(launch_k(lin::bn_bwd_reduce_kernel<true>, dim3(grid), dim3(256), 0, (cudaStream_t)stream, dY, H, bn, sums, M, C, fin));
-    else CRF_CUDA(launch_k(lin::bn_bwd_reduce_kernel<false>, dim3(grid), dim3(256), 0, (cudaStream_t)stream, dY, H, bn, sums, M, C, fin));
+    if (act_ref) lin::bn_bwd_reduce_kernel<true><<<grid, 256, 0, (cudaStream_t)stream>>>(dY, H, bn, sums, M, C, fin);
+    else lin::bn_bwd_reduce_kernel<false><<<grid, 256, 0, (cudaStream_t)stream>>>(dY, H, bn, sums, M, C, fin);
     CRF_LAUNCH_CHECK();
     return CRF_OK;
 }

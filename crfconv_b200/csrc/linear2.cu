@@ -766,8 +766,8 @@ int try_fwd2(const FwdArgs& a, int precision, cudaStream_t st) {
     auto go = [&](auto bnv) {
         constexpr int BN = decltype(bnv)::value;
         if (precision == 0)              // fp32-grade forward (3xTF32)
-            return launch<false>(fwd2t_kernel<BN>, dim3(std::min(ntiles, FwdT<BN>::CTAS * kNumSMs)), dim3(kThreads), fwd2t_smem<BN>(Kpad), st, a, ntiles);
-        return launch<false>(fwd2_kernel<BN>, dim3(std::min(ntiles, 2 * kNumSMs)), dim3(kThreads), fwd2_smem<BN>(Kpad), st, a, ntiles);
+            return launch(fwd2t_kernel<BN>, dim3(std::min(ntiles, FwdT<BN>::CTAS * kNumSMs)), dim3(kThreads), fwd2t_smem<BN>(Kpad), st, a, ntiles);
+        return launch(fwd2_kernel<BN>, dim3(std::min(ntiles, 2 * kNumSMs)), dim3(kThreads), fwd2_smem<BN>(Kpad), st, a, ntiles);
     };
     if (a.Cout > 32) return go(std::integral_constant<int, 64>{});
     if (a.Cout > 16) return go(std::integral_constant<int, 32>{});
@@ -789,10 +789,10 @@ int try_dgrad2(const DgradArgs& a, int precision, cudaStream_t st) {
         constexpr int BM = 16 * (8 / (BN >= 64 ? 2 : 1));
         const int ntiles = (int)ceil_div(a.M, BM);
         const dim3 grid(std::min(ntiles, 2 * kNumSMs));
-        if (ref) return x3 ? launch<false>(dgrad2_kernel<BN, true, true>, grid, dim3(kThreads), dgrad2_smem<BN, true>(Kpad), st, a, ntiles)
-                           : launch<false>(dgrad2_kernel<BN, false, true>, grid, dim3(kThreads), dgrad2_smem<BN, true>(Kpad), st, a, ntiles);
-        return x3 ? launch<false>(dgrad2_kernel<BN, true, false>, grid, dim3(kThreads), dgrad2_smem<BN, false>(Kpad), st, a, ntiles)
-                  : launch<false>(dgrad2_kernel<BN, false, false>, grid, dim3(kThreads), dgrad2_smem<BN, false>(Kpad), st, a, ntiles);
+        if (ref) return x3 ? launch(dgrad2_kernel<BN, true, true>, grid, dim3(kThreads), dgrad2_smem<BN, true>(Kpad), st, a, ntiles)
+                           : launch(dgrad2_kernel<BN, false, true>, grid, dim3(kThreads), dgrad2_smem<BN, true>(Kpad), st, a, ntiles);
+        return x3 ? launch(dgrad2_kernel<BN, true, false>, grid, dim3(kThreads), dgrad2_smem<BN, false>(Kpad), st, a, ntiles)
+                  : launch(dgrad2_kernel<BN, false, false>, grid, dim3(kThreads), dgrad2_smem<BN, false>(Kpad), st, a, ntiles);
     };
     if (Ktot > 64) return go(std::integral_constant<int, 128>{});
     if (Ktot > 32) return go(std::integral_constant<int, 64>{});
@@ -813,8 +813,8 @@ int try_wgrad2(const WgradArgs& a, int precision, cudaStream_t st) {
     if (a.Cout == 32 && Ktot == 32 && a.C2 == 0) {
         const int ntiles = (int)ceil_div(a.M, 128);
         const dim3 grid(std::min(ntiles, 4 * kNumSMs));
-        return ref ? launch<false>(wgrad_small_kernel<32, true>, grid, dim3(kThreads), 0, st, a, ntiles)
-                   : launch<false>(wgrad_small_kernel<32, false>, grid, dim3(kThreads), 0, st, a, ntiles);
+        return ref ? launch(wgrad_small_kernel<32, true>, grid, dim3(kThreads), 0, st, a, ntiles)
+                   : launch(wgrad_small_kernel<32, false>, grid, dim3(kThreads), 0, st, a, ntiles);
     }
     const int CO = a.Cout <= 16 ? 16 : (a.Cout <= 32 ? 32 : 64);
     const int KP = Ktot <= 16 ? 16 : (Ktot <= 32 ? 32 : (Ktot <= 64 ? 64 : 128));
@@ -822,10 +822,10 @@ int try_wgrad2(const WgradArgs& a, int precision, cudaStream_t st) {
     const dim3 grid(std::min(ntiles, 2 * kNumSMs));
 #define CRF_WG(co, kp)                                                                                                                       \
     if (CO == co && KP == kp) {                                                                                                              \
-        if (ref) return x3 ? launch<false>(wgrad2_kernel<co, kp, true, true>, grid, dim3(kThreads), wgrad2_smem<co, kp, true>(), st, a, ntiles)     \
-                           : launch<false>(wgrad2_kernel<co, kp, false, true>, grid, dim3(kThreads), wgrad2_smem<co, kp, true>(), st, a, ntiles);   \
-        return x3 ? launch<false>(wgrad2_kernel<co, kp, true, false>, grid, dim3(kThreads), wgrad2_smem<co, kp, false>(), st, a, ntiles)            \
-                  : launch<false>(wgrad2_kernel<co, kp, false, false>, grid, dim3(kThreads), wgrad2_smem<co, kp, false>(), st, a, ntiles);          \
+        if (ref) return x3 ? launch(wgrad2_kernel<co, kp, true, true>, grid, dim3(kThreads), wgrad2_smem<co, kp, true>(), st, a, ntiles)     \
+                           : launch(wgrad2_kernel<co, kp, false, true>, grid, dim3(kThreads), wgrad2_smem<co, kp, true>(), st, a, ntiles);   \
+        return x3 ? launch(wgrad2_kernel<co, kp, true, false>, grid, dim3(kThreads), wgrad2_smem<co, kp, false>(), st, a, ntiles)            \
+                  : launch(wgrad2_kernel<co, kp, false, false>, grid, dim3(kThreads), wgrad2_smem<co, kp, false>(), st, a, ntiles);          \
     }
     CRF_WG(64, 128) CRF_WG(64, 64) CRF_WG(64, 32) CRF_WG(64, 16)
     CRF_WG(32, 128) CRF_WG(32, 64) CRF_WG(32, 32)

@@ -85,7 +85,6 @@ __global__ void __launch_bounds__(kThreads, 1) fwd3_kernel(const FwdArgs a, cons
     uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(tempty + 2);
 
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    pdl_trigger();                                                 // (common.cuh) the weight staging below overlaps the previous kernel's tail
     if (warp == 0) tmem_alloc(tmem_slot, L::kTmemCols);
     if (tid == kEpiWarps * 32) {
         for (int i = 0; i < RING; ++i) { mbar_init(full + i, 1); mbar_init(empty + i, 1); }
@@ -124,7 +123,6 @@ __global__ void __launch_bounds__(kThreads, 1) fwd3_kernel(const FwdArgs a, cons
             }
         }
     }
-    pdl_wait();                                                    // weights are parameters; scale1 / shift1 and the activations are upstream results
     for (int k = tid; k < Kpad; k += kThreads) {
         float sc = 1.f, sh = 0.f;
         if (a.scale1 && k < nch1 * BK && k < a.C1) { sc = __ldg(a.scale1 + k); sh = __ldg(a.shift1 + k); }
@@ -395,9 +393,9 @@ int try_fwd3(const FwdArgs& a, int precision, cudaStream_t st) {
     if (ntiles <= 0) return kDeclined;
     if (a.fin.part && (a.fin.part != a.stats || (a.Cout != 64 && a.Cout != 32 && a.Cout != 16))) return kDeclined;   // fused finalize: Cout == BN only
     const dim3 grid(std::min(ntiles, kNumSMs));
-    if (a.Cout > 32) return launch<true>(fwd3_kernel<64>, grid, dim3(kThreads), Layout<64>::bytes(nch), st, a, ntiles);
-    if (a.Cout > 16) return launch<true>(fwd3_kernel<32>, grid, dim3(kThreads), Layout<32>::bytes(nch), st, a, ntiles);
-    return launch<true>(fwd3_kernel<16>, grid, dim3(kThreads), Layout<16>::bytes(nch), st, a, ntiles);
+    if (a.Cout > 32) return launch(fwd3_kernel<64>, grid, dim3(kThreads), Layout<64>::bytes(nch), st, a, ntiles);
+    if (a.Cout > 16) return launch(fwd3_kernel<32>, grid, dim3(kThreads), Layout<32>::bytes(nch), st, a, ntiles);
+    return launch(fwd3_kernel<16>, grid, dim3(kThreads), Layout<16>::bytes(nch), st, a, ntiles);
 }
 
 }  // namespace lin

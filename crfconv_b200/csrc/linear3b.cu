@@ -74,7 +74,6 @@ __global__ void __launch_bounds__(kThreads, 1) bwd3_kernel(const DgradArgs d, co
     const int T = nchX + NB;                                                  // tasks per stage
     const bool plain = a.bn.scale == nullptr;
 
-    pdl_trigger();
     if (warp == 0) tmem_alloc(tmem_slot, kTmemCols);
     if (tid == kEpiWarps * 32) {
         for (int i = 0; i < kStages; ++i) {
@@ -106,7 +105,6 @@ __global__ void __launch_bounds__(kThreads, 1) bwd3_kernel(const DgradArgs d, co
             }
         }
     }
-    pdl_wait();
     for (int k = tid; k < BN; k += kThreads) {
         const float4 p = (!plain && k < C) ? a.bn.coef(k) : make_float4(1.f, 0.f, 0.f, 0.f);
         s_par[k] = p.x; s_par[BN + k] = p.y; s_par[2 * BN + k] = p.z; s_par[3 * BN + k] = p.w;
@@ -389,7 +387,7 @@ int try_bwd3(const DgradArgs& d, const WgradArgs& w, int precision, cudaStream_t
     if ((d.dX1 && !aligned16(d.dX1)) || (d.dX2 && !aligned16(d.dX2))) return kDeclined;
     const int ntiles = (int)ceil_div(w.M, RS);
     if (ntiles <= 0) return kDeclined;
-    return launch<true>(bwd3_kernel, dim3(std::min(ntiles, kNumSMs)), dim3(kThreads), kSmemBytes, st, d, w, ntiles);
+    return launch(bwd3_kernel, dim3(std::min(ntiles, kNumSMs)), dim3(kThreads), kSmemBytes, st, d, w, ntiles);
 }
 
 }  // namespace lin

@@ -51,7 +51,6 @@ __global__ void __launch_bounds__(kThreads, 1) dgrad3_kernel(const DgradArgs a, 
 
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const bool plain = a.bn.scale == nullptr;
-    pdl_trigger();
     if (warp == 0) tmem_alloc(tmem_slot, kTmemCols);
     if (tid == kEpiWarps * 32) {
         for (int i = 0; i < RING; ++i) { mbar_init(full + i, 1); mbar_init(empty + i, 1); }
@@ -85,7 +84,6 @@ __global__ void __launch_bounds__(kThreads, 1) dgrad3_kernel(const DgradArgs a, 
             }
         }
     }
-    pdl_wait();                                                    // W is a parameter; the BatchNorm constants, dY and H are upstream results
     for (int k = tid; k < Kpad; k += kThreads) {
         const float4 p = (!plain && k < C) ? a.bn.coef(k) : make_float4(1.f, 0.f, 0.f, 0.f);
         s_par[k] = p.x; s_par[Kpad + k] = p.y; s_par[2 * Kpad + k] = p.z; s_par[3 * Kpad + k] = p.w;
@@ -252,7 +250,7 @@ int try_dgrad3(const DgradArgs& a, int precision, cudaStream_t st) {
     if (Ktot <= 64 || a.Cout <= 32) return kDeclined;  // narrower products: the mma.sync kernel is as fast or faster (measured)
     const int ntiles = (int)ceil_div(a.M, BM);
     if (ntiles <= 0) return kDeclined;
-    return launch<true>(dgrad3_kernel, dim3(std::min(ntiles, kNumSMs)), dim3(kThreads), smem_bytes((a.Cout + BK - 1) / BK), st, a, ntiles);
+    return launch(dgrad3_kernel, dim3(std::min(ntiles, kNumSMs)), dim3(kThreads), smem_bytes((a.Cout + BK - 1) / BK), st, a, ntiles);
 }
 
 }  // namespace lin

@@ -63,14 +63,12 @@ __global__ void __launch_bounds__(kThreads, 1) wgrad3_kernel(const WgradArgs a, 
     const int T = 2 * (nchX + NB);                                            // tasks per stage
     const bool plain = a.bn.scale == nullptr;
 
-    pdl_trigger();
     if (warp == 0) tmem_alloc(tmem_slot, L::kTmemCols);
     if (tid == kEpiWarps * 32) {
         for (int i = 0; i < 2; ++i) { mbar_init(full + i, (uint32_t)T); mbar_init(empty + i, 1); }
         mbar_init(done, 1);
         mbar_init_fence();
     }
-    pdl_wait();
     for (int k = tid; k < BN; k += kThreads) {
         const float4 p = (!plain && k < C) ? a.bn.coef(k) : make_float4(1.f, 0.f, 0.f, 0.f);
         s_par[k] = p.x; s_par[BN + k] = p.y; s_par[2 * BN + k] = p.z; s_par[3 * BN + k] = p.w;
@@ -261,8 +259,8 @@ int try_wgrad3(const WgradArgs& a, int precision, cudaStream_t st) {
     const int ntiles = (int)ceil_div(a.M, RS);
     if (ntiles <= 0) return kDeclined;
     const dim3 grid(std::min(ntiles, kNumSMs));
-    if (a.Cout > 32) return launch<true>(wgrad3_kernel<64>, grid, dim3(kThreads), Layout<64>::bytes(), st, a, ntiles);
-    return launch<true>(wgrad3_kernel<32>, grid, dim3(kThreads), Layout<32>::bytes(), st, a, ntiles);
+    if (a.Cout > 32) return launch(wgrad3_kernel<64>, grid, dim3(kThreads), Layout<64>::bytes(), st, a, ntiles);
+    return launch(wgrad3_kernel<32>, grid, dim3(kThreads), Layout<32>::bytes(), st, a, ntiles);
 }
 
 }  // namespace lin

@@ -68,19 +68,13 @@ struct WgradArgs {
 constexpr int kDeclined = -1000;   // below every CRF_ERR_* code; cudaError_t values are >= 0
 
 // Raises kernel's dynamic shared-memory limit to smem (when smem > 0), launches it and returns CRF_OK or the CUDA error.
-// PDL = true launches through launch_k (common.cuh): only for kernels that execute pdl_wait().  The others are launched
-// plainly and must never carry the programmatic-serialization attribute.
-template <bool PDL, typename... KArgs, typename... Args>
+template <typename... KArgs, typename... Args>
 inline int launch(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args&&... args) {
     cudaError_t e = cudaSuccess;
     if (smem > 0) e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e == cudaSuccess) {
-        if constexpr (PDL) {
-            e = launch_k(kernel, grid, block, smem, st, static_cast<Args&&>(args)...);
-        } else {
-            kernel<<<grid, block, smem, st>>>(static_cast<KArgs>(args)...);
-            e = cudaPeekAtLastError();
-        }
+        kernel<<<grid, block, smem, st>>>(static_cast<KArgs>(args)...);
+        e = cudaPeekAtLastError();
     }
     return e == cudaSuccess ? CRF_OK : (int)e;
 }

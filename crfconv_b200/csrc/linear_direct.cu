@@ -174,7 +174,7 @@ inline int run(const WgradArgs& a, cudaStream_t st) {
     constexpr int per_sm = MB * NB > 4 ? 1 : 2;
     const int64_t tiles = ceil_div(a.M, 16);
     const unsigned grid = (unsigned)std::max<int64_t>(1, std::min<int64_t>(ceil_div(tiles, kWarps), (int64_t)kNumSMs * per_sm));
-    return launch<false>(wgrad_direct_kernel<MB, NB>, dim3(grid), dim3(kThreads), 0, st, a);
+    return launch(wgrad_direct_kernel<MB, NB>, dim3(grid), dim3(kThreads), 0, st, a);
 }
 
 }  // namespace dw
@@ -346,7 +346,7 @@ template <int KP, int NP>
 inline int run(const UpArgs& a, cudaStream_t st) {
     const int64_t tiles = ceil_div(a.M, (int64_t)16);
     const unsigned grid = (unsigned)std::max<int64_t>(1, std::min<int64_t>(ceil_div(tiles, (int64_t)kWarps), (int64_t)kNumSMs * (NP > 64 ? 1 : 2)));
-    return launch<false>(upproj_kernel<KP, NP>, dim3(grid), dim3(kThreads), 0, st, a);
+    return launch(upproj_kernel<KP, NP>, dim3(grid), dim3(kThreads), 0, st, a);
 }
 
 inline int dispatch(const UpArgs& a, cudaStream_t st) {

@@ -355,7 +355,7 @@ int try_narrow_fwd(const FwdArgs& a, cudaStream_t st) {
     if (!aligned16(a.X1) || (a.C2 && !aligned16(a.X2)) || !aligned16(a.Y)) return kDeclined;
     const int ntiles = (int)ceil_div(a.M, TR);
     auto go = [&](auto kern, size_t smem) {
-        return launch<false>(kern, dim3(std::min(ntiles, ctas_per_sm(smem) * kNumSMs)), dim3(TR), smem, st, a, ntiles);
+        return launch(kern, dim3(std::min(ntiles, ctas_per_sm(smem) * kNumSMs)), dim3(TR), smem, st, a, ntiles);
     };
     if (a.Cout > 8) return go(fwd_kernel<16>, fwd_smem<16>(Ktot));
     return go(fwd_kernel<8>, fwd_smem<8>(Ktot));
@@ -379,7 +379,7 @@ int try_narrow_bwd(const DgradArgs& d, const WgradArgs* w, cudaStream_t st) {
     const bool ref = d.bn.scale && d.bn.act_ref;
     const int ntiles = (int)ceil_div(d.M, TR);
     auto go = [&](auto kern, size_t smem) {
-        return launch<false>(kern, dim3(std::min(ntiles, ctas_per_sm(smem) * kNumSMs)), dim3(TR), smem, st, b, ntiles);
+        return launch(kern, dim3(std::min(ntiles, ctas_per_sm(smem) * kNumSMs)), dim3(TR), smem, st, b, ntiles);
     };
     if (C > 8) return ref ? go(bwd_kernel<16, 16, true>, bwd_smem<16, 16, true>()) : go(bwd_kernel<16, 16, false>, bwd_smem<16, 16, false>());
     return ref ? go(bwd_kernel<8, 16, true>, bwd_smem<8, 16, true>()) : go(bwd_kernel<8, 16, false>, bwd_smem<8, 16, false>());

@@ -370,7 +370,7 @@ int try_fwd_small(const FwdArgs& a, cudaStream_t st) {
     const int tn = (int)ceil_div(a.Cout, BN);
     if (!few_rows(a.M, tn)) return kDeclined;
     const dim3 grid((unsigned)ceil_div(a.M, (int64_t)BM), (unsigned)tn);
-    return launch<false>(BN == 64 ? fwd_small_kernel<64> : fwd_small_kernel<32>, grid, dim3(kThreads), 0, st, a);
+    return launch(BN == 64 ? fwd_small_kernel<64> : fwd_small_kernel<32>, grid, dim3(kThreads), 0, st, a);
 }
 
 int try_dgrad_small(const DgradArgs& a, cudaStream_t st) {
@@ -385,8 +385,8 @@ int try_dgrad_small(const DgradArgs& a, cudaStream_t st) {
     const dim3 grid((unsigned)ceil_div(a.M, (int64_t)BM), (unsigned)tn);
     const size_t smem = a.bn.scale ? (size_t)a.Cout * sizeof(float4) : 0;
     const bool ref = a.bn.scale && a.bn.act_ref;
-    if (BN == 64) return launch<false>(ref ? dgrad_small_kernel<64, true> : dgrad_small_kernel<64, false>, grid, dim3(kThreads), smem, st, a);
-    return launch<false>(ref ? dgrad_small_kernel<32, true> : dgrad_small_kernel<32, false>, grid, dim3(kThreads), smem, st, a);
+    if (BN == 64) return launch(ref ? dgrad_small_kernel<64, true> : dgrad_small_kernel<64, false>, grid, dim3(kThreads), smem, st, a);
+    return launch(ref ? dgrad_small_kernel<32, true> : dgrad_small_kernel<32, false>, grid, dim3(kThreads), smem, st, a);
 }
 
 int try_wgrad_rows(WgradArgs a, cudaStream_t st) {
@@ -401,7 +401,7 @@ int try_wgrad_rows(WgradArgs a, cudaStream_t st) {
     a.rows_per_cta = ceil_div(ceil_div(a.M, splits), (int64_t)BM) * BM;
     splits = ceil_div(a.M, a.rows_per_cta);
     const dim3 grid((unsigned)splits, (unsigned)ty, (unsigned)tz);
-    return launch<false>(a.bn.scale && a.bn.act_ref ? wgrad_rows_kernel<true> : wgrad_rows_kernel<false>, grid, dim3(kThreads), 0, st, a);
+    return launch(a.bn.scale && a.bn.act_ref ? wgrad_rows_kernel<true> : wgrad_rows_kernel<false>, grid, dim3(kThreads), 0, st, a);
 }
 
 }  // namespace lin

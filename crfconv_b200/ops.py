@@ -312,23 +312,6 @@ def crf_upsample_fwd(Hu, bn: BN, up_idx, B, N, Nc):
     return z
 
 
-def crf_upsample_fwd_packed(Hu, bn: BN, up_idx, YX, B, N, Nc):
-    """z = BN(Hu)[up_idx] written into the z half of the packed [B·N,32] mean-field buffer."""
-    L = _lib.lib()
-    with _call("crf_upsample_fwd_packed", 1, _nbytes(Hu, up_idx) + YX.numel() * 2):
-        rc = L.crfconv_crf_upsample_fwd_packed(_p(Hu), _p(bn.scale), _p(bn.shift), _p(up_idx), _p(YX), B, N, Nc, _lib.stream_ptr())
-    _lib.check(rc, "crf_upsample_fwd_packed")
-
-
-def crf_step_fwd_packed(YX, scale_y, nbr, Cm, Minv, B, N):
-    L = _lib.lib()
-    xout = torch.empty((B * N, 16), dtype=torch.float32, device=YX.device)
-    with _call("crf_step_fwd_packed", 1, _nbytes(YX, nbr, xout)):
-        rc = L.crfconv_crf_step_fwd_packed(_p(YX), _p(scale_y), _p(nbr), _p(Cm), _p(Minv), _p(xout), B, N, _lib.stream_ptr())
-    _lib.check(rc, "crf_step_fwd_packed")
-    return xout
-
-
 def crf_upsample_bwd(Gz, G0, up_idx, Gu, B, N, Nc):
     L = _lib.lib()
     with _call(f"crf_upsample_bwd[{Gz.shape[1]}]", 1, _nbytes(Gz, G0, up_idx, Gu)):
@@ -542,10 +525,9 @@ def _bn_fin_args(bn_module):
             _p(bn_module.running_var) if track else None, float(bn_module.eps), float(bn_module.momentum))
 
 
-def lin16_fwd(X, W, bn: BN, bn_module, part, counter, pre: BN = None, pslope=1.0, out=None, packed_out=None):
+def lin16_fwd(X, W, bn: BN, bn_module, part, counter, pre: BN = None, pslope=1.0, out=None):
     """H = act(X)·Wᵀ (16 output channels) with `bn`'s scale/shift/mean/invstd (and the module's running statistics) finalized by
-    the same launch.  pre: BN state whose affine + LeakyReLU(pslope) is applied to X on the fly (X has 16 channels then).
-    packed_out: [M,32] buffer that also receives H in the mean field's packed layout (crf_step_fwd_packed)."""
+    the same launch.  pre: BN state whose affine + LeakyReLU(pslope) is applied to X on the fly (X has 16 channels then)."""
     L = _lib.lib()
     M, Cin = X.shape
     Y = out if out is not None else torch.empty((M, 16), dtype=torch.float32, device=X.device)
@@ -553,7 +535,7 @@ def lin16_fwd(X, W, bn: BN, bn_module, part, counter, pre: BN = None, pslope=1.0
     bn.count, bn.training = int(M), True
     with _call(f"lin16_fwd[{Cin}]", 1, _nbytes(X, Y)):
         rc = L.crfconv_lin16_fwd(_p(X), int(Cin), _p(W), _p(pre.scale) if pre else None, _p(pre.shift) if pre else None, float(pslope),
-                                 _p(Y), _p(packed_out), int(M), _p(part), _p(counter), gm, bt, rm, rv, eps, mom, _p(bn.scale), _p(bn.shift), _p(bn.mean),
+                                 _p(Y), int(M), _p(part), _p(counter), gm, bt, rm, rv, eps, mom, _p(bn.scale), _p(bn.shift), _p(bn.mean),
                                  _p(bn.invstd), _lib.stream_ptr())
     _lib.check(rc, "lin16_fwd")
     return Y
@@ -641,13 +623,12 @@ def out16_bwd(dO, H3, bn3: BN, slope3, X, W3, part, counter, dgamma, dbeta, dW3,
 
 
 def crf_step_bwd_fused(Hy, bn_y: BN, z, xprev, nbr, Cm, Minv, g, xT, Q, a0, Gz, gz_acc, gprev, Gy, GC_slots, GM_slots, slot_stride, ysum,
-                       B, N, K, finalize, counter, gamma_y, dgamma, dbeta, packed=False):
-    """packed: Hy is the [M,32] packed {Hy | z} buffer of the first step (z / xprev are ignored and may be None)."""
+                       B, N, K, finalize, counter, gamma_y, dgamma, dbeta):
     L = _lib.lib()
     with _call("crf_step_bwd_fused", 1, _nbytes(Hy, z, xprev, nbr, g, xT, Gz, gprev, Gy)):
         rc = L.crfconv_crf_step_bwd_fused(_p(Hy), _p(bn_y.scale), _p(z), _p(xprev), _p(nbr), _p(Cm), _p(Minv), _p(g), _p(xT), _p(Q), _p(a0),
                                           _p(Gz), int(gz_acc), _p(gprev), _p(Gy), _p(GC_slots), _p(GM_slots), int(slot_stride), _p(ysum),
-                                          B, N, K, Gz.shape[1], int(bool(packed)), int(bool(finalize)), _p(counter), _p(gamma_y), _p(bn_y.k1), _p(bn_y.k2),
+                                          B, N, K, Gz.shape[1], int(bool(finalize)), _p(counter), _p(gamma_y), _p(bn_y.k1), _p(bn_y.k2),
                                           _p(dgamma), _p(dbeta), _lib.stream_ptr())
     _lib.check(rc, "crf_step_bwd_fused")
 

@@ -155,13 +155,6 @@ int crfconv_crf_compat_bwd(const float* c, const float* Minv, const float* GC, c
 /* z[B·N,F] = (Hu*scale + shift)[up_idx]  — unary_nn's last BatchNorm fused into the nearest-coarse upsample. */
 int crfconv_crf_upsample_fwd(const float* Hu, const float* scale, const float* shift, const int64_t* up_idx, float* z, int64_t B,
                              int64_t N, int64_t Nc, int F, void* stream);
-/* Packed mean-field operands (F = 16, K = 16, first step: x^0 = z): YX[B·N,32], floats [8s, 8s+4) = Hy[4s..4s+3], [8s+4, 8s+8) = z[4s..4s+3]
- * (32-byte aligned).  One 128-byte line per gathered neighbour instead of two half lines; the Hy half is written by crfconv_lin16_fwd
- * (Ypk), the z half by crfconv_crf_upsample_fwd_packed.  Same arithmetic as crfconv_crf_upsample_fwd / crfconv_crf_step_fwd. */
-int crfconv_crf_upsample_fwd_packed(const float* Hu, const float* scale, const float* shift, const int64_t* up_idx, float* YX, int64_t B,
-                                    int64_t N, int64_t Nc, void* stream);
-int crfconv_crf_step_fwd_packed(const float* YX, const float* scale_y, const int64_t* neighbor_idx, const float* Cm, const float* Minv,
-                                float* xout, int64_t B, int64_t N, void* stream);
 /* Gu[B·Nc,F] += (Gz + G0) scattered through up_idx (G0 may be NULL). */
 int crfconv_crf_upsample_bwd(const float* Gz, const float* G0, const int64_t* up_idx, float* Gu, int64_t B, int64_t N, int64_t Nc,
                              int F, void* stream);
@@ -187,14 +180,12 @@ int crfconv_fused_max_parts(void);        /* largest grid of a kernel with an ar
 int crfconv_fused_part_floats(void);      /* floats of every `part` scratch argument (per-CTA rows + per-group rows) */
 int crfconv_fused_counter_ints(void);     /* uint32 per `counter` argument */
 int crfconv_out_bwd_part_floats(void);    /* floats of crfconv_out16_bwd's `part` (zero-initialised) */
-/* Tuning knobs for experiments (key 0: CTAs/SM of the mean-field backward, 2 or 3).  Returns the previous value. */
-int crfconv_fused_tune(int key, int value);
 
 /* H[M,16] = act(X[M,Cin])·Wᵀ + BatchNorm finalize of H (MLP(Cin,16), common.py:26-40).  Cin ∈ {64,128}: X raw; Cin = 16: X is the
  * previous layer's pre-BN output and pscale/pshift/pslope its BN affine + LeakyReLU. */
-int crfconv_lin16_fwd(const float* X, int Cin, const float* W, const float* pscale, const float* pshift, float pslope, float* Y, float* Ypk,
-                      int64_t M, float* part, unsigned int* counter, const float* gamma, const float* beta, float* running_mean,
-                      float* running_var, float eps, float momentum, float* scale, float* shift, float* mean, float* invstd, void* stream);
+int crfconv_lin16_fwd(const float* X, int Cin, const float* W, const float* pscale, const float* pshift, float pslope, float* Y, int64_t M,
+                      float* part, unsigned int* counter, const float* gamma, const float* beta, float* running_mean, float* running_var,
+                      float eps, float momentum, float* scale, float* shift, float* mean, float* invstd, void* stream);
 /* H[M,Cout] = X[M,16]·Wᵀ + BatchNorm finalize of H (MLP(16,Cout), Cout = 64: out_nn).  stats [CRFCONV_STAT_SLOTS][2·Cout] zeroed. */
 int crfconv_up16_fwd(const float* X, const float* W, int Cout, float* Y, int64_t M, float* stats, unsigned int* counter, const float* gamma,
                      const float* beta, float* running_mean, float* running_var, float eps, float momentum, float* scale, float* shift,
@@ -229,7 +220,7 @@ int crfconv_out16_bwd(const float* dO, const float* H3, const float* sc3, const 
 int crfconv_crf_step_bwd_fused(const float* Hy, const float* sc_y, const float* z, const float* xprev, const int64_t* neighbor_idx,
                                const float* Cm, const float* Minv, const float* g, const float* xT, const float* Q, const float* a0,
                                float* Gz, int gz_acc, float* gprev, float* Gy, float* GC, float* GM, int64_t slot_stride,
-                               float* ysum, int64_t B, int64_t N, int K, int F, int packed, int finalize, unsigned int* counter,
+                               float* ysum, int64_t B, int64_t N, int K, int F, int finalize, unsigned int* counter,
                                const float* gamma_y, float* k1, float* k2, float* dgamma, float* dbeta, void* stream);
 /* crfconv_crf_upsample_bwd for F = 16 + the BatchNorm-backward constants of unary_nn[1] (Hu = its pre-BN output). */
 int crfconv_crf_upsample_bwd_fused(const float* Gz, const float* G0, const int64_t* up_idx, const float* Hu, const float* mu,

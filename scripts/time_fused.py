@@ -75,10 +75,6 @@ c = torch.eye(F, device=dev) + 0.1 * rnd(F, F)
 Cm, Minv = ops.crf_compat_fwd(c)
 timeit("crf_step_fwd", lambda: ops.crf_step_fwd(H2p, b2.scale, z, z, nbr, Cm, Minv, B, N, K), fb * M * F * 3 + 8 * M * K)
 x1 = ops.crf_step_fwd(H2p, b2.scale, z, z, nbr, Cm, Minv, B, N, K)
-YX = torch.empty(M, 32, device=dev)
-timeit("lin16_fwd[16]  H1p -> H2p + packed copy", lambda: ops.lin16_fwd(H1p, W2, b2, bnm16, part, cnt, pre=b1, pslope=0.1, out=H2p, packed_out=YX), fb * M * 3 * F)
-timeit("crf_upsample_fwd_packed", lambda: ops.crf_upsample_fwd_packed(H2u, b2, up, YX, B, N, Nc), fb * (Mc * F + M * F) + 8 * M)
-timeit("crf_step_fwd_packed", lambda: ops.crf_step_fwd_packed(YX, b2.scale, nbr, Cm, Minv, B, N), fb * M * F * 3 + 8 * M * K)
 H3, Hf = torch.empty(M, Co, device=dev), torch.empty(M, Co, device=dev)
 b3.stats.zero_(); bf.stats.zero_()
 timeit("up16_fwd[64] (mma.sync + fin)", lambda: ops.up16_fwd(x1, Wo, b3, bnm64, cnt, out=H3), fb * M * (F + Co))
@@ -113,21 +109,8 @@ ysum = torch.zeros(128, device=dev)
 gam = torch.ones(F, device=dev)
 d16, e16 = torch.zeros(F, device=dev), torch.zeros(F, device=dev)
 Q.copy_(0.01 * (Q.new_ones(F, F))); a0.zero_()
-for variant in (2, 3):
-    ops._lib.lib().crfconv_fused_tune(0, variant)
-    timeit(f"crf_step_bwd_fused (CTAs/SM = {variant})", lambda: ops.crf_step_bwd_fused(H2p, b2, z, z, nbr, Cm, Minv, T, x1, Q, a0, Gz, False, gp, Gy, scr, scr[256:], 20000,
-                                                                                 ysum, B, N, K, True, cnt, gam, d16, e16), fb * M * F * 7 + 8 * M * K)
-ops._lib.lib().crfconv_fused_tune(0, 0)
-for variant in (2, 3):
-    ops._lib.lib().crfconv_fused_tune(0, variant)
-    timeit(f"crf_step_bwd_fused packed (CTAs/SM = {variant})", lambda: ops.crf_step_bwd_fused(YX, b2, None, None, nbr, Cm, Minv, T, x1, Q, a0, Gz, False, gp, Gy, scr, scr[256:], 20000,
-                                                                                        ysum, B, N, K, True, cnt, gam, d16, e16, packed=True), fb * M * F * 7 + 8 * M * K)
-ops._lib.lib().crfconv_fused_tune(0, 0)
-for mask, what in ((1, "no Gy reds"), (2, "no gprev reds"), (3, "no reds"), (4, "no GC/GM MMA"), (7, "gathers + math only")):
-    ops._lib.lib().crfconv_fused_tune(2, mask)
-    timeit(f"  [timing probe, wrong results] {what}", lambda: ops.crf_step_bwd_fused(H2p, b2, z, z, nbr, Cm, Minv, T, x1, Q, a0, Gz, False, gp, Gy, scr, scr[256:], 20000,
-                                                                                  ysum, B, N, K, True, cnt, gam, d16, e16), fb * M * F * 7 + 8 * M * K)
-ops._lib.lib().crfconv_fused_tune(2, 0)
+timeit("crf_step_bwd_fused", lambda: ops.crf_step_bwd_fused(H2p, b2, z, z, nbr, Cm, Minv, T, x1, Q, a0, Gz, False, gp, Gy, scr, scr[256:], 20000,
+                                                             ysum, B, N, K, True, cnt, gam, d16, e16), fb * M * F * 7 + 8 * M * K)
 mo, vo, ho = (torch.empty(M, F, device=dev) for _ in range(3))
 cgrad, w2grad, w1grad = torch.zeros(F, F, device=dev), torch.zeros(F, F, device=dev), torch.zeros(16, Co, device=dev)
 timeit("  generic crf_step_bwd + GC/GM GEMMs", lambda: (ops.crf_step_bwd(H2p, b2.scale, z, z, nbr, Cm, Minv, T, Gz, gp, Gy, mo, vo, ho, False, B, N, K),

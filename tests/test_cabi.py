@@ -15,10 +15,35 @@ def built():
     return build.build()
 
 
-def _declared():
+def _header():
     src = open(os.path.join(ROOT, "include", "crfconv_b200.h")).read()
     src = re.sub(r"/\*.*?\*/", "", src, flags=re.S)
-    return sorted(set(re.findall(r"\b(crfconv_[a-z0-9_]+)\s*\(", src)))
+    return re.sub(r"//[^\n]*", "", src)
+
+
+def _declared():
+    return sorted(set(re.findall(r"\b(crfconv_[a-z0-9_]+)\s*\(", _header())))
+
+
+_SCALARS = ("int", "int64_t", "size_t", "uint32_t", "float")
+
+
+def _kind(decl):
+    """Kind of a C parameter or return type: 'pointer' or one of _SCALARS ('const float* X' -> 'pointer', 'int64_t M' -> 'int64_t')."""
+    if "*" in decl:
+        return "pointer"
+    typ = decl.split()[0]
+    assert typ in _SCALARS, f"unexpected C type in {decl!r}"
+    return typ
+
+
+def _prototypes():
+    """name -> (return kind, [argument kinds]) for every prototype of the header."""
+    out = {}
+    for ret, name, args in re.findall(r"((?:const\s+)?\w+\s*\**)\s*\b(crfconv_[a-z0-9_]+)\s*\(([^)]*)\)\s*;", _header()):
+        args = " ".join(args.split())
+        out[name] = (_kind(ret), [] if args in ("", "void") else [_kind(a.strip()) for a in args.split(",")])
+    return out
 
 
 def test_library_exports_every_declared_symbol(built):
@@ -30,9 +55,17 @@ def test_library_exports_every_declared_symbol(built):
 
 
 def test_python_signature_table_matches_header(built):
+    """Names, argument counts and argument kinds: ctypes forwards surplus arguments silently, so one stray `int` in _lib would
+    shift every later argument of a call without any error on the host."""
     from crfconv_b200 import _lib
     assert sorted(_lib.SIGNATURES) == _declared()
-    assert _lib.lib().crfconv_abi_version() >= 1
+    protos = _prototypes()
+    assert sorted(protos) == _declared()
+    kind = {ctypes.c_void_p: "pointer", ctypes.c_char_p: "pointer", ctypes.c_int: "int", ctypes.c_int64: "int64_t",
+            ctypes.c_size_t: "size_t", ctypes.c_uint32: "uint32_t", ctypes.c_float: "float"}
+    for name, (res, args) in _lib.SIGNATURES.items():
+        assert (kind[res], [kind[a] for a in args]) == protos[name], name
+    assert _lib.lib().crfconv_abi_version() == 2
     assert _lib.lib().crfconv_status_string(-2) == b"workspace too small"
 
 
